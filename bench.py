@@ -20,7 +20,7 @@ gpu_eager_baseline  the same module as plain PyTorch ops (the oracle's restateme
 train   BASELINE configs[2] ("cfg3") inside the same line: a full bf16 training step (forward, BCE loss, backward,
         NCCL gradient all-reduce when N > 1, AdamW) of the 3-D SwinFusion workload, batch 8 per GPU, samples/s.
 
-  python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--batch B]
+  python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--batch B] [--dump-outputs DIR]
   torchrun ... bench.py --gpus N ...        (one rank per GPU, NCCL; weak scaling)
   python bench.py --workload cfg3|cfg5|cfg5-sweep|mha      (other BASELINE configs as the primary line)
 """
@@ -452,6 +452,22 @@ def workload_config(batch, world):
             "parallelism": f"dp{world}"}
 
 
+DUMP_ROWS = 32768      # token rows of y and dx that --dump-outputs keeps: 12.6 MB each in float32 (all of them: 403 MB at batch 32)
+
+
+def dump_outputs(path, y, dx, attn):
+    """--dump-outputs: the cfg2 step's results as float32 .npy files -- y and dx at a fixed sample of token rows (seed 0,
+    the same rows for the same --batch) and every weight gradient the step produced, in full."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    y, dx = y.detach().reshape(-1, C), dx.reshape(-1, C)
+    rows = torch.randperm(y.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values.to(y.device)
+    arrays = {"y": y[rows], "dx": dx[rows]}
+    arrays.update({f"grad.{n}": p.grad for n, p in attn.named_parameters() if p.grad is not None})
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------
@@ -488,7 +504,14 @@ def main():
                     help="gradient exchange of the training step: one all-reduce of the flat gradient buffer after a graph-replayed "
                          "backward (default) or torch DistributedDataParallel (eager, bucketed overlap)")
     ap.add_argument("--checkpoint", action="store_true", help="activation checkpointing in the training-step workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="cfg2 line: write what the last of the --steps timed steps returned (y, dx, weight gradients) as "
+                         "float32 DIR/<name>.npy, so that two builds can be compared output for output on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "cfg2"):
+        ap.error("--dump-outputs applies to the cfg2 line of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -755,7 +778,13 @@ def main():
     # clocks / throttle reasons are sampled from here to the end of the nested training step: every timed region of the line
     clk = ClockSampler(local)
     clk.__enter__()
-    ms, _, _ = timed(step_fn, args.steps)
+    last = {}
+
+    def timed_step():
+        last["y"] = step_fn()
+    ms, _, _ = timed(timed_step, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["y"], x.grad, attn)
     e2e_prepare()
     for _ in range(2):
         step_e2e()

@@ -1,9 +1,9 @@
 """Generate the golden fixtures in this directory by importing and running the UNMODIFIED
-reference modules from /root/reference (read-only) on seeded synthetic inputs.
+reference modules (read-only) on seeded synthetic inputs.
 
-Run here (CPU container, reference mounted):   python tests/golden/make_golden.py
-The fixtures (*.npz) are committed; /root/reference does not exist on the GPU box, so
-nothing at test time reads it.  Harness-side shims only (SURVEY.md 8c): a `timm` stub on
+Run on a CPU with a checkout of the reference:   MMN_REFERENCE=<dir> python tests/golden/make_golden.py
+The fixtures (*.npz) are committed, so nothing at test time reads the reference.
+Harness-side shims only (SURVEY.md 8c): a `timm` stub on
 sys.path and a CPU `Tensor.get_device` patch for swin_v2_module.py:154.  Gotchas honoured:
 LayerNorm weights randomised (F10), bias tables scaled up, logit_scale values on both sides
 of the ln(100) clamp, k != v tensors for the 3-projection MHA branch, a shifted block whose
@@ -16,7 +16,9 @@ import numpy as np
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("MMN_REFERENCE", "/root/reference")
+REF = os.environ.get("MMN_REFERENCE", "")
+if not (REF and os.path.isdir(os.path.join(REF, "modules"))):
+    sys.exit("set MMN_REFERENCE to a checkout of the reference (the directory holding model.py and modules/)")
 sys.path.insert(0, os.path.join(HERE, "_shims"))
 sys.path.insert(1, REF)
 

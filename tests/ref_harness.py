@@ -1,4 +1,4 @@
-"""Harness for driving the UNMODIFIED reference (`/root/reference`, read-only) from tests and
+"""Harness for driving the UNMODIFIED reference (the checkout MMN_REFERENCE names, read-only) from tests and
 fixture generators: import-time stubs for the packages the reference imports but this image
 lacks, the three shims of SURVEY.md 8c, and `main.py`'s own default arguments per phase.
 
@@ -21,7 +21,7 @@ import types
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = os.environ.get("MMN_REFERENCE", "/root/reference")
+REF = os.environ.get("MMN_REFERENCE", "")
 
 # model class -> (phase whose `_phaseN` flags configure it, extra command line) -- main.py:209-332, utils.py:95-128
 MODELS = {
@@ -35,7 +35,7 @@ MODELS = {
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REF, "model.py"))
+    return bool(REF) and os.path.isfile(os.path.join(REF, "model.py"))
 
 
 class _Stub(types.ModuleType):
