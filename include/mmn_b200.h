@@ -24,6 +24,13 @@
  * mmn_last_error() gives the thread-local message.  There is NO CPU path: every entry
  * point fails with MMN_ERR_CUDA when no CUDA device is usable.
  *
+ * Deterministic mode.  By default the backward entry points accumulate cross-block sums (bias and scale gradients,
+ * column sums, LayerNorm dgamma / dbeta, bias-table gradients) with float atomics, so their last bits can change from run
+ * to run.  mmn_winattn_desc.deterministic, the `deterministic` arguments and the inverse bias index select kernels that
+ * write per-block partial sums and add them in a fixed order instead: the same inputs then give bit-identical outputs
+ * on one GPU model with one build (grid sizes follow the SM count, so not across GPU models).  Their workspace sizes
+ * come from the *_workspace_bytes queries; with the flag off the queries return what the default kernels need.
+ *
  * Token addressing.  A "token row" is num_heads*head_dim contiguous elements; row r of
  * head h of tensor X lives at  X + row_offset(r) + h*head_dim  (element units).
  *   window attention: tokens are indexed in the UN-windowed, UN-shifted (batch, grid...)
@@ -41,7 +48,7 @@
 extern "C" {
 #endif
 
-#define MMN_ABI_VERSION 4
+#define MMN_ABI_VERSION 5
 /* scratch every window-attention launch needs: the tensor-core kernels keep the counters of their run-time work queue
  * there (zeroed by the library on the launch's stream; one buffer per launch, never shared between launches in flight) */
 #define MMN_WINATTN_WORK_BYTES 2048
@@ -73,6 +80,7 @@ typedef struct mmn_winattn_desc {
   uint64_t seed, offset;   /* Philox stream for dropout (same values in fwd and bwd)          */
   int64_t q_row_stride, k_row_stride, v_row_stride, o_row_stride;
   int64_t do_row_stride, dq_row_stride, dk_row_stride, dv_row_stride;   /* bwd only          */
+  int32_t deterministic;   /* bwd: nonzero selects the fixed-order reductions (see above)     */
 } mmn_winattn_desc;
 
 typedef struct mmn_mha_desc {
@@ -114,8 +122,9 @@ int mmn_winattn_fwd(const mmn_winattn_desc* desc, const void* q, const void* k, 
  * ACCUMULATED, may be NULL: column sums over all tokens of dq, dk, dv -- the bias gradients of the
  * projections that produced q, k, v (replaces the reductions autograd does for F.linear's bias,
  * swin_v2_module.py:147-148, swinfusion_module.py:121,221-222).  `workspace`: scratch of
- * max(2*batch*nW*num_heads*N floats, MMN_WINATTN_WORK_BYTES), owned by this launch until it has completed, contents
- * undefined on return. */
+ * mmn_winattn_bwd_workspace_bytes(desc) bytes (16-byte aligned), owned by this launch until it has completed, contents
+ * undefined on return.  With desc->deterministic == 0 that is max(2*batch*nW*num_heads*N floats, MMN_WINATTN_WORK_BYTES). */
+size_t mmn_winattn_bwd_workspace_bytes(const mmn_winattn_desc* desc);
 int mmn_winattn_bwd(const mmn_winattn_desc* desc, const void* q, const void* k, const void* v,
                     const float* bias, const float* head_scale, const float* mask,
                     const void* out, const float* lse, const void* dout,
@@ -136,32 +145,41 @@ int mmn_mha_avg_weights(const mmn_mha_desc* desc, const void* q, const void* k, 
                         const float* lse, float* avg, int device, void* stream);
 
 /* out[c] += sum over rows of x[r*row_stride + c]: the bias gradient of the output projection
- * (F.linear backward, swin_v2_module.py:176) at memory speed.  cols % 8 == 0, cols <= 2048. */
+ * (F.linear backward, swin_v2_module.py:176) at memory speed.  cols % 8 == 0, cols <= 2048.
+ * deterministic != 0: per-block partial sums in `workspace` (mmn_colsum_workspace_bytes(rows, cols) bytes), then a
+ * fixed-order reduction; workspace may be NULL otherwise. */
+size_t mmn_colsum_workspace_bytes(int64_t rows, int32_t cols);
 int mmn_colsum(const void* x, int io_dtype, int64_t rows, int32_t cols, int64_t row_stride, float* out,
-               int device, void* stream);
+               float* workspace, int deterministic, int device, void* stream);
 
 /* SwinV2 continuous relative-position bias (swin_v2_module.py:158-162), fp32:
  *   bias[h][e] = 16 sigmoid(tab[index[e]][h]),  tab[t][h] = sum_j w2[h][j] relu(w1[j] . coords[t] + b1[j])
  * coords (T, n_in) with n_in <= 3, w1 (J, n_in), b1 (J), w2 (nH, J) with nH <= 64, index (NN) int64 in [0, T).
  * fwd writes tab16 (T, nH) [= 16 sigmoid(tab), kept for the backward] and bias (nH, NN).
  * bwd: dbias (nH, NN) -> dw1 (J, n_in), db1 (J), dw2 (nH, J), all OVERWRITTEN; scratch (T, nH) floats.
+ * inv_perm / inv_offsets: NULL, or the inverse of `index` in CSR form -- inv_perm (NN) int32 = the entries e in increasing
+ * order of (index[e], e), inv_offsets (T + 1) int32 = where each table entry's run starts, inv_offsets[T] == NN.  Given,
+ * the table gradient is a gather that sums each entry's dbias values in increasing e (deterministic); NULL, a scatter with
+ * float atomics.  A kernel that finds inv_offsets[T] != NN writes NaN into its output.
  * T * nH <= 12288 (the backward stages d tab in shared memory); MMN_ERR_UNSUPPORTED otherwise. */
 int mmn_cpb_bias_fwd(const float* coords, const float* w1, const float* b1, const float* w2, const int64_t* index,
                      int32_t T, int32_t n_in, int32_t J, int32_t num_heads, int32_t NN,
                      float* tab16, float* bias, int device, void* stream);
 int mmn_cpb_bias_bwd(const float* coords, const float* w1, const float* b1, const float* w2, const int64_t* index,
+                     const int32_t* inv_perm, const int32_t* inv_offsets,
                      const float* tab16, const float* dbias, int32_t T, int32_t n_in, int32_t J, int32_t num_heads, int32_t NN,
                      float* scratch, float* dw1, float* db1, float* dw2, int device, void* stream);
 
 /* Learned relative-position bias table of the fusion blocks (swinfusion_module.py:58-60,127-130,228-231), fp32:
  *   fwd: bias[h][e] = table[index[e]][h]            table (T, nH), index (NN) int64 in [0, T), bias (nH, NN)
- *   bwd: dtable[t][h] = sum over e with index[e] == t of dbias[h][e]     (dtable OVERWRITTEN; float atomics)
+ *   bwd: dtable[t][h] = sum over e with index[e] == t of dbias[h][e]     (dtable OVERWRITTEN; float atomics, or with
+ *        inv_perm / inv_offsets given a fixed-order gather: see mmn_cpb_bias_bwd)
  * i.e. `table[index].view(N, N, nH).permute(2, 0, 1).contiguous()` and its backward in one launch each (PyTorch: index_select +
  * permute copy forward, zeros + index_add backward). */
 int mmn_table_bias_fwd(const float* table, const int64_t* index, int32_t T, int32_t num_heads, int32_t NN, float* bias,
                        int device, void* stream);
-int mmn_table_bias_bwd(const float* dbias, const int64_t* index, int32_t T, int32_t num_heads, int32_t NN, float* dtable,
-                       int device, void* stream);
+int mmn_table_bias_bwd(const float* dbias, const int64_t* index, const int32_t* inv_perm, const int32_t* inv_offsets, int32_t T,
+                       int32_t num_heads, int32_t NN, float* dtable, int device, void* stream);
 
 /* Projections on the tensor cores (csrc/gemm_tc.cu, csrc/linbwd_tc.cu).  They replace the F.linear calls of the path and
  * their autograd backward: swin_v2_module.py:148,176 (qkv, proj) and :27-31 (Mlp: fc1 -> GELU -> fc2),
@@ -176,7 +194,8 @@ int mmn_table_bias_bwd(const float* dbias, const int64_t* index, int32_t T, int3
  *             input) had an activation; act_aux is the y_pre ITS forward wrote, (rows, in) with leading dimension ld_aux;
  *             dw (out, in) fp32 = dy^T x, OVERWRITTEN; db (out) fp32 = column sums of dy, OVERWRITTEN.  dx or dw may be NULL
  *             to skip that half (then db is skipped with dw == NULL only if db is NULL too).
- *             workspace: mmn_linear_bwd_workspace_bytes(rows, in, out) bytes, contents undefined on return.
+ *             workspace: mmn_linear_bwd_workspace_bytes(rows, in, out, deterministic) bytes, contents undefined on return.
+ *             deterministic != 0: db of the dgrad + wgrad path is summed in a fixed order (the fused pass always is).
  *             in = 96 and out in {96, 192, 288, 384} with no activation run as ONE pass over dy and x (linbwd_tc.cu). */
 enum { MMN_ACT_NONE = 0, MMN_ACT_RELU = 1, MMN_ACT_GELU = 2 };
 int mmn_linear_supported(int io_dtype, int64_t rows, int32_t in_features, int32_t out_features, int64_t ld_x, int64_t ld_y);
@@ -184,10 +203,10 @@ int mmn_linear_fwd(const void* x, const void* w, const float* bias, void* y, voi
                    int32_t in_features, int32_t out_features, int64_t ld_x, int64_t ld_y, int device, void* stream);
 int mmn_linear_bwd_supported(int io_dtype, int64_t rows, int32_t in_features, int32_t out_features,
                              int64_t ld_dy, int64_t ld_x, int64_t ld_dx);
-size_t mmn_linear_bwd_workspace_bytes(int64_t rows, int32_t in_features, int32_t out_features);
+size_t mmn_linear_bwd_workspace_bytes(int64_t rows, int32_t in_features, int32_t out_features, int deterministic);
 int mmn_linear_bwd(const void* dy, const void* x, const void* w, void* dx, float* dw, float* db, void* workspace,
                    const void* act_aux, int64_t ld_aux, int act, int io_dtype, int64_t rows, int32_t in_features,
-                   int32_t out_features, int64_t ld_dy, int64_t ld_x, int64_t ld_dx, int device, void* stream);
+                   int32_t out_features, int64_t ld_dy, int64_t ld_x, int64_t ld_dx, int deterministic, int device, void* stream);
 
 /* LayerNorm fused with the residual add around it (csrc/layernorm.cu), one pass over the rows forward, one backward.
  * Replaces the norm + add (+ autocast cast) sequences of swin_v2_module.py:299,302 (res-post-norm),
@@ -199,15 +218,19 @@ int mmn_linear_bwd(const void* dy, const void* x, const void* w, void* dx, float
  * for the backward.  cols even and <= 1536.
  * Backward: g_sum / g_norm = gradients w.r.t. out_sum / out_norm (either may be NULL), x = the normalised quantity (PRE: s,
  * i.e. out_sum or the lone input; POST: delta).  d_resid / d_delta may be NULL.  dgamma / dbeta (cols) fp32 are ACCUMULATED
- * into with atomics (the caller zeroes them); either may be NULL. */
+ * into (the caller zeroes them); either may be NULL.  By default each block adds its column sums with atomics;
+ * deterministic != 0 has each block write them to `workspace` (mmn_layernorm_bwd_workspace_bytes(rows, cols) bytes) and
+ * adds them in block order.  workspace may be NULL otherwise. */
 enum { MMN_LN_PRE = 0, MMN_LN_POST = 1 };
 int mmn_layernorm_supported(int32_t cols);
 int mmn_layernorm_fwd(const void* resid, int resid_dtype, const void* delta, int delta_dtype, const float* gamma, const float* beta,
                       float eps, int mode, void* out_sum, int sum_dtype, void* out_norm, int norm_dtype, float* mean, float* rstd,
                       int64_t rows, int32_t cols, int device, void* stream);
+size_t mmn_layernorm_bwd_workspace_bytes(int64_t rows, int32_t cols);
 int mmn_layernorm_bwd(const void* g_sum, int gs_dtype, const void* g_norm, int gn_dtype, const void* x, int x_dtype,
                       const float* gamma, const float* mean, const float* rstd, int mode, void* d_resid, int dr_dtype,
-                      void* d_delta, int dd_dtype, float* dgamma, float* dbeta, int64_t rows, int32_t cols, int device, void* stream);
+                      void* d_delta, int dd_dtype, float* dgamma, float* dbeta, float* workspace, int deterministic,
+                      int64_t rows, int32_t cols, int device, void* stream);
 
 #ifdef __cplusplus
 }

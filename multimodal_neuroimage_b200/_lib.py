@@ -42,11 +42,12 @@ MASK_NONE, MASK_SHIFT, MASK_TENSOR, MASK_FUTURE = 0, 1, 2, 3
 PATH_AUTO, PATH_GENERIC, PATH_TCGEN05 = 0, 1, 2
 ACT_NONE, ACT_RELU, ACT_GELU = 0, 1, 2
 LN_PRE, LN_POST = 0, 1
-ABI_VERSION = 4
+ABI_VERSION = 5
 WINATTN_WORK_BYTES = 2048
 
 EXPORTS = ["mmn_abi_version", "mmn_last_error", "mmn_winattn_path", "mmn_mha_path", "mmn_launch_count",
-           "mmn_winattn_fwd", "mmn_winattn_bwd", "mmn_mha_fwd", "mmn_mha_bwd", "mmn_mha_avg_weights", "mmn_colsum",
+           "mmn_winattn_fwd", "mmn_winattn_bwd", "mmn_winattn_bwd_workspace_bytes", "mmn_mha_fwd", "mmn_mha_bwd", "mmn_mha_avg_weights",
+           "mmn_colsum", "mmn_colsum_workspace_bytes", "mmn_layernorm_bwd_workspace_bytes",
            "mmn_linear_supported", "mmn_linear_fwd", "mmn_linear_bwd", "mmn_linear_bwd_supported", "mmn_linear_bwd_workspace_bytes",
            "mmn_cpb_bias_fwd", "mmn_cpb_bias_bwd", "mmn_table_bias_fwd", "mmn_table_bias_bwd", "mmn_layernorm_supported", "mmn_layernorm_fwd", "mmn_layernorm_bwd"]
 
@@ -61,7 +62,7 @@ class WinAttnDesc(C.Structure):
                 ("seed", C.c_uint64), ("offset", C.c_uint64),
                 ("q_row_stride", C.c_int64), ("k_row_stride", C.c_int64), ("v_row_stride", C.c_int64),
                 ("o_row_stride", C.c_int64), ("do_row_stride", C.c_int64), ("dq_row_stride", C.c_int64),
-                ("dk_row_stride", C.c_int64), ("dv_row_stride", C.c_int64)]
+                ("dk_row_stride", C.c_int64), ("dv_row_stride", C.c_int64), ("deterministic", C.c_int32)]
 
 
 class MhaDesc(C.Structure):
@@ -137,6 +138,8 @@ def load() -> C.CDLL:
         lib.mmn_mha_path.argtypes = [C.POINTER(MhaDesc)]
         lib.mmn_winattn_fwd.restype = C.c_int
         lib.mmn_winattn_fwd.argtypes = [C.POINTER(WinAttnDesc), vp, vp, vp, fp, fp, fp, vp, fp, vp, C.c_int, vp]
+        lib.mmn_winattn_bwd_workspace_bytes.restype = C.c_size_t
+        lib.mmn_winattn_bwd_workspace_bytes.argtypes = [C.POINTER(WinAttnDesc)]
         lib.mmn_winattn_bwd.restype = C.c_int
         lib.mmn_winattn_bwd.argtypes = [C.POINTER(WinAttnDesc), vp, vp, vp, fp, fp, fp, vp, fp, vp, vp, vp, vp, fp, fp, fp, fp,
                                         C.c_int, vp]
@@ -147,23 +150,25 @@ def load() -> C.CDLL:
         lib.mmn_mha_avg_weights.restype = C.c_int
         lib.mmn_mha_avg_weights.argtypes = [C.POINTER(MhaDesc), vp, vp, fp, fp, fp, C.c_int, vp]
         lib.mmn_colsum.restype = C.c_int
-        lib.mmn_colsum.argtypes = [vp, C.c_int, C.c_int64, C.c_int32, C.c_int64, fp, C.c_int, vp]
+        lib.mmn_colsum.argtypes = [vp, C.c_int, C.c_int64, C.c_int32, C.c_int64, fp, fp, C.c_int, C.c_int, vp]
+        lib.mmn_colsum_workspace_bytes.restype = C.c_size_t
+        lib.mmn_colsum_workspace_bytes.argtypes = [C.c_int64, C.c_int32]
         lib.mmn_cpb_bias_fwd.restype = C.c_int
         lib.mmn_cpb_bias_fwd.argtypes = [fp, fp, fp, fp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, fp, fp, C.c_int, vp]
         lib.mmn_table_bias_fwd.restype = C.c_int
         lib.mmn_table_bias_fwd.argtypes = [fp, vp, C.c_int32, C.c_int32, C.c_int32, fp, C.c_int, vp]
         lib.mmn_table_bias_bwd.restype = C.c_int
-        lib.mmn_table_bias_bwd.argtypes = [fp, vp, C.c_int32, C.c_int32, C.c_int32, fp, C.c_int, vp]
+        lib.mmn_table_bias_bwd.argtypes = [fp, vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, fp, C.c_int, vp]
         lib.mmn_cpb_bias_bwd.restype = C.c_int
-        lib.mmn_cpb_bias_bwd.argtypes = [fp, fp, fp, fp, vp, fp, fp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+        lib.mmn_cpb_bias_bwd.argtypes = [fp, fp, fp, fp, vp, vp, vp, fp, fp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                          fp, fp, fp, fp, C.c_int, vp]
         lib.mmn_linear_bwd_supported.restype = C.c_int
         lib.mmn_linear_bwd_supported.argtypes = [C.c_int, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int64]
         lib.mmn_linear_bwd_workspace_bytes.restype = C.c_size_t
-        lib.mmn_linear_bwd_workspace_bytes.argtypes = [C.c_int64, C.c_int32, C.c_int32]
+        lib.mmn_linear_bwd_workspace_bytes.argtypes = [C.c_int64, C.c_int32, C.c_int32, C.c_int]
         lib.mmn_linear_bwd.restype = C.c_int
         lib.mmn_linear_bwd.argtypes = [vp, vp, vp, vp, fp, fp, vp, vp, C.c_int64, C.c_int, C.c_int, C.c_int64, C.c_int32, C.c_int32,
-                                       C.c_int64, C.c_int64, C.c_int64, C.c_int, vp]
+                                       C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int, vp]
         lib.mmn_linear_supported.restype = C.c_int
         lib.mmn_linear_supported.argtypes = [C.c_int, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int64]
         lib.mmn_linear_fwd.restype = C.c_int
@@ -176,7 +181,9 @@ def load() -> C.CDLL:
                                           C.c_int64, C.c_int32, C.c_int, vp]
         lib.mmn_layernorm_bwd.restype = C.c_int
         lib.mmn_layernorm_bwd.argtypes = [vp, C.c_int, vp, C.c_int, vp, C.c_int, fp, fp, fp, C.c_int, vp, C.c_int, vp, C.c_int, fp, fp,
-                                          C.c_int64, C.c_int32, C.c_int, vp]
+                                          fp, C.c_int, C.c_int64, C.c_int32, C.c_int, vp]
+        lib.mmn_layernorm_bwd_workspace_bytes.restype = C.c_size_t
+        lib.mmn_layernorm_bwd_workspace_bytes.argtypes = [C.c_int64, C.c_int32]
         if lib.mmn_abi_version() != ABI_VERSION:
             raise RuntimeError("libmmn_b200.so ABI version mismatch")
         _lib = lib

@@ -14,6 +14,8 @@
 // query row; dkv: thread per key row), recomputing probabilities from the saved
 // log-sum-exp; no atomics except the cross-window reductions dbias / dhead_scale.  The
 // backward never reads the forward output: delta = rowsum(P o dP) is recomputed exactly.
+// Deterministic mode passes no reduction outputs to those two kernels and computes them afterwards in a fixed order:
+// attn_bias_grad_generic (dbias, dhead_scale partials) and the column-sum partials below (dcolsum).
 #pragma once
 
 #include <cuda_bf16.h>
@@ -465,6 +467,67 @@ attn_bwd_dkv_generic(GenericProblem P, GenericLaunch L, const T* __restrict__ q,
 }
 
 // ---------------------------------------------------------------------------------------
+// Deterministic mode: dbias and dhead_scale without atomics.  Thread per (h, i, j): walks head h's windows in order and
+// recomputes ds_ij exactly as attn_bwd_dq_generic does (delta and the row normaliser come from delta_ws), adds sum_w ds
+// into dbias[h][i][j] and writes sum_w ds * dot to dsp[(i * nk + j) * nH + h], which reduce_partials turns into
+// dhead_scale.  Window attention (kind 0) only.
+// ---------------------------------------------------------------------------------------
+template <typename T, int DMAX>
+__global__ void __launch_bounds__(kGenericThreads)
+attn_bias_grad_generic(GenericProblem P, const T* __restrict__ q, const T* __restrict__ k, const T* __restrict__ v,
+                       const float* __restrict__ lse, const T* __restrict__ dout, const float* __restrict__ delta_ws,
+                       float* __restrict__ dbias, float* __restrict__ dsp) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (long long)P.nH * P.nq * P.nk) return;
+  const int j = (int)(idx % P.nk);
+  const long long r = idx / P.nk;
+  const int i = (int)(r % P.nq), h = (int)(r / P.nq), d = P.d;
+  const float hscale = P.cosine ? __ldg(P.head_scale + h) : 1.f;
+  float db = 0.f, dsd = 0.f;
+  for (int outer = 0; outer < P.n_items / P.nH; ++outer) {
+    const int item = outer * P.nH + h;
+    int rid_i, rid_j;
+    const long long qo = row_offset(P, item, i, P.q_s0, P.q_s1, &rid_i), doo = row_offset(P, item, i, P.do_s0, P.do_s1, &rid_i);
+    const long long ko = row_offset(P, item, j, P.k_s0, P.k_s1, &rid_j), vo = row_offset(P, item, j, P.v_s0, P.v_s1, &rid_j);
+    float qr[DMAX], kr[DMAX];
+    float qss = 0.f, kss = 0.f;
+#pragma unroll
+    for (int c = 0; c < DMAX; ++c) {
+      qr[c] = c < d ? ldf(q + qo + c) : 0.f;
+      kr[c] = c < d ? ldf(k + ko + c) : 0.f;
+      qss += qr[c] * qr[c];
+    }
+    for (int c = 0; c < d; ++c) kss += kr[c] * kr[c];
+    const float qmul = P.cosine ? inv_norm(qss) : P.scale, kmul = P.cosine ? inv_norm(kss) : 1.f;
+    float dot = 0.f, dp = 0.f;
+#pragma unroll
+    for (int c = 0; c < DMAX; ++c)
+      if (c < d) { dot += (qr[c] * qmul) * (kr[c] * kmul); dp += ldf(dout + doo + c) * ldf(v + vo + c); }
+    const float s = logit(P, item, dot, i, j, rid_i, rid_j, hscale);
+    if (s == -INFINITY) continue;
+    const long long row = (long long)item * P.nq + i;
+    const float p = expf(s - lse[row]) * delta_ws[(long long)P.n_items * P.nq + row];
+    const float ds = p * (dp * keep_scale(P, item, i, j) - delta_ws[row]);
+    db += ds;
+    dsd += ds * dot;
+  }
+  if (dbias) dbias[idx] += db;
+  if (dsp) dsp[((long long)i * P.nk + j) * P.nH + h] = dsd;
+}
+
+// Deterministic column sums, any width: block b sums rows [b * rpb, (b + 1) * rpb) of every column into part[b][c].
+template <typename T>
+__global__ void __launch_bounds__(256)
+colsum_part_any(const T* __restrict__ x, long long rows, int cols, long long row_stride, long long rpb, float* __restrict__ part) {
+  const long long r0 = (long long)blockIdx.x * rpb, r1 = r0 + rpb < rows ? r0 + rpb : rows;
+  for (int c = threadIdx.x; c < cols; c += blockDim.x) {
+    float acc = 0.f;
+    for (long long r = r0; r < r1; ++r) acc += ldf(x + r * row_stride + c);
+    part[(size_t)blockIdx.x * cols + c] = acc;
+  }
+}
+
+// ---------------------------------------------------------------------------------------
 // Head-averaged attention probabilities (multihead_attention.py:131-133): thread per (b,i,j).
 // ---------------------------------------------------------------------------------------
 template <typename T>
@@ -494,10 +557,12 @@ mha_avg_weights_generic(GenericProblem P, int B, const T* __restrict__ q, const 
 // ---------------------------------------------------------------------------------------
 // Column sums of a (rows, cols) matrix into fp32 (accumulated): the bias gradient of a
 // projection, at memory speed.  Thread = 8 consecutive columns; a block strides over rows.
+// part != null (deterministic mode): the block's sums go to part[blockIdx.x][c] instead of atomics into out.
 // ---------------------------------------------------------------------------------------
 template <typename T>
 __global__ void __launch_bounds__(256)
-colsum_kernel(const T* __restrict__ x, long long rows, int cols, long long row_stride, float* __restrict__ out) {
+colsum_kernel(const T* __restrict__ x, long long rows, int cols, long long row_stride, float* __restrict__ out,
+              float* __restrict__ part) {
   constexpr int V = 8;
   const int vcols = cols / V;
   const int rpb = 256 / vcols;                        // rows handled in parallel by a block
@@ -542,7 +607,8 @@ colsum_kernel(const T* __restrict__ x, long long rows, int cols, long long row_s
   for (int c = threadIdx.x; c < vcols * V; c += 256) {   // column (cols may exceed the block size: up to 2048)
     float s = 0.f;
     for (int y = 0; y < rpb; ++y) s += red[(y * vcols + c / V) * V + c % V];
-    atomicAdd(out + c, s);
+    if (part) part[(size_t)blockIdx.x * cols + c] = s;
+    else atomicAdd(out + c, s);
   }
 }
 

@@ -71,11 +71,42 @@ __global__ void cpb_scatter_kernel(const float* __restrict__ dbias, const long l
   for (int h = 0; h < nH; ++h) atomicAdd(dtab16 + t * nH + h, __ldg(dbias + (size_t)h * NN + e));
 }
 
+// Deterministic variant of the scatter: a gather over the inverse of `index` in CSR form (inv_perm = the entries e sorted
+// by (index[e], e), inv_offsets = the run of each table entry).  Thread per (t, h) sums dbias[h][e] over its run in
+// increasing e.  An inverse that does not cover NN entries is not the inverse of this index: the output becomes NaN.
+__global__ void cpb_gather_grad_kernel(const float* __restrict__ dbias, const int* __restrict__ inv_perm, const int* __restrict__ inv_offsets,
+                                       int T, int NN, int nH, float* __restrict__ dtab16) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x;
+  if (x >= T * nH) return;
+  const int t = x / nH, h = x - t * nH;
+  float acc = 0.f;
+  if (__ldg(inv_offsets + T) != NN) {
+    acc = __int_as_float(0x7fffffff);
+  } else {
+    const float* row = dbias + (size_t)h * NN;
+    for (int k = __ldg(inv_offsets + t), k1 = __ldg(inv_offsets + t + 1); k < k1; ++k) acc += __ldg(row + __ldg(inv_perm + k));
+  }
+  dtab16[x] = acc;
+}
+
+// dtab[t][h] = sum over e with index[e] == t of dbias[h][e]: the scatter (after zeroing) or, with the inverse index, the gather
+cudaError_t table_grad(const float* dbias, const long long* index, const int* inv_perm, const int* inv_offsets, int T, int nH, int NN,
+                       float* dtab, cudaStream_t st) {
+  if (inv_perm) {
+    cpb_gather_grad_kernel<<<(T * nH + 255) / 256, 256, 0, st>>>(dbias, inv_perm, inv_offsets, T, NN, nH, dtab);
+    return cudaGetLastError();
+  }
+  cudaError_t e = zero_words_async(dtab, (size_t)T * nH, st);
+  if (e != cudaSuccess) return e;
+  cpb_scatter_kernel<<<(NN + 255) / 256, 256, 0, st>>>(dbias, index, NN, nH, dtab);
+  return cudaGetLastError();
+}
+
 // Backward of the MLP.  A block owns 32 hidden units; its 16 warps split the T table entries (warp w takes
 // t = w, w + 16, ...), every thread recomputes its unit's activation and accumulates dW2[:, j], dW1[j, :], db1[j] for
 // its slice in registers; the 16 slices are then summed through shared memory in a fixed order (this kernel uses no
 // atomics; the scatter of dbias into the table before it, cpb_scatter_kernel, does -- float atomicAdd, so the
-// last bits of the CPB gradients can differ from run to run).  g[t][h] = d tab[t][h] is staged in shared memory eight heads at a time:
+// last bits of the CPB gradients can differ from run to run unless the deterministic gather replaces it).  g[t][h] = d tab[t][h] is staged in shared memory eight heads at a time:
 // d/dx 16 sigmoid(x) = tab16 (1 - tab16 / 16).  (One thread per hidden unit walking all T entries alone -- four blocks
 // on four SMs -- took 58 us at BASELINE cfg2, 4 % of the whole fused-module step.)
 constexpr int kCpbBwdUnits = 32, kCpbBwdSlices = 16;
@@ -175,11 +206,9 @@ cudaError_t table_bias_fwd(const float* table, const long long* index, int nH, i
   return e;
 }
 
-cudaError_t table_bias_bwd(const float* dbias, const long long* index, int T, int nH, int NN, float* dtable, cudaStream_t st, int* launches) {
-  cudaError_t e = zero_words_async(dtable, (size_t)T * nH, st);
-  if (e != cudaSuccess) return e;
-  cpb_scatter_kernel<<<(NN + 255) / 256, 256, 0, st>>>(dbias, index, NN, nH, dtable);
-  e = cudaGetLastError();
+cudaError_t table_bias_bwd(const float* dbias, const long long* index, const int* inv_perm, const int* inv_offsets, int T, int nH, int NN,
+                           float* dtable, cudaStream_t st, int* launches) {
+  cudaError_t e = table_grad(dbias, index, inv_perm, inv_offsets, T, nH, NN, dtable, st);
   if (e == cudaSuccess) *launches += 1;
   return e;
 }
@@ -194,11 +223,10 @@ cudaError_t cpb_bias_fwd(const float* coords, const float* w1, const float* b1, 
 }
 
 cudaError_t cpb_bias_bwd(const float* coords, const float* w1, const float* b1, const float* w2, const long long* index,
-                         const float* tab16, const float* dbias, int T, int n_in, int J, int nH, int NN, float* dtab16, float* dw1,
-                         float* db1, float* dw2, cudaStream_t st, int* launches) {
-  cudaError_t e = zero_words_async(dtab16, (size_t)T * nH, st);
+                         const int* inv_perm, const int* inv_offsets, const float* tab16, const float* dbias, int T, int n_in, int J,
+                         int nH, int NN, float* dtab16, float* dw1, float* db1, float* dw2, cudaStream_t st, int* launches) {
+  cudaError_t e = table_grad(dbias, index, inv_perm, inv_offsets, T, nH, NN, dtab16, st);
   if (e != cudaSuccess) return e;
-  cpb_scatter_kernel<<<(NN + 255) / 256, 256, 0, st>>>(dbias, index, NN, nH, dtab16);
   const size_t smem = cpb_bwd_smem_bytes(T);
   if (smem > 48 * 1024) {      // 2-D windows of 16 (T = 961), 3-D windows of 6 / 7 (T = 1331 / 2197): opt in to large dynamic smem
     static std::once_flag once;

@@ -12,6 +12,8 @@
 // either input may be absent (PRE with delta == null is a plain LayerNorm), either output may be skipped, and every
 // tensor is fp32 or bf16 independently (residual stream fp32, activations bf16 under autocast).  mean / rstd per row are
 // kept for the backward, which returns d resid, d delta and (accumulated with atomics over row blocks) d gamma, d beta.
+// Deterministic mode hands the backward kernels a `part` buffer: block b writes its column sums to part[0 / 1][b][c] (d gamma
+// / d beta) instead, and reduce_partials adds them into the caller's buffers in block order.
 //
 // One warp per row; lane l owns the column pairs 2 (l + 32 k): 4-byte (bf16x2) or 8-byte (float2) accesses, fully
 // coalesced, values stay in registers between the statistics pass and the normalisation pass.  fp32 arithmetic.
@@ -128,7 +130,7 @@ template <int K>
 __global__ void __launch_bounds__(kLnWarps * 32)
 ln_bwd_kernel(LnTensor gs, LnTensor gn, LnTensor x, const float* __restrict__ gamma, const float* __restrict__ mean,
               const float* __restrict__ rstd, int mode, LnOut d_resid, LnOut d_delta, float* __restrict__ dgamma,
-              float* __restrict__ dbeta, long long rows, int cols) {
+              float* __restrict__ dbeta, float* __restrict__ part, long long rows, int cols) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   float2 g[K], ag[K], ab[K];
 #pragma unroll
@@ -196,7 +198,8 @@ ln_bwd_kernel(LnTensor gs, LnTensor gn, LnTensor x, const float* __restrict__ ga
         float s = 0.f;
 #pragma unroll
         for (int w = 0; w < kLnWarps; ++w) s += red[w][threadIdx.x];
-        atomicAdd(dst + c, s);
+        if (part) part[((size_t)pass_id * gridDim.x + blockIdx.x) * cols + c] = s;
+        else atomicAdd(dst + c, s);
       }
       __syncthreads();
     }
@@ -318,7 +321,7 @@ template <int LPR, int V, int MODE, int U>
 __global__ void __launch_bounds__(kLnWarps * 32, V <= 3 ? 3 : 1)
 ln_bwd_v4_kernel(LnTensor gs, LnTensor gn, LnTensor x, const float* __restrict__ gamma, const float* __restrict__ mean,
                  const float* __restrict__ rstd, LnOut d_resid, LnOut d_delta, float* __restrict__ dgamma,
-                 float* __restrict__ dbeta, long long rows, int cols) {
+                 float* __restrict__ dbeta, float* __restrict__ part, long long rows, int cols) {
   constexpr int R = 32 / LPR;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int lr = lane % LPR, sub = lane / LPR;
@@ -418,7 +421,8 @@ ln_bwd_v4_kernel(LnTensor gs, LnTensor gn, LnTensor x, const float* __restrict__
       float s = 0.f;
 #pragma unroll
       for (int w = 0; w < kLnWarps; ++w) s += red[w][c];
-      atomicAdd(dst + c, s);
+      if (part) part[((size_t)pass_id * gridDim.x + blockIdx.x) * cols + c] = s;
+      else atomicAdd(dst + c, s);
     }
     __syncthreads();
   }
@@ -467,6 +471,14 @@ int ln_grid(long long rows) {
   long long want = (rows + kLnWarps - 1) / kLnWarps;
   const long long cap = 148ll * 8;
   return (int)(want < cap ? want : cap);
+}
+
+// blocks the backward launched (both kernels are one-wave grid-stride launches); adds their partials in block order
+cudaError_t ln_reduce(const float* part, int blocks, int cols, float* dgamma, float* dbeta, cudaStream_t st, int* launches) {
+  cudaError_t e = cudaSuccess;
+  if (dgamma) e = reduce_partials(part, blocks, cols, dgamma, st, launches);
+  if (e == cudaSuccess && dbeta) e = reduce_partials(part + (size_t)blocks * cols, blocks, cols, dbeta, st, launches);
+  return e;
 }
 
 }  // namespace
@@ -523,8 +535,10 @@ cudaError_t layernorm_fwd(const void* resid, int resid_dt, const void* delta, in
 
 cudaError_t layernorm_bwd(const void* g_sum, int gs_dt, const void* g_norm, int gn_dt, const void* x, int x_dt, const float* gamma,
                           const float* mean, const float* rstd, int mode, void* d_resid, int dr_dt, void* d_delta, int dd_dt,
-                          float* dgamma, float* dbeta, long long rows, int cols, cudaStream_t st, int* launches) {
+                          float* dgamma, float* dbeta, float* part, long long rows, int cols, cudaStream_t st, int* launches) {
   const int kk = ln_pairs(cols);
+  if (!dgamma && !dbeta) part = nullptr;
+  int blocks = 0;
   LnTensor gs{g_sum, gs_dt}, gn{g_norm, gn_dt}, xx{x, x_dt};
   LnOut dr{d_resid, dr_dt}, dd{d_delta, dd_dt};
   const V4Cfg vc = v4_cfg(cols);
@@ -533,19 +547,28 @@ cudaError_t layernorm_bwd(const void* g_sum, int gs_dt, const void* g_norm, int 
       constexpr int U = 1;                                                                           \
       auto k0 = ln_bwd_v4_kernel<L_, V_, 0, U>;                                                      \
       auto k1 = ln_bwd_v4_kernel<L_, V_, 1, U>;                                                      \
-      if (mode == 0) k0<<<ln_grid_v4(rows, L_, U, resident_blocks((const void*)k0)), kLnWarps * 32, 0, st>>>(gs, gn, xx, gamma, mean, rstd, dr, dd, dgamma, dbeta, rows, cols); \
-      else k1<<<ln_grid_v4(rows, L_, U, resident_blocks((const void*)k1)), kLnWarps * 32, 0, st>>>(gs, gn, xx, gamma, mean, rstd, dr, dd, dgamma, dbeta, rows, cols);           \
+      if (mode == 0) { blocks = ln_grid_v4(rows, L_, U, resident_blocks((const void*)k0)); k0<<<blocks, kLnWarps * 32, 0, st>>>(gs, gn, xx, gamma, mean, rstd, dr, dd, dgamma, dbeta, part, rows, cols); } \
+      else { blocks = ln_grid_v4(rows, L_, U, resident_blocks((const void*)k1)); k1<<<blocks, kLnWarps * 32, 0, st>>>(gs, gn, xx, gamma, mean, rstd, dr, dd, dgamma, dbeta, part, rows, cols); }        \
     }
     MMN_LN_V4(8, 1) MMN_LN_V4(8, 2) MMN_LN_V4(8, 3) MMN_LN_V4(16, 2) MMN_LN_V4(16, 3) MMN_LN_V4(32, 2) MMN_LN_V4(32, 3) MMN_LN_V4(32, 4) MMN_LN_V4(32, 6)
 #undef MMN_LN_V4
     cudaError_t e4 = cudaGetLastError();
-    if (e4 == cudaSuccess) ++*launches;
-    return e4;
+    if (e4 != cudaSuccess) return e4;
+    ++*launches;
+    return part ? ln_reduce(part, blocks, cols, dgamma, dbeta, st, launches) : cudaSuccess;
   }
-  MMN_LN_DISPATCH(kk, (ln_bwd_kernel<K><<<ln_grid(rows), kLnWarps * 32, 0, st>>>(gs, gn, xx, gamma, mean, rstd, mode, dr, dd, dgamma, dbeta, rows, cols)));
+  blocks = ln_grid(rows);
+  MMN_LN_DISPATCH(kk, (ln_bwd_kernel<K><<<blocks, kLnWarps * 32, 0, st>>>(gs, gn, xx, gamma, mean, rstd, mode, dr, dd, dgamma, dbeta, part, rows, cols)));
   cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess) ++*launches;
-  return e;
+  if (e != cudaSuccess) return e;
+  ++*launches;
+  return part ? ln_reduce(part, blocks, cols, dgamma, dbeta, st, launches) : cudaSuccess;
+}
+
+// Either kernel launches at most 148 x 8 blocks (a 256-thread block per 8 rows at least), two rows of partials per block.
+size_t layernorm_bwd_workspace_floats(long long rows, int cols) {
+  const long long want = (rows + kLnWarps - 1) / kLnWarps, blocks = want < 148ll * 8 ? want : 148ll * 8;
+  return (size_t)(blocks > 0 ? blocks : 0) * 2 * cols;
 }
 
 }  // namespace mmn

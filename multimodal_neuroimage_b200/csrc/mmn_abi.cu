@@ -166,6 +166,17 @@ int mmn_winattn_fwd(const mmn_winattn_desc* d, const void* q, const void* k, con
   return finish(e, n, "attn_fwd_generic");
 }
 
+size_t mmn_winattn_bwd_workspace_bytes(const mmn_winattn_desc* d) {
+  if (validate_win(d) != MMN_OK) return 0;
+  const mmn::GenericProblem P = problem_from(d, nullptr, nullptr, nullptr);
+  const size_t base = mmn::generic_bwd_workspace_floats(P, false) * sizeof(float);
+  size_t bytes = base > MMN_WINATTN_WORK_BYTES ? base : MMN_WINATTN_WORK_BYTES;
+  if (!d->deterministic) return bytes;
+  const size_t det = d->path != MMN_PATH_GENERIC && mmn::tc::bwd_why_not(d) == nullptr ? mmn::tc::bwd_det_workspace_bytes(d)
+                                                                                      : mmn::generic_bwd_workspace_floats(P, true) * sizeof(float);
+  return det > bytes ? det : bytes;
+}
+
 int mmn_winattn_bwd(const mmn_winattn_desc* d, const void* q, const void* k, const void* v, const float* bias,
                     const float* head_scale, const float* mask, const void* out, const float* lse, const void* dout,
                     void* dq, void* dk, void* dv, float* dbias, float* dhead_scale, float* dcolsum, float* workspace,
@@ -191,7 +202,7 @@ int mmn_winattn_bwd(const mmn_winattn_desc* d, const void* q, const void* k, con
   mmn::GenericProblem P = problem_from(d, bias, head_scale, mask);
   int n = 0;
   cudaError_t e = mmn::generic_bwd(P, d->io_dtype, q, k, v, lse, dout, dq, dk, dv, bias ? dbias : nullptr,
-                                 P.cosine ? dhead_scale : nullptr, workspace, dcolsum, st, &n);
+                                 P.cosine ? dhead_scale : nullptr, workspace, dcolsum, d->deterministic != 0, st, &n);
   return finish(e, n, "attn_bwd_generic");
 }
 
@@ -235,7 +246,7 @@ int mmn_mha_bwd(const mmn_mha_desc* d, const void* q, const void* k, const void*
     return rc;
   }
   cudaError_t e = mmn::generic_bwd(problem_from(d, mask), d->io_dtype, q, k, v, lse, dout, dq, dk, dv, nullptr, nullptr, workspace,
-                                 nullptr, (cudaStream_t)stream, &n);
+                                 nullptr, false, (cudaStream_t)stream, &n);
   return finish(e, n, "attn_bwd_generic");
 }
 
@@ -252,8 +263,15 @@ int mmn_mha_avg_weights(const mmn_mha_desc* d, const void* q, const void* k, con
   return finish(e, n, "mha_avg_weights_generic");
 }
 
-int mmn_colsum(const void* x, int io_dtype, int64_t rows, int32_t cols, int64_t row_stride, float* out, int device, void* stream) {
+size_t mmn_colsum_workspace_bytes(int64_t rows, int32_t cols) {
+  if (rows < 1 || cols < 8 || cols % 8 != 0 || cols > 2048) return 0;
+  return mmn::colsum_workspace_floats(rows, cols) * sizeof(float);
+}
+
+int mmn_colsum(const void* x, int io_dtype, int64_t rows, int32_t cols, int64_t row_stride, float* out, float* workspace,
+               int deterministic, int device, void* stream) {
   if (!x || !out || rows < 0 || cols < 1) return fail(MMN_ERR_INVALID, "bad colsum arguments");
+  if (deterministic && !workspace) return fail(MMN_ERR_INVALID, "deterministic colsum needs a workspace");
   if (io_dtype != MMN_DT_F32 && io_dtype != MMN_DT_BF16) return fail(MMN_ERR_INVALID, "bad io_dtype");
   if (cols % 8 != 0 || cols > 2048) return fail(MMN_ERR_UNSUPPORTED, "colsum needs cols %% 8 == 0 and cols <= 2048 (got %d)", cols);
   if (!have_device()) return fail(MMN_ERR_CUDA, "no CUDA device: libmmn_b200 has no CPU path");
@@ -261,7 +279,7 @@ int mmn_colsum(const void* x, int io_dtype, int64_t rows, int32_t cols, int64_t 
   if (!g.ok) return fail(MMN_ERR_CUDA, "cannot select device %d", device);
   if (rows == 0) return MMN_OK;
   int n = 0;
-  cudaError_t e = mmn::colsum(io_dtype, x, rows, cols, row_stride, out, (cudaStream_t)stream, &n);
+  cudaError_t e = mmn::colsum(io_dtype, x, rows, cols, row_stride, out, deterministic ? workspace : nullptr, (cudaStream_t)stream, &n);
   return finish(e, n, "colsum_kernel");
 }
 
@@ -284,14 +302,16 @@ int mmn_table_bias_fwd(const float* table, const int64_t* index, int32_t T, int3
   return finish(e, n, "table_bias_fwd");
 }
 
-int mmn_table_bias_bwd(const float* dbias, const int64_t* index, int32_t T, int32_t nH, int32_t NN, float* dtable, int device, void* stream) {
+int mmn_table_bias_bwd(const float* dbias, const int64_t* index, const int32_t* inv_perm, const int32_t* inv_offsets, int32_t T, int32_t nH,
+                       int32_t NN, float* dtable, int device, void* stream) {
   if (!dbias || !index || !dtable) return fail(MMN_ERR_INVALID, "null tensor pointer");
+  if (!inv_perm != !inv_offsets) return fail(MMN_ERR_INVALID, "inv_perm and inv_offsets go together");
   if (T < 1 || nH < 1 || NN < 1) return fail(MMN_ERR_INVALID, "bad bias table dimensions");
   if (!have_device()) return fail(MMN_ERR_CUDA, "no CUDA device: libmmn_b200 has no CPU path");
   DeviceGuard g(device);
   if (!g.ok) return fail(MMN_ERR_CUDA, "cannot select device %d", device);
   int n = 0;
-  cudaError_t e = mmn::table_bias_bwd(dbias, (const long long*)index, T, nH, NN, dtable, (cudaStream_t)stream, &n);
+  cudaError_t e = mmn::table_bias_bwd(dbias, (const long long*)index, inv_perm, inv_offsets, T, nH, NN, dtable, (cudaStream_t)stream, &n);
   return finish(e, n, "table_bias_bwd");
 }
 
@@ -308,17 +328,19 @@ int mmn_cpb_bias_fwd(const float* coords, const float* w1, const float* b1, cons
 }
 
 int mmn_cpb_bias_bwd(const float* coords, const float* w1, const float* b1, const float* w2, const int64_t* index,
+                     const int32_t* inv_perm, const int32_t* inv_offsets,
                      const float* tab16, const float* dbias, int32_t T, int32_t n_in, int32_t J, int32_t nH, int32_t NN,
                      float* scratch, float* dw1, float* db1, float* dw2, int device, void* stream) {
   if (!coords || !w1 || !b1 || !w2 || !index || !tab16 || !dbias || !scratch || !dw1 || !db1 || !dw2)
     return fail(MMN_ERR_INVALID, "null tensor pointer");
+  if (!inv_perm != !inv_offsets) return fail(MMN_ERR_INVALID, "inv_perm and inv_offsets go together");
   int rc = cpb_check(T, n_in, J, nH, NN);
   if (rc) return rc;
   DeviceGuard g(device);
   if (!g.ok) return fail(MMN_ERR_CUDA, "cannot select device %d", device);
   int n = 0;
-  cudaError_t e = mmn::cpb_bias_bwd(coords, w1, b1, w2, (const long long*)index, tab16, dbias, T, n_in, J, nH, NN, scratch, dw1, db1,
-                                    dw2, (cudaStream_t)stream, &n);
+  cudaError_t e = mmn::cpb_bias_bwd(coords, w1, b1, w2, (const long long*)index, inv_perm, inv_offsets, tab16, dbias, T, n_in, J, nH, NN,
+                                    scratch, dw1, db1, dw2, (cudaStream_t)stream, &n);
   return finish(e, n, "cpb_bias_bwd");
 }
 
@@ -356,15 +378,22 @@ int mmn_linear_bwd_supported(int io_dtype, int64_t rows, int32_t in_features, in
   return mmn::tc::linear_why_not(io_dtype, rows, in_features, out_features, ld_x, ld_dy) == nullptr && ld_dx % 8 == 0;
 }
 
-size_t mmn_linear_bwd_workspace_bytes(int64_t rows, int32_t in_features, int32_t out_features) {
+// Deterministic mode reuses the workspace for db's column-sum partials once the weight gradient (stream-ordered before them)
+// is done with it.
+size_t mmn_linear_bwd_workspace_bytes(int64_t rows, int32_t in_features, int32_t out_features, int deterministic) {
   const size_t a = mmn::tc::linbwd_workspace_bytes(out_features);
   const size_t b = mmn::tc::linear_wgrad_workspace_bytes(rows, in_features, out_features);
-  return a > b ? a : b;
+  size_t bytes = a > b ? a : b;
+  if (deterministic && rows > 0 && out_features >= 8) {
+    const size_t c = mmn::colsum_workspace_floats(rows, out_features < 2048 ? out_features : 2048) * sizeof(float);
+    if (c > bytes) bytes = c;
+  }
+  return bytes;
 }
 
 int mmn_linear_bwd(const void* dy, const void* x, const void* w, void* dx, float* dw, float* db, void* workspace,
                    const void* act_aux, int64_t ld_aux, int act, int io_dtype, int64_t rows, int32_t in_features,
-                   int32_t out_features, int64_t ld_dy, int64_t ld_x, int64_t ld_dx, int device, void* stream) {
+                   int32_t out_features, int64_t ld_dy, int64_t ld_x, int64_t ld_dx, int deterministic, int device, void* stream) {
   if (!dy || !w || !workspace || (!dx && !dw)) return fail(MMN_ERR_INVALID, "null tensor pointer");
   if (dw && !x) return fail(MMN_ERR_INVALID, "dw needs x");
   if (act != MMN_ACT_NONE && act != MMN_ACT_RELU && act != MMN_ACT_GELU) return fail(MMN_ERR_INVALID, "bad activation %d", act);
@@ -389,7 +418,7 @@ int mmn_linear_bwd(const void* dy, const void* x, const void* w, void* dx, float
       cudaError_t e = mmn::zero_words_async(db, (size_t)out_features, st);
       for (int c0 = 0; e == cudaSuccess && c0 < out_features; c0 += 2048)
         e = mmn::colsum(MMN_DT_BF16, static_cast<const uint16_t*>(dy) + c0, rows, out_features - c0 < 2048 ? out_features - c0 : 2048, ld_dy,
-                        db + c0, st, &n);
+                        db + c0, deterministic ? static_cast<float*>(workspace) : nullptr, st, &n);
       if (e != cudaSuccess) { g_launches.fetch_add((uint64_t)n, std::memory_order_relaxed); return finish(e, 0, "colsum_kernel"); }
     }
   }
@@ -420,10 +449,17 @@ int mmn_layernorm_fwd(const void* resid, int resid_dtype, const void* delta, int
   return finish(e, n, "ln_fwd_kernel");
 }
 
+size_t mmn_layernorm_bwd_workspace_bytes(int64_t rows, int32_t cols) {
+  if (rows < 1 || !mmn::layernorm_supported(cols)) return 0;
+  return mmn::layernorm_bwd_workspace_floats(rows, cols) * sizeof(float);
+}
+
 int mmn_layernorm_bwd(const void* g_sum, int gs_dtype, const void* g_norm, int gn_dtype, const void* x, int x_dtype, const float* gamma,
                       const float* mean, const float* rstd, int mode, void* d_resid, int dr_dtype, void* d_delta, int dd_dtype,
-                      float* dgamma, float* dbeta, int64_t rows, int32_t cols, int device, void* stream) {
+                      float* dgamma, float* dbeta, float* workspace, int deterministic, int64_t rows, int32_t cols, int device,
+                      void* stream) {
   if ((!g_sum && !g_norm) || !x || !gamma || !mean || !rstd) return fail(MMN_ERR_INVALID, "null tensor pointer");
+  if (deterministic && (dgamma || dbeta) && !workspace) return fail(MMN_ERR_INVALID, "deterministic layernorm backward needs a workspace");
   if (mode != MMN_LN_PRE && mode != MMN_LN_POST) return fail(MMN_ERR_INVALID, "bad layernorm mode %d", mode);
   if (!ln_dt_ok(gs_dtype) || !ln_dt_ok(gn_dtype) || !ln_dt_ok(x_dtype) || !ln_dt_ok(dr_dtype) || !ln_dt_ok(dd_dtype)) return fail(MMN_ERR_INVALID, "bad dtype");
   if (!mmn::layernorm_supported(cols)) return fail(MMN_ERR_UNSUPPORTED, "layernorm: cols = %d (even, <= 1536)", cols);
@@ -433,7 +469,7 @@ int mmn_layernorm_bwd(const void* g_sum, int gs_dtype, const void* g_norm, int g
   if (rows <= 0) return MMN_OK;
   int n = 0;
   cudaError_t e = mmn::layernorm_bwd(g_sum, gs_dtype, g_norm, gn_dtype, x, x_dtype, gamma, mean, rstd, mode, d_resid, dr_dtype, d_delta,
-                                     dd_dtype, dgamma, dbeta, rows, cols, (cudaStream_t)stream, &n);
+                                     dd_dtype, dgamma, dbeta, deterministic ? workspace : nullptr, rows, cols, (cudaStream_t)stream, &n);
   return finish(e, n, "ln_bwd_kernel");
 }
 

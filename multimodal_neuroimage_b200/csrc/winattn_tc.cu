@@ -82,9 +82,10 @@ int winattn_bwd(const mmn_winattn_desc* d, const void* q, const void* k, const v
                 const float* head_scale, const float* mask, const void* /*out*/, const float* lse, const void* dout, void* dq,
                 void* dk, void* dv, float* dbias, float* dhead_scale, float* dcolsum, float* workspace, cudaStream_t st,
                 char* err, size_t errlen, int* launches) {
-  int rc = winattn_bwd_launch(d, q, k, v, bias, head_scale, mask, lse, dout, dq, dk, dv, dbias, dhead_scale, dcolsum, workspace, st, err, errlen);
-  if (rc == MMN_OK) ++*launches;
-  return rc;
+  return winattn_bwd_launch(d, q, k, v, bias, head_scale, mask, lse, dout, dq, dk, dv, dbias, dhead_scale, dcolsum, workspace, st, err, errlen,
+                            launches);
 }
+
+size_t bwd_det_workspace_bytes(const mmn_winattn_desc* d) { return bwd_det_workspace_bytes_impl(d); }
 
 }}  // namespace mmn::tc

@@ -16,6 +16,8 @@ int winattn_bwd(const mmn_winattn_desc* d, const void* q, const void* k, const v
                 const float* head_scale, const float* mask, const void* out, const float* lse, const void* dout, void* dq,
                 void* dk, void* dv, float* dbias, float* dhead_scale, float* dcolsum, float* workspace, cudaStream_t st,
                 char* err, size_t errlen, int* launches);
+// workspace of the deterministic backward (desc->deterministic != 0): one slot of partial sums per CTA
+size_t bwd_det_workspace_bytes(const mmn_winattn_desc* d);
 // fused projection backward (linbwd_tc.cu)
 const char* linbwd_why_not(int io_dtype, long long rows, int in_features, int out_features, long long ld_dy, long long ld_x, long long ld_dx);
 size_t linbwd_workspace_bytes(int out_features);

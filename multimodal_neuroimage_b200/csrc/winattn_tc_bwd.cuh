@@ -73,11 +73,18 @@ struct BwdParams {
   float* dhead_scale;   // (nH) accumulated, may be null
   float* dcolsum;       // (3, nH*32) accumulated column sums of dq, dk, dv (= projection bias grads), may be null
   int* work;            // dynamic schedule counters (winattn_tc_fwd.cuh: arm_work_counters)
+  float* part;          // deterministic kernels: per-CTA partial sums, kDetSlotFloats per CTA (winattn_bwd_det_reduce)
   TraceCfg trace;       // debug: clock64 stamps of one CTA (MMN_TC_TRACE_BWD=<file>)
 };
 
 
-template <bool COS, int MASK>
+// Deterministic kernels (DET): CTA k of head h walks the static cost-balanced item range k of the head instead of the
+// run-time queue, and its dbias / dcolsum / dhead_scale sums go to a slot of the workspace that only it writes, in program
+// order; winattn_bwd_det_reduce then adds the slots of a head in CTA order.  Every slot entry that is read is written:
+// the dbias region by the first flush (or zeros when the CTA had no item), the others once at the end.
+constexpr int kDetColsum = kN * kN, kDetHscale = kN * kN + 3 * kD, kDetSlotFloats = kN * kN + 3 * kD + 4;
+
+template <bool COS, int MASK, bool DET>
 __global__ void __launch_bounds__(kBwdThreads, 1)
 winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
   extern __shared__ uint8_t smem_raw[];
@@ -118,6 +125,7 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
   const Sched& sc = P.sc;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int h = blockIdx.x % P.nH;
+  float* const det_slot = DET ? P.part + (size_t)(h * P.per_head + blockIdx.x / P.nH) * kDetSlotFloats : nullptr;
 
   // ---- one-time setup
   for (int i = tid; i < (kStagesB * kStageBytesB + kPDBytes) / 16; i += kBwdThreads)
@@ -165,34 +173,47 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
       // (An L2 prefetch of item n + 1's boxes issued right after item n's loads made the kernel 33 % SLOWER, 0.46 -> 0.61 ms:
       // the extra boxes queue in the SM's TMA unit in front of the next loads and the gradient stores.)
       int n = 0;
-      ClassQueue wq;
-      wq.init(sc, sched_range_begin(sc, blockIdx.x / P.nH, P.per_head), P.work + h * 8, kChunkB, lane);
-      for (int c0, m; wq.next(sc, P.work + h * 8, kChunkB, lane, c0, m);) {
+      // one item: descriptor ring (sItem is published by the arrival on full[stage]), tiles, and per slot (lane = slot)
+      // the window's record of norms and lse, already in tile row order.  The same in both schedules.
+#define MMN_BWD_LOAD_ITEM(cur)                                                                                           \
+  do {                                                                                                                 \
+    const int stage = n % kStagesB, phase = (n / kStagesB) & 1;                                                       \
+    if ((cur).cls != plan.cls) plan.build(S, (cur).cls, lane, maps, dst_base, slot_stride);                           \
+    const int nvalid = (cur).slot_valid(1) ? 2 : 1;                                                                   \
+    int w0, w1;                                                                                                       \
+    const WinStart ws0 = cursor_start(S, cur, 0, w0), ws1 = cursor_start(S, cur, 1, w1);                              \
+    trace_ev(P.trace, 2, n, 0);                                                                                       \
+    mbar_wait(&empty[stage], phase ^ 1);                                                                              \
+    trace_ev(P.trace, 2, n, 1);                                                                                       \
+    if (lane == 0) {                                                                                                  \
+      sItem[n & 7] = make_int4((cur).cls, w0, w1, nvalid);                                                          \
+      sGeo[(n & 7) * 2] = make_int4(ws0.b, ws0.s0, ws0.s1, ws0.s2);                                                   \
+      sGeo[(n & 7) * 2 + 1] = make_int4(ws1.b, ws1.s0, ws1.s1, ws1.s2);                                               \
+      mbar_arrive_expect_tx(&full[stage], nvalid * (4 * kWinBytes + 3 * kN * 4));                                     \
+    }                                                                                                                 \
+    __syncwarp();                                                                                                     \
+    plan.issue<true>(S, ws0, ws1, nvalid, h * kD, sStage + stage * kStageBytesB, &full[stage], lane);                 \
+    if (lane < nvalid)                                                                                                \
+      bulk_load_1d(sRec + (stage * 2 + lane) * (3 * kN), P.lse + P.slab + ((long long)(lane ? w1 : w0) * P.nH + h) * (3 * kN),\
+                   3 * kN * 4, &full[stage]);                                                                         \
+    trace_ev(P.trace, 2, n, 2);                                                                                       \
+  } while (0)
+      if (DET) {
+        const int k = blockIdx.x / P.nH, end = sched_range_begin(sc, k + 1, P.per_head);
+        int it = sched_range_begin(sc, k, P.per_head);
         ItemCursor cur;
-        cur.seek(sc, c0);
-        for (int t = 0; t < m; ++t, ++n, cur.next_item(sc)) {
-          const int stage = n % kStagesB, phase = (n / kStagesB) & 1;
-          if (cur.cls != plan.cls) plan.build(S, cur.cls, lane, maps, dst_base, slot_stride);
-          const int nvalid = cur.slot_valid(1) ? 2 : 1;
-          int w0, w1;
-          const WinStart ws0 = cursor_start(S, cur, 0, w0), ws1 = cursor_start(S, cur, 1, w1);
-          trace_ev(P.trace, 2, n, 0);
-          mbar_wait(&empty[stage], phase ^ 1);
-          trace_ev(P.trace, 2, n, 1);
-          if (lane == 0) {
-            sItem[n & 7] = make_int4(cur.cls, w0, w1, nvalid);          // published by the arrival below
-            sGeo[(n & 7) * 2] = make_int4(ws0.b, ws0.s0, ws0.s1, ws0.s2);
-            sGeo[(n & 7) * 2 + 1] = make_int4(ws1.b, ws1.s0, ws1.s1, ws1.s2);
-            mbar_arrive_expect_tx(&full[stage], nvalid * (4 * kWinBytes + 3 * kN * 4));
-          }
-          __syncwarp();
-          plan.issue<true>(S, ws0, ws1, nvalid, h * kD, sStage + stage * kStageBytesB, &full[stage], lane);
-          if (lane < nvalid)                   // lane = slot: the window's record (norms and lse, already in tile row order)
-            bulk_load_1d(sRec + (stage * 2 + lane) * (3 * kN), P.lse + P.slab + ((long long)(lane ? w1 : w0) * P.nH + h) * (3 * kN),
-                         3 * kN * 4, &full[stage]);
-          trace_ev(P.trace, 2, n, 2);
+        cur.seek(sc, it);
+        for (; it < end; ++it, ++n, cur.next_item(sc)) MMN_BWD_LOAD_ITEM(cur);
+      } else {
+        ClassQueue wq;
+        wq.init(sc, sched_range_begin(sc, blockIdx.x / P.nH, P.per_head), P.work + h * 8, kChunkB, lane);
+        for (int c0, m; wq.next(sc, P.work + h * 8, kChunkB, lane, c0, m);) {
+          ItemCursor cur;
+          cur.seek(sc, c0);
+          for (int t = 0; t < m; ++t, ++n, cur.next_item(sc)) MMN_BWD_LOAD_ITEM(cur);
         }
       }
+#undef MMN_BWD_LOAD_ITEM
       {   // end marker
         const int stage = n % kStagesB, phase = (n / kStagesB) & 1;
         mbar_wait(&empty[stage], phase ^ 1);
@@ -359,7 +380,10 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
           v += __shfl_xor_sync(0xffffffffu, v, 4);
           v += __shfl_xor_sync(0xffffffffu, v, 8);
           v += __shfl_xor_sync(0xffffffffu, v, 16);
-          if (lane < 4) atomicAdd(P.dcolsum + t * C + h * kD + cg * 8 + e, v);
+          if (lane < 4) {
+            if (DET) det_slot[kDetColsum + t * kD + cg * 8 + e] = v;
+            else atomicAdd(P.dcolsum + t * C + h * kD + cg * 8 + e, v);
+          }
         }
     }
   } else if (warp >= kEpiWarp0) {
@@ -461,7 +485,10 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
     if (COS && P.dhead_scale) {                          // d s_ij / d(logit scale) = cos_ij = (s_ij - bias_ij) / logit scale
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) dscale_acc += __shfl_xor_sync(0xffffffffu, dscale_acc, o);
-      if (lane == 0) atomicAdd(P.dhead_scale + h, dscale_acc * inv_hscale);
+      if (lane == 0) {
+        if (DET) det_slot[kDetHscale + (warp - kEpiWarp0)] = dscale_acc * inv_hscale;
+        else atomicAdd(P.dhead_scale + h, dscale_acc * inv_hscale);
+      }
     }
   } else {
     // ============================== softmax (512 threads: 4 per row, 16 keys each) ==============================
@@ -479,6 +506,7 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
 #pragma unroll
     for (int j = 0; j < KP; ++j) dbacc[j] = 0.f;
     const int trole = warp == 0 ? 0 : -1;
+    bool det_flushed = false;                           // DET: this CTA's dbias slot has been written once
 #define TRB(item, ev) do { if (trole >= 0) trace_ev(P.trace, trole, item, ev); } while (0)
 
     // dbias of a wrap class leaves the CTA through the (idle at that moment) table buffer: the two windows of the tile
@@ -507,8 +535,14 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
       const uint8_t* pos = sPos + cls * 64;
       for (int e = tid; e < kN * kN; e += kSoftmaxThreadsB) {
         const int ti = e >> 6, tj = e & 63;
-        atomicAdd(gdb_head + (int)pos[ti] * kN + pos[tj], sTbl[ti * kTblLd + tj]);
+        if (DET) {                                      // pos is a permutation: the flush covers the whole slot
+          float* dst = det_slot + (int)pos[ti] * kN + pos[tj];
+          *dst = (det_flushed ? *dst : 0.f) + sTbl[ti * kTblLd + tj];
+        } else {
+          atomicAdd(gdb_head + (int)pos[ti] * kN + pos[tj], sTbl[ti * kTblLd + tj]);
+        }
       }
+      det_flushed = true;
     };
 
     // Everything an item needs besides its logits -- descriptor, this row's lse, the q / k norms -- arrives in shared
@@ -647,6 +681,8 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
     if (gdb_head && cls_loaded >= 0) {
       named_bar_sync(3, kSoftmaxThreadsB);              // everyone is done reading the table
       flush_dbias(cls_loaded);
+    } else if (DET && gdb_head) {                       // no item: the slot still enters the reduction
+      for (int e = tid; e < kN * kN; e += kSoftmaxThreadsB) det_slot[e] = 0.f;
     }
   }
 
@@ -659,6 +695,67 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
 constexpr size_t kBwdSmemBytes = 1024 + kStagesB * kStageBytesB + kPDBytes + 3 * kTile + kN * kTblLd * 4 +
                                  (kStagesB * 2 * 3 * kN + 512 + 16) * 4 + 1024 + 24 * 16 + 16 + 24 * 8;
 
+// Deterministic mode, second launch: for each head, the per_head slots of its CTAs summed in CTA order and added into dbias,
+// dcolsum and dhead_scale (each may be null).  Block = 128 slot entries (one float4 per lane) x 32 slices of the CTA range,
+// as gemm_reduce_kernel: pure latency, at most ceil(per_head / 32) loads per thread; fixed summation order.
+constexpr int kDetRedSlices = 32;
+__global__ void __launch_bounds__(kDetRedSlices * 32)
+winattn_bwd_det_reduce(const float* __restrict__ part, int per_head, int nH, float* __restrict__ dbias, float* __restrict__ dcolsum,
+                       float* __restrict__ dhead_scale) {
+  __shared__ float4 red[kDetRedSlices][32];
+  const int lane = threadIdx.x & 31, sl = threadIdx.x >> 5, h = blockIdx.y;
+  const int e = (blockIdx.x * 32 + lane) * 4;
+  const float* base = part + (size_t)h * per_head * kDetSlotFloats;
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (e < kDetSlotFloats) {
+#pragma unroll 4
+    for (int k = sl; k < per_head; k += kDetRedSlices) {
+      const float4 v = __ldg(reinterpret_cast<const float4*>(base + (size_t)k * kDetSlotFloats + e));
+      acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+    }
+  }
+  red[sl][lane] = acc;
+  __syncthreads();
+  if (sl < 4) {
+    acc = red[8 * sl][lane];
+#pragma unroll
+    for (int k = 1; k < 8; ++k) { const float4 v = red[8 * sl + k][lane]; acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w; }
+    red[8 * sl][lane] = acc;
+  }
+  __syncthreads();
+  if (sl != 0 || e >= kDetSlotFloats) return;
+#pragma unroll
+  for (int k = 1; k < 4; ++k) { const float4 v = red[8 * k][lane]; acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w; }
+  if (e < kDetColsum) {
+    if (dbias) {
+      float4* o = reinterpret_cast<float4*>(dbias + (size_t)h * kN * kN + e);
+      float4 r = *o;
+      r.x += acc.x; r.y += acc.y; r.z += acc.z; r.w += acc.w;
+      *o = r;
+    }
+  } else if (e < kDetHscale) {
+    if (dcolsum) {
+      const int t = (e - kDetColsum) / kD, c = (e - kDetColsum) % kD;
+      float* o = dcolsum + (size_t)t * nH * kD + h * kD + c;
+      o[0] += acc.x; o[1] += acc.y; o[2] += acc.z; o[3] += acc.w;
+    }
+  } else if (dhead_scale) {                                      // the four epilogue warps' sums
+    dhead_scale[h] += (acc.x + acc.y) + (acc.z + acc.w);
+  }
+}
+
+// CTAs per head of the backward launch (one CTA per SM over all heads, at least one per head, at most one per item).
+inline int bwd_ctas_per_head(const WinShape& S, const mmn_winattn_desc* d) {
+  int per_head = num_sms_cached() / d->num_heads;
+  if (per_head < 1) per_head = 1;
+  const int n_items = make_sched(S, d->batch, true).n_items;
+  return per_head > n_items ? n_items : per_head;
+}
+
+inline size_t bwd_det_workspace_bytes_impl(const mmn_winattn_desc* d) {
+  return (size_t)bwd_ctas_per_head(shape_from(d), d) * d->num_heads * kDetSlotFloats * sizeof(float);
+}
+
 inline const char* bwd_why_not_impl(const mmn_winattn_desc* d) {
   const char* w = fwd_why_not_impl(d);
   if (w) return w;
@@ -668,7 +765,8 @@ inline const char* bwd_why_not_impl(const mmn_winattn_desc* d) {
 
 inline int winattn_bwd_launch(const mmn_winattn_desc* d, const void* q, const void* k, const void* v, const float* bias,
                               const float* head_scale, const float* mask, const float* lse, const void* dout, void* dq, void* dk,
-                              void* dv, float* dbias, float* dhead_scale, float* dcolsum, void* workspace, cudaStream_t st, char* err, size_t errlen) {
+                              void* dv, float* dbias, float* dhead_scale, float* dcolsum, void* workspace, cudaStream_t st, char* err, size_t errlen,
+                              int* launches) {
   BwdParams P;
   P.S = shape_from(d);
   P.sc = make_sched(P.S, d->batch, true);
@@ -689,30 +787,49 @@ inline int winattn_bwd_launch(const mmn_winattn_desc* d, const void* q, const vo
   P.dbias = bias ? dbias : nullptr;
   P.dhead_scale = d->score_kind == MMN_SCORE_COSINE ? dhead_scale : nullptr;
   P.dcolsum = dcolsum;
-  P.work = arm_work_counters(workspace, st, err, errlen);
-  if (!P.work) return MMN_ERR_CUDA;
+  const bool det = d->deterministic != 0;
+  P.work = nullptr;
+  P.part = nullptr;
+  if (det) {                                           // static schedule: no counters; the workspace holds the CTA slots
+    if (!workspace || reinterpret_cast<uintptr_t>(workspace) % 16) { snprintf(err, errlen, "workspace missing or misaligned"); return MMN_ERR_CUDA; }
+    P.part = static_cast<float*>(workspace);
+  } else {
+    P.work = arm_work_counters(workspace, st, err, errlen);
+    if (!P.work) return MMN_ERR_CUDA;
+  }
   const char* trace_path = getenv("MMN_TC_TRACE_BWD");
   P.trace = trace_setup(trace_path, st);
 
   using Kern = void (*)(const BwdParams);
-  static const Kern kernels[2][3] = {
-      {winattn_bwd_tc_kernel<false, MMN_MASK_NONE>, winattn_bwd_tc_kernel<false, MMN_MASK_SHIFT>, winattn_bwd_tc_kernel<false, MMN_MASK_TENSOR>},
-      {winattn_bwd_tc_kernel<true, MMN_MASK_NONE>, winattn_bwd_tc_kernel<true, MMN_MASK_SHIFT>, winattn_bwd_tc_kernel<true, MMN_MASK_TENSOR>}};
+  static const Kern kernels[2][2][3] = {
+      {{winattn_bwd_tc_kernel<false, MMN_MASK_NONE, false>, winattn_bwd_tc_kernel<false, MMN_MASK_SHIFT, false>, winattn_bwd_tc_kernel<false, MMN_MASK_TENSOR, false>},
+       {winattn_bwd_tc_kernel<true, MMN_MASK_NONE, false>, winattn_bwd_tc_kernel<true, MMN_MASK_SHIFT, false>, winattn_bwd_tc_kernel<true, MMN_MASK_TENSOR, false>}},
+      {{winattn_bwd_tc_kernel<false, MMN_MASK_NONE, true>, winattn_bwd_tc_kernel<false, MMN_MASK_SHIFT, true>, winattn_bwd_tc_kernel<false, MMN_MASK_TENSOR, true>},
+       {winattn_bwd_tc_kernel<true, MMN_MASK_NONE, true>, winattn_bwd_tc_kernel<true, MMN_MASK_SHIFT, true>, winattn_bwd_tc_kernel<true, MMN_MASK_TENSOR, true>}}};
   static std::once_flag once;
   std::call_once(once, [] {
-    for (int c = 0; c < 2; ++c)
-      for (int m = 0; m < 3; ++m) cudaFuncSetAttribute(kernels[c][m], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmemBytes);
+    for (int t = 0; t < 2; ++t)
+      for (int c = 0; c < 2; ++c)
+        for (int m = 0; m < 3; ++m) cudaFuncSetAttribute(kernels[t][c][m], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmemBytes);
   });
-  const Kern kern = kernels[d->score_kind == MMN_SCORE_COSINE ? 1 : 0][d->mask_kind];
-  int per_head = num_sms_cached() / P.nH;
-  if (per_head < 1) per_head = 1;
-  if (per_head > P.sc.n_items) per_head = P.sc.n_items;
-  P.per_head = per_head;
-  kern<<<per_head * P.nH, kBwdThreads, kBwdSmemBytes, st>>>(P);
+  const Kern kern = kernels[det ? 1 : 0][d->score_kind == MMN_SCORE_COSINE ? 1 : 0][d->mask_kind];
+  P.per_head = bwd_ctas_per_head(P.S, d);
+  kern<<<P.per_head * P.nH, kBwdThreads, kBwdSmemBytes, st>>>(P);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {
     snprintf(err, errlen, "winattn_bwd_tc_kernel: %s", cudaGetErrorString(e));
     return MMN_ERR_CUDA;
+  }
+  ++*launches;
+  if (det && (P.dbias || P.dhead_scale || P.dcolsum)) {
+    winattn_bwd_det_reduce<<<dim3((kDetSlotFloats / 4 + 31) / 32, P.nH), kDetRedSlices * 32, 0, st>>>(P.part, P.per_head, P.nH, P.dbias,
+                                                                                                    P.dcolsum, P.dhead_scale);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) {
+      snprintf(err, errlen, "winattn_bwd_det_reduce: %s", cudaGetErrorString(e));
+      return MMN_ERR_CUDA;
+    }
+    ++*launches;
   }
   if (P.trace.buf) dump_trace(P.trace.buf, trace_path, st);
   return MMN_OK;

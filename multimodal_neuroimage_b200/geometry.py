@@ -97,6 +97,16 @@ def relative_position_index(window: Sequence[int]) -> torch.Tensor:
     return idx
 
 
+def inverse_index(index: torch.Tensor, table_rows: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Inverse of a (NN,) bias-table index in CSR form, on the index's device: (perm, offsets) int32 with perm = the entries
+    e sorted by (index[e], e) and offsets (table_rows + 1) the start of each table entry's run, offsets[-1] = NN.  What the
+    deterministic table-gradient gather walks (csrc/cpb_bias.cu: each entry sums its dbias values in increasing e)."""
+    index = index.reshape(-1)
+    srt, perm = torch.sort(index, stable=True)
+    offsets = torch.searchsorted(srt, torch.arange(table_rows + 1, dtype=index.dtype, device=index.device))
+    return perm.to(torch.int32), offsets.to(torch.int32)
+
+
 def cpb_coords_table(window: Sequence[int], pretrained_window: Optional[Sequence[int]] = None) -> torch.Tensor:
     """(1, 2w_0-1, ..., n) fp32: sign(x)*log2(|x|+1)/log2(8) of 8*delta/(w-1)."""
     window = tuple(int(w) for w in window)

@@ -7,6 +7,10 @@ graph; the arithmetic happens in libmmn_b200.so.  Ops:
   mmn_b200::mha_fwd / mha_bwd           (T,B,E) multi-head attention core
   mmn_b200::mha_avg_weights             head-averaged probabilities
 
+Under `torch.use_deterministic_algorithms(True)` the backward ops select the library's deterministic kernels (fixed-order
+reductions instead of float atomics), as PyTorch's own ops do; the flag is read when the op runs, so a CUDA graph
+captured with it on replays them.
+
 Window attention takes its q/k/v in one of two packings so that the backward can write one
 packed gradient tensor (no slice-backward copies):
   a = qkv (..., 3C), b = None            self attention   (swin_v2 / swinfusion self)
@@ -20,7 +24,7 @@ from typing import List, Optional, Tuple
 
 import torch
 
-from . import _lib
+from . import _lib, geometry
 from ._lib import MhaDesc, WinAttnDesc
 
 Tensor = torch.Tensor
@@ -116,6 +120,32 @@ def _row_stride(t: Tensor) -> int:
 
 def _stream(t: Tensor):
     return C.c_void_p(torch.cuda.current_stream(t.device).cuda_stream)
+
+
+def _deterministic() -> bool:
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def _workspace(nbytes: int, like: Tensor) -> Tensor:
+    return torch.empty((nbytes + 3) // 4, dtype=torch.float32, device=like.device)
+
+
+# Inverse of a bias-table index (geometry.inverse_index) for the deterministic table-gradient gather, per index tensor.  The
+# entry keeps the index alive, so its address cannot be reused by another index while the entry exists; an in-place write
+# to the index bumps its version and misses.  Inverses built during graph capture are not cached (their values only exist
+# once the graph replays).
+_INVERSE = {}
+
+
+def _inverse_index(index: Tensor, T: int) -> Tuple[Tensor, Tensor]:
+    key = (index.device, index.data_ptr(), index.numel(), index._version, T)
+    hit = _INVERSE.get(key)
+    if hit is not None:
+        return hit[1], hit[2]
+    perm, offsets = geometry.inverse_index(index.reshape(-1), T)
+    if not torch.cuda.is_current_stream_capturing():
+        _INVERSE[key] = (index, perm, offsets)
+    return perm, offsets
 
 
 # Optional live kernel timing (bench.py): when KERNEL_EVENTS is a dict, every C call is
@@ -237,9 +267,10 @@ def winattn_bwd(dout: Tensor, a: Tensor, b: Optional[Tensor], bias: Optional[Ten
         d.dk_row_stride = d.dv_row_stride = 2 * Cc
     d.o_row_stride = _row_stride(out)
     d.do_row_stride = Cc
+    d.deterministic = int(_deterministic())
     dbias = torch.zeros_like(bias) if bias is not None else a.new_empty(0, dtype=torch.float32)
     dhs = torch.zeros_like(head_scale) if head_scale is not None else a.new_empty(0, dtype=torch.float32)
-    ws = lse.new_empty(max(2 * lse[0].numel(), _lib.WINATTN_WORK_BYTES // 4))
+    ws = _workspace(lib.mmn_winattn_bwd_workspace_bytes(C.byref(d)), lse)
     dcs = torch.zeros(3, Cc, dtype=torch.float32, device=a.device) if want_colsum else a.new_empty(0, dtype=torch.float32)
     with _timed("winattn_bwd", a):
         _lib.check(lib.mmn_winattn_bwd(C.byref(d), q, k, v, _ptr(bias), _ptr(head_scale), _ptr(mask), _ptr(out), _ptr(lse),
@@ -401,9 +432,11 @@ def colsum(x: Tensor) -> Tensor:
     if x.dim() != 2 or x.stride(1) != 1 or x.dtype not in _DT:
         raise RuntimeError("colsum expects a 2-D float32/bfloat16 tensor with contiguous columns")
     out = torch.zeros(x.shape[1], dtype=torch.float32, device=x.device)
+    lib, det = _lib.load(), _deterministic()
+    ws = _workspace(lib.mmn_colsum_workspace_bytes(x.shape[0], x.shape[1]), x) if det else None
     with _timed("colsum", x):
-        _lib.check(_lib.load().mmn_colsum(_ptr(x), _DT[x.dtype], x.shape[0], x.shape[1], x.stride(0), _ptr(out),
-                                          x.device.index, _stream(x)), "mmn_colsum")
+        _lib.check(lib.mmn_colsum(_ptr(x), _DT[x.dtype], x.shape[0], x.shape[1], x.stride(0), _ptr(out), _ptr(ws), int(det),
+                                  x.device.index, _stream(x)), "mmn_colsum")
     return out
 
 
@@ -437,8 +470,9 @@ def table_bias_bwd(dbias: Tensor, index: Tensor, table_rows: int) -> Tensor:
     dbias = dbias.contiguous()
     nH, NN = dbias.shape[0], index.numel()
     dtable = torch.empty(table_rows, nH, dtype=torch.float32, device=dbias.device)
-    _lib.check(_lib.load().mmn_table_bias_bwd(_ptr(dbias), _ptr(index), table_rows, nH, NN, _ptr(dtable), dbias.device.index,
-                                             _stream(dbias)), "mmn_table_bias_bwd")
+    perm, offsets = _inverse_index(index, table_rows) if _deterministic() else (None, None)
+    _lib.check(_lib.load().mmn_table_bias_bwd(_ptr(dbias), _ptr(index), _ptr(perm), _ptr(offsets), table_rows, nH, NN, _ptr(dtable),
+                                             dbias.device.index, _stream(dbias)), "mmn_table_bias_bwd")
     return dtable
 
 
@@ -495,7 +529,9 @@ def cpb_bias_bwd(dbias: Tensor, coords: Tensor, w1: Tensor, b1: Tensor, w2: Tens
     dbias = dbias.contiguous()
     dw1, db1, dw2 = torch.empty_like(w1), torch.empty_like(b1), torch.empty_like(w2)
     scratch = torch.empty(T, nH, dtype=torch.float32, device=coords.device)
-    _lib.check(_lib.load().mmn_cpb_bias_bwd(_ptr(coords), _ptr(w1), _ptr(b1), _ptr(w2), _ptr(index), _ptr(tab16), _ptr(dbias),
+    perm, offsets = _inverse_index(index, T) if _deterministic() else (None, None)
+    _lib.check(_lib.load().mmn_cpb_bias_bwd(_ptr(coords), _ptr(w1), _ptr(b1), _ptr(w2), _ptr(index), _ptr(perm), _ptr(offsets),
+                                           _ptr(tab16), _ptr(dbias),
                                            T, n_in, J, nH, NN, _ptr(scratch), _ptr(dw1), _ptr(db1), _ptr(dw2),
                                            coords.device.index, _stream(coords)), "mmn_cpb_bias_bwd")
     return dw1, db1, dw2
@@ -580,14 +616,15 @@ def linear_bwd(dy: Tensor, x: Tensor, w: Tensor, act_aux: Optional[Tensor] = Non
     dx = torch.empty(rows, n_in, dtype=dy.dtype, device=dy.device) if want_dx else dy.new_empty(0)
     dw = torch.empty(n_out, n_in, dtype=torch.float32, device=dy.device) if want_dw else dy.new_empty(0, dtype=torch.float32)
     db = torch.empty(n_out, dtype=torch.float32, device=dy.device) if want_dw else dy.new_empty(0, dtype=torch.float32)
-    ws = torch.empty(lib.mmn_linear_bwd_workspace_bytes(rows, n_in, n_out), dtype=torch.uint8, device=dy.device)
+    det = _deterministic()
+    ws = torch.empty(lib.mmn_linear_bwd_workspace_bytes(rows, n_in, n_out, int(det)), dtype=torch.uint8, device=dy.device)
     if act_aux is not None and (not _rows2d(act_aux) or act_aux.shape != (rows, n_in)):
         raise RuntimeError("act_aux must be a bf16 (rows, in) tensor with contiguous columns")
     with _timed("linear_bwd", dy):
         _lib.check(lib.mmn_linear_bwd(_ptr(dy), _ptr(x), _ptr(w), _ptr(dx) if want_dx else None, _ptr(dw) if want_dw else None,
                                       _ptr(db) if want_dw else None, _ptr(ws), _ptr(act_aux),
                                       act_aux.stride(0) if act_aux is not None else 0, act if act_aux is not None else 0,
-                                      _DT[dy.dtype], rows, n_in, n_out, dy.stride(0), x.stride(0), n_in, dy.device.index,
+                                      _DT[dy.dtype], rows, n_in, n_out, dy.stride(0), x.stride(0), n_in, int(det), dy.device.index,
                                       _stream(dy)), "mmn_linear_bwd")
     return dx, dw, db
 
@@ -698,11 +735,14 @@ def layernorm_bwd(g_sum: Optional[Tensor], g_norm: Optional[Tensor], x: Tensor, 
     dgamma = torch.zeros(cols, dtype=torch.float32, device=x.device)
     dbeta = torch.zeros(cols, dtype=torch.float32, device=x.device) if want_beta else x.new_empty(0, dtype=torch.float32)
     dt = lambda t: _DTC[t.dtype] if t is not None else 0
+    lib, det = _lib.load(), _deterministic()
+    ws = _workspace(lib.mmn_layernorm_bwd_workspace_bytes(rows, cols), x) if det else None
     with _timed("layernorm_bwd", x):
-        _lib.check(_lib.load().mmn_layernorm_bwd(_ptr(g_sum), dt(g_sum), _ptr(g_norm), dt(g_norm), _ptr(x), _DTC[x.dtype], _ptr(gamma),
+        _lib.check(lib.mmn_layernorm_bwd(_ptr(g_sum), dt(g_sum), _ptr(g_norm), dt(g_norm), _ptr(x), _DTC[x.dtype], _ptr(gamma),
                                                  _ptr(mean), _ptr(rstd), mode, _ptr(d_resid) if resid_dt >= 0 else None, max(resid_dt, 0),
                                                  _ptr(d_delta) if delta_dt >= 0 else None, max(delta_dt, 0), _ptr(dgamma),
-                                                 _ptr(dbeta) if want_beta else None, rows, cols, x.device.index, _stream(x)),
+                                                 _ptr(dbeta) if want_beta else None, _ptr(ws), int(det), rows, cols, x.device.index,
+                                                 _stream(x)),
                    "mmn_layernorm_bwd")
     return d_resid, d_delta, dgamma, dbeta
 
