@@ -31,6 +31,12 @@
  * on one GPU model with one build (grid sizes follow the SM count, so not across GPU models).  Their workspace sizes
  * come from the *_workspace_bytes queries; with the flag off the queries return what the default kernels need.
  *
+ * Dropout stream.  Attention dropout (dropout_p > 0) draws its mask from Philox4x32-10 keyed by a 64-bit seed and offset.
+ * They come from the descriptor's `seed` / `offset`, or, when `rng` is non-NULL, from the two uint64 words it points to in
+ * device memory, which the kernels read when they run.  A CUDA graph bakes the descriptor's values into its kernel
+ * parameters; with `rng` the caller can write fresh words before each replay (PyTorch's CUDA generator does so for a
+ * captured torch.randint), so every replay draws a new mask.  The same (seed, offset) gives the same mask either way.
+ *
  * Token addressing.  A "token row" is num_heads*head_dim contiguous elements; row r of
  * head h of tensor X lives at  X + row_offset(r) + h*head_dim  (element units).
  *   window attention: tokens are indexed in the UN-windowed, UN-shifted (batch, grid...)
@@ -48,7 +54,7 @@
 extern "C" {
 #endif
 
-#define MMN_ABI_VERSION 5
+#define MMN_ABI_VERSION 6
 /* scratch every window-attention launch needs: the tensor-core kernels keep the counters of their run-time work queue
  * there (zeroed by the library on the launch's stream; one buffer per launch, never shared between launches in flight) */
 #define MMN_WINATTN_WORK_BYTES 2048
@@ -81,6 +87,7 @@ typedef struct mmn_winattn_desc {
   int64_t q_row_stride, k_row_stride, v_row_stride, o_row_stride;
   int64_t do_row_stride, dq_row_stride, dk_row_stride, dv_row_stride;   /* bwd only          */
   int32_t deterministic;   /* bwd: nonzero selects the fixed-order reductions (see above)     */
+  const uint64_t* rng;     /* NULL, or a device pointer to {seed, offset} (see "Dropout stream" above) */
 } mmn_winattn_desc;
 
 typedef struct mmn_mha_desc {
@@ -95,6 +102,7 @@ typedef struct mmn_mha_desc {
   int64_t o_stride_t, o_stride_b;
   int64_t do_stride_t, do_stride_b, dq_stride_t, dq_stride_b, dk_stride_t, dk_stride_b;
   int64_t dv_stride_t, dv_stride_b;
+  const uint64_t* rng;     /* NULL, or a device pointer to {seed, offset} (see "Dropout stream" above) */
 } mmn_mha_desc;
 
 int mmn_abi_version(void);

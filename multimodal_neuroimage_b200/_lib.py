@@ -42,7 +42,7 @@ MASK_NONE, MASK_SHIFT, MASK_TENSOR, MASK_FUTURE = 0, 1, 2, 3
 PATH_AUTO, PATH_GENERIC, PATH_TCGEN05 = 0, 1, 2
 ACT_NONE, ACT_RELU, ACT_GELU = 0, 1, 2
 LN_PRE, LN_POST = 0, 1
-ABI_VERSION = 5
+ABI_VERSION = 6
 WINATTN_WORK_BYTES = 2048
 
 EXPORTS = ["mmn_abi_version", "mmn_last_error", "mmn_winattn_path", "mmn_mha_path", "mmn_launch_count",
@@ -62,7 +62,8 @@ class WinAttnDesc(C.Structure):
                 ("seed", C.c_uint64), ("offset", C.c_uint64),
                 ("q_row_stride", C.c_int64), ("k_row_stride", C.c_int64), ("v_row_stride", C.c_int64),
                 ("o_row_stride", C.c_int64), ("do_row_stride", C.c_int64), ("dq_row_stride", C.c_int64),
-                ("dk_row_stride", C.c_int64), ("dv_row_stride", C.c_int64), ("deterministic", C.c_int32)]
+                ("dk_row_stride", C.c_int64), ("dv_row_stride", C.c_int64), ("deterministic", C.c_int32),
+                ("rng", C.c_void_p)]
 
 
 class MhaDesc(C.Structure):
@@ -72,7 +73,8 @@ class MhaDesc(C.Structure):
                 ("io_dtype", C.c_int32), ("path", C.c_int32),
                 ("scale", C.c_float), ("dropout_p", C.c_float),
                 ("seed", C.c_uint64), ("offset", C.c_uint64)] + \
-               [(f"{t}_stride_{a}", C.c_int64) for t in ("q", "k", "v", "o", "do", "dq", "dk", "dv") for a in ("t", "b")]
+               [(f"{t}_stride_{a}", C.c_int64) for t in ("q", "k", "v", "o", "do", "dq", "dk", "dv") for a in ("t", "b")] + \
+               [("rng", C.c_void_p)]
 
 
 def _stamp(files) -> float:

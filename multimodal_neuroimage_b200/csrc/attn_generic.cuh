@@ -40,6 +40,7 @@ struct GenericProblem {
   float scale, dropout_p;
   unsigned long long seed, offset;
   DropoutCfg drop;                // the mask generator's constants (make_dropout(dropout_p, seed, offset))
+  const unsigned long long* rng;  // null, or device {seed, offset} replacing seed / offset (dropout_at_entry)
   const float* bias;              // (nH, nq, nk) or null
   const float* head_scale;        // (nH) when cosine
   const float* mask;              // MMN_MASK_TENSOR
@@ -83,9 +84,10 @@ __device__ __forceinline__ long long row_offset(const GenericProblem& P, int ite
 
 // Dropout keep-scale for probability (item, i, j): 0 or 1/(1-p).  Counter-based (dropout_rng.cuh), so the
 // forward and both backward kernels -- and the tensor-core MHA kernels -- regenerate the same mask without storing it.
-__device__ __forceinline__ float keep_scale(const GenericProblem& P, int item, int i, int j) {
+// `drop` is the kernel's dropout_at_entry(P.drop, P.rng).
+__device__ __forceinline__ float keep_scale(const GenericProblem& P, const DropoutCfg& drop, int item, int i, int j) {
   if (P.dropout_p <= 0.f) return 1.f;
-  return dropout_keep(P.drop, item, i, j) ? P.drop.inv_keep : 0.f;
+  return dropout_keep(drop, item, i, j) ? drop.inv_keep : 0.f;
 }
 
 // Logit for (i, j) from the raw dot product.
@@ -172,6 +174,7 @@ attn_fwd_generic(GenericProblem P, GenericLaunch L, const T* __restrict__ q, con
   const int item = item0 + slot;
   const int row = blockIdx.y * L.rows_per_slot + r_in;
   const bool active = slot < slots && item < P.n_items && row < P.nq;
+  const DropoutCfg drop = dropout_at_entry(P.drop, P.rng);
 
   float qr[DMAX], acc[DMAX];
   int rid_i = 0;
@@ -212,7 +215,7 @@ attn_fwd_generic(GenericProblem P, GenericLaunch L, const T* __restrict__ q, con
         float corr = expf(m - mn);                      // exp(-inf) = 0 on the first valid key
         float p = expf(s - mn);
         l = l * corr + p;
-        float pk = p * keep_scale(P, item, row, k0 + j);
+        float pk = p * keep_scale(P, drop, item, row, k0 + j);
 #pragma unroll
         for (int c = 0; c < DMAX; ++c) if (c < d) acc[c] = acc[c] * corr + pk * Vs[j * d + c];
         m = mn;
@@ -250,6 +253,7 @@ attn_bwd_dq_generic(GenericProblem P, GenericLaunch L, const T* __restrict__ q, 
   const int item = item0 + slot;
   const int row = blockIdx.y * L.rows_per_slot + r_in;
   const bool active = slot < slots && item < P.n_items && row < P.nq;
+  const DropoutCfg drop = dropout_at_entry(P.drop, P.rng);
 
   float qr[DMAX], dor[DMAX], dqr[DMAX];
   int rid_i = 0;
@@ -293,7 +297,7 @@ attn_bwd_dq_generic(GenericProblem P, GenericLaunch L, const T* __restrict__ q, 
         if (s == -INFINITY) continue;
         float p = expf(s - lse_i);
         psum += p;
-        delta += p * dp * keep_scale(P, item, row, k0 + j);
+        delta += p * dp * keep_scale(P, drop, item, row, k0 + j);
       }
     }
     __syncthreads();
@@ -324,7 +328,7 @@ attn_bwd_dq_generic(GenericProblem P, GenericLaunch L, const T* __restrict__ q, 
         float s = logit(P, item, dot, row, k0 + j, rid_i, Rs[j], hscale);
         if (s == -INFINITY) continue;
         float p = expf(s - lse_i) * pnorm;
-        float ds = p * (dp * keep_scale(P, item, row, k0 + j) - delta);
+        float ds = p * (dp * keep_scale(P, drop, item, row, k0 + j) - delta);
         float g = ds * hscale;
 #pragma unroll
         for (int c = 0; c < DMAX; ++c) if (c < d) dqr[c] += g * Ks[j * d + c];
@@ -381,6 +385,7 @@ attn_bwd_dkv_generic(GenericProblem P, GenericLaunch L, const T* __restrict__ q,
   const int item = item0 + slot;
   const int col = blockIdx.y * L.rows_per_slot + r_in;
   const bool active = slot < slots && item < P.n_items && col < P.nk;
+  const DropoutCfg drop = dropout_at_entry(P.drop, P.rng);
 
   float kr[DMAX], vr[DMAX], dkr[DMAX], dvr[DMAX];
   int rid_j = 0;
@@ -436,7 +441,7 @@ attn_bwd_dkv_generic(GenericProblem P, GenericLaunch L, const T* __restrict__ q,
         float s = logit(P, item, dot, q0 + i, col, Rs[i], rid_j, hscale);
         if (s == -INFINITY) continue;
         float p = expf(s - sLse[slot * cap + i]) * sNorm[slot * cap + i];
-        float ks = keep_scale(P, item, q0 + i, col);
+        float ks = keep_scale(P, drop, item, q0 + i, col);
         float ds = p * (dp * ks - sDelta[slot * cap + i]);
         float pk = p * ks, g = ds * hscale;
 #pragma unroll
@@ -483,6 +488,7 @@ attn_bias_grad_generic(GenericProblem P, const T* __restrict__ q, const T* __res
   const long long r = idx / P.nk;
   const int i = (int)(r % P.nq), h = (int)(r / P.nq), d = P.d;
   const float hscale = P.cosine ? __ldg(P.head_scale + h) : 1.f;
+  const DropoutCfg drop = dropout_at_entry(P.drop, P.rng);
   float db = 0.f, dsd = 0.f;
   for (int outer = 0; outer < P.n_items / P.nH; ++outer) {
     const int item = outer * P.nH + h;
@@ -507,7 +513,7 @@ attn_bias_grad_generic(GenericProblem P, const T* __restrict__ q, const T* __res
     if (s == -INFINITY) continue;
     const long long row = (long long)item * P.nq + i;
     const float p = expf(s - lse[row]) * delta_ws[(long long)P.n_items * P.nq + row];
-    const float ds = p * (dp * keep_scale(P, item, i, j) - delta_ws[row]);
+    const float ds = p * (dp * keep_scale(P, drop, item, i, j) - delta_ws[row]);
     db += ds;
     dsd += ds * dot;
   }
@@ -540,6 +546,7 @@ mha_avg_weights_generic(GenericProblem P, int B, const T* __restrict__ q, const 
   int j = (int)(idx % P.nk);
   long long r = idx / P.nk;
   int i = (int)(r % P.nq), b = (int)(r / P.nq);
+  const DropoutCfg drop = dropout_at_entry(P.drop, P.rng);
   float sum = 0.f;
   for (int h = 0; h < P.nH; ++h) {
     int item = b * P.nH + h, rid;
@@ -548,7 +555,7 @@ mha_avg_weights_generic(GenericProblem P, int B, const T* __restrict__ q, const 
     float dot = 0.f;
     for (int c = 0; c < P.d; ++c) dot += ldf(qp + c) * P.scale * ldf(kp + c);
     float s = logit(P, item, dot, i, j, 0, 0, 1.f);
-    if (s != -INFINITY) sum += expf(s - lse[(long long)item * P.nq + i]) * keep_scale(P, item, i, j);
+    if (s != -INFINITY) sum += expf(s - lse[(long long)item * P.nq + i]) * keep_scale(P, drop, item, i, j);
   }
   avg[idx] = sum / (float)P.nH;
 }

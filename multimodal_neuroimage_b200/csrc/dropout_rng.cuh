@@ -4,6 +4,7 @@
 // One Philox4x32-10 call covers the 2 x 2 block (i >> 1, j >> 1): word (i & 1) * 2 + (j & 1) decides element (i, j).
 // A thread that walks along a row (forward, dQ) and one that walks along a column (dK / dV: lane = key, columns = queries)
 // both get two elements per call.  Element kept iff the word's top 24 bits >= ceil(p * 2^24).
+// oracle/philox.py is the host-side transcription the tests compare the kernels' masks with.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -29,16 +30,31 @@ struct DropoutCfg {
   float inv_keep;      // 1 / (1 - p)
 };
 
+// the stream-dependent half of the constants: counter word 3 and the key
+__host__ __device__ __forceinline__ void dropout_set_stream(DropoutCfg& c, unsigned long long seed, unsigned long long offset) {
+  c.off_lo = (uint32_t)offset;
+  c.key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32) ^ (uint32_t)(offset >> 32));
+}
+
 inline DropoutCfg make_dropout(float p, unsigned long long seed, unsigned long long offset) {
   DropoutCfg c;
   const float scaled = p * 16777216.0f;                    // exact: a power-of-two multiple
   uint32_t t = (uint32_t)scaled;
   if ((float)t < scaled) ++t;
   c.thr = p > 0.f ? t : 0u;
-  c.off_lo = (uint32_t)offset;
-  c.key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32) ^ (uint32_t)(offset >> 32));
+  dropout_set_stream(c, seed, offset);
   c.inv_keep = p > 0.f ? 1.f / (1.f - p) : 1.f;
   return c;
+}
+
+// The constants a kernel uses: `c` as make_dropout built them on the host, or -- with dropout on and `rng` given -- with the
+// stream read from rng[0] = seed, rng[1] = offset in device memory at kernel entry.  A CUDA graph replays kernel parameters
+// unchanged, so this is how a replay gets a fresh mask (the caller rewrites rng before each replay).  thr and inv_keep
+// depend on p only and stay host-side.
+__device__ __forceinline__ DropoutCfg dropout_at_entry(const DropoutCfg& c, const unsigned long long* rng) {
+  DropoutCfg r = c;
+  if (c.thr != 0u && rng != nullptr) dropout_set_stream(r, rng[0], rng[1]);
+  return r;
 }
 
 // the four words of block (i2, j2) = (i >> 1, j >> 1) of attention item `item` (= batch * heads + head)

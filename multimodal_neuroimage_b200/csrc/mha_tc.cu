@@ -48,6 +48,7 @@ struct MhaParams {
   __nv_bfloat16* out; long long o_st, o_sb;    // forward output rows (t, b): out + t * o_st + b * o_sb + h * D
   float* lse;                                  // (B * nH, T) natural-log log-sum-exp
   DropoutCfg drop;                             // attention dropout (dropout_rng.cuh); thr == 0: none
+  const unsigned long long* rng;               // null, or device {seed, offset} replacing drop's stream (dropout_at_entry)
   const float* rowdata; int Tpad;              // backward: (B * nH, Tpad / 2, 4) per query pair {-lse2, -lse2, -delta scale, -delta scale}
   __nv_bfloat16 *dq, *dk, *dv;                 // backward outputs
   long long dq_st, dq_sb, dk_st, dk_sb, dv_st, dv_sb;
@@ -157,6 +158,7 @@ mha_fwd_tc_kernel(const __grid_constant__ MhaParams P) {
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int t0 = blockIdx.x * 256, h = blockIdx.y, b = blockIdx.z;
+  const DropoutCfg drop = DROP ? dropout_at_entry(P.drop, P.rng) : P.drop;
   int n_g[2];
 #pragma unroll
   for (int g = 0; g < 2; ++g) n_g[g] = t0 + g * 128 < P.T ? visible_key_tiles(P, t0 + g * 128) : 0;
@@ -347,9 +349,9 @@ mha_fwd_tc_kernel(const __grid_constant__ MhaParams P) {
         exp2_pair<MMN_MHA_POLY_FWD>(fma2(pk2u(v[2 * e], v[2 * e + 1]), a2, nm2), e, x0, x1);
         rs2[e & 1] = add2(rs2[e & 1], pk2(x0, x1));
         if (DROP) {                                   // dropped probabilities leave the row sum untouched, not P V; 1 / (1 - p) is folded into 1 / l
-          const uint4 rr = dropout_block(P.drop, b * P.nH + h, t >> 1, (s0 >> 1) + e);
-          if (!dropout_keep_word((t & 1) ? rr.z : rr.x, P.drop.thr)) x0 = 0.f;
-          if (!dropout_keep_word((t & 1) ? rr.w : rr.y, P.drop.thr)) x1 = 0.f;
+          const uint4 rr = dropout_block(drop, b * P.nH + h, t >> 1, (s0 >> 1) + e);
+          if (!dropout_keep_word((t & 1) ? rr.z : rr.x, drop.thr)) x0 = 0.f;
+          if (!dropout_keep_word((t & 1) ? rr.w : rr.y, drop.thr)) x1 = 0.f;
         }
         pk[e] = pack_bf16x2(x0, x1);
       }
@@ -374,7 +376,7 @@ mha_fwd_tc_kernel(const __grid_constant__ MhaParams P) {
       mbar_wait(&pv_done[g], (n_tiles - 1) & 1);
       tcgen05_fence_after();
     }
-    const float inv = l > 0.f ? __frcp_rn(l) * (DROP ? P.drop.inv_keep : 1.f) : 0.f;
+    const float inv = l > 0.f ? __frcp_rn(l) * (DROP ? drop.inv_keep : 1.f) : 0.f;
     uint4* dst = reinterpret_cast<uint4*>(P.out + (long long)t * P.o_st + (long long)b * P.o_sb + h * D);
 #pragma unroll
     for (int c = 0; c < D / 32; ++c) {
@@ -520,6 +522,7 @@ mha_bwd_tc_kernel(const __grid_constant__ MhaParams P) {
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int total = (((MODE == 0 ? P.S : P.T) + 127) >> 7) * P.nH * P.B;
+  const DropoutCfg drop = DROP ? dropout_at_entry(P.drop, P.rng) : P.drop;
 
   if (tid == 0) {
     for (int i = 0; i < 2; ++i) { mbar_init(&r_full[i], 1); mbar_init(&r_empty[i], 1); }
@@ -686,7 +689,7 @@ mha_bwd_tc_kernel(const __grid_constant__ MhaParams P) {
             for (int e = 0; e < 32; ++e) vs[e] = e < e_lim ? vs[e] : 0xff800000u;
           }
         }
-        const float scd = DROP ? P.scale * P.drop.inv_keep : P.scale;
+        const float scd = DROP ? P.scale * drop.inv_keep : P.scale;
         const uint64_t a2 = pk2(a_mul, a_mul), sc2 = pk2(scd, scd);
         uint32_t pp[16], dd[16];
 #pragma unroll
@@ -705,13 +708,13 @@ mha_bwd_tc_kernel(const __grid_constant__ MhaParams P) {
             // uses the dropped P (its 1 / (1 - p) is applied to dV in the epilogue)
             bool k0, k1;
             if (MODE == 0) {                          // lane = key, the pair = two queries of one block row pair
-              const uint4 rr = dropout_block(P.drop, (int)item, ((t0 + col0) >> 1) + e, (s0 + r) >> 1);
+              const uint4 rr = dropout_block(drop, (int)item, ((t0 + col0) >> 1) + e, (s0 + r) >> 1);
               const bool odd = (s0 + r) & 1;
-              k0 = dropout_keep_word(odd ? rr.y : rr.x, P.drop.thr); k1 = dropout_keep_word(odd ? rr.w : rr.z, P.drop.thr);
+              k0 = dropout_keep_word(odd ? rr.y : rr.x, drop.thr); k1 = dropout_keep_word(odd ? rr.w : rr.z, drop.thr);
             } else {                                  // lane = query, the pair = two keys
-              const uint4 rr = dropout_block(P.drop, (int)item, (t0 + r) >> 1, ((s0 + col0) >> 1) + e);
+              const uint4 rr = dropout_block(drop, (int)item, (t0 + r) >> 1, ((s0 + col0) >> 1) + e);
               const bool odd = (t0 + r) & 1;
-              k0 = dropout_keep_word(odd ? rr.z : rr.x, P.drop.thr); k1 = dropout_keep_word(odd ? rr.w : rr.y, P.drop.thr);
+              k0 = dropout_keep_word(odd ? rr.z : rr.x, drop.thr); k1 = dropout_keep_word(odd ? rr.w : rr.y, drop.thr);
             }
             if (!k0) vd[2 * e] = 0u;
             if (!k1) vd[2 * e + 1] = 0u;
@@ -753,7 +756,7 @@ mha_bwd_tc_kernel(const __grid_constant__ MhaParams P) {
         }
         if (DROP && MODE == 0 && which == 0) {         // dV = (P_drop / (1 - p))^T dO
 #pragma unroll
-          for (int e = 0; e < D; ++e) v[e] = __float_as_uint(__uint_as_float(v[e]) * P.drop.inv_keep);
+          for (int e = 0; e < D; ++e) v[e] = __float_as_uint(__uint_as_float(v[e]) * drop.inv_keep);
         }
         if (orow < limit) {
           uint4* dst = reinterpret_cast<uint4*>(base + (long long)orow * st + (long long)b * sb + h * D);
@@ -810,6 +813,7 @@ static void fill_common(MhaParams& P, const mmn_mha_desc* d, const float* mask) 
   P.T = d->tgt_len; P.S = d->src_len; P.B = d->batch; P.nH = d->num_heads;
   P.mask_kind = d->mask_kind; P.mask_diag = d->mask_diagonal; P.scale = d->scale; P.mask = mask;
   P.drop = make_dropout(d->dropout_p, d->seed, d->offset);
+  P.rng = reinterpret_cast<const unsigned long long*>(d->rng);
 }
 
 template <int D, bool DROP>

@@ -92,6 +92,7 @@ mmn::GenericProblem problem_from(const mmn_winattn_desc* d, const float* bias, c
   P.mask_kind = d->mask_kind; P.mask_windows = d->mask_windows > 0 ? d->mask_windows : 1;
   P.scale = d->scale; P.dropout_p = d->dropout_p; P.seed = d->seed; P.offset = d->offset;
   P.drop = mmn::make_dropout(d->dropout_p, d->seed, d->offset);
+  P.rng = reinterpret_cast<const unsigned long long*>(d->rng);
   P.bias = bias; P.head_scale = head_scale; P.mask = mask;
   return P;
 }
@@ -111,6 +112,7 @@ mmn::GenericProblem problem_from(const mmn_mha_desc* d, const float* mask) {
   P.mask_kind = d->mask_kind; P.mask_diag = d->mask_diagonal; P.mask_windows = 1;
   P.scale = d->scale; P.dropout_p = d->dropout_p; P.seed = d->seed; P.offset = d->offset;
   P.drop = mmn::make_dropout(d->dropout_p, d->seed, d->offset);
+  P.rng = reinterpret_cast<const unsigned long long*>(d->rng);
   P.mask = mask;
   return P;
 }

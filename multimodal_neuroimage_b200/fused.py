@@ -55,11 +55,11 @@ class WindowAttentionModuleFn(torch.autograd.Function):
             wa, wb, wp = castw(w_a), castw(w_b), castw(w_proj)       # biases stay in their own dtype: added in fp32
             a = _project(xc, wa, b_a).view(B, *grid, -1)
             b = _project(yc, wb, b_b).view(B, *grid, -1) if y is not None else None
-            p, seed, off = dropout
+            p, seed, off, rng = dropout
             out, lse = torch.ops.mmn_b200.winattn_fwd(a, b, bias, head_scale, None, list(grid), list(window), list(shift),
-                                                      num_heads, score_kind, mask_kind, scale, p, seed, off, path)
+                                                      num_heads, score_kind, mask_kind, scale, p, seed, off, path, rng)
             res = _project(out.view(B * L, C), wp, b_proj).view(B, L, C).to(odt)
-        ctx.save_for_backward(xc, yc, a, b, out, lse, wa, wb, wp, bias, head_scale)
+        ctx.save_for_backward(xc, yc, a, b, out, lse, wa, wb, wp, bias, head_scale, rng)
         ctx.cfg = (list(grid), list(window), list(shift), num_heads, score_kind, mask_kind, scale, p, seed, off, path)
         ctx.meta = (x.dtype, None if y is None else y.dtype, w_a.dtype, None if b_a is None else b_a.dtype,
                     None if w_b is None else w_b.dtype, None if b_b is None else b_b.dtype, w_proj.dtype,
@@ -69,7 +69,7 @@ class WindowAttentionModuleFn(torch.autograd.Function):
     @staticmethod
     @torch.autograd.function.once_differentiable
     def backward(ctx, dres):
-        xc, yc, a, b, out, lse, wa, wb, wp, bias, head_scale = ctx.saved_tensors
+        xc, yc, a, b, out, lse, wa, wb, wp, bias, head_scale, rng = ctx.saved_tensors
         xdt, ydt, wadt, badt, wbdt, bbdt, wpdt, bpdt, (B, L, C) = ctx.meta
         with torch.autocast("cuda", enabled=False):
             dy = dres.to(xc.dtype).reshape(B * L, C)
@@ -89,7 +89,7 @@ class WindowAttentionModuleFn(torch.autograd.Function):
                 d_wp = _mm_f32(dy.t(), out2).to(wpdt)
                 dout = (dy @ wp).view(out.shape)
             da, db, dbias, dhs, dcs = torch.ops.mmn_b200.winattn_bwd(dout, a, b, bias, head_scale, None, out, lse, *ctx.cfg,
-                                                                     True)
+                                                                     True, rng)
             da2 = da.view(B * L, -1)
             if ops.linear_bwd_supported(da2, xc, wa):
                 dx, d_wa, _ = torch.ops.mmn_b200.linear_bwd(da2, xc, wa)
@@ -116,7 +116,8 @@ class WindowAttentionModuleFn(torch.autograd.Function):
 
 def window_attention_module(x: torch.Tensor, y: Optional[torch.Tensor], w_a, b_a, w_b, b_b, w_proj, b_proj, bias, head_scale,
                             grid, window, shift, num_heads: int, score_kind: int, mask_kind: int, scale: float,
-                            dropout=(0.0, 0, 0), path: int = 0) -> torch.Tensor:
+                            dropout=(0.0, 0, 0, None), path: int = 0) -> torch.Tensor:
+    """dropout: (p, seed, offset, rng) as ops.next_dropout_stream returns it."""
     return WindowAttentionModuleFn.apply(x, y, w_a, b_a, w_b, b_b, w_proj, b_proj, bias, head_scale, tuple(grid), tuple(window),
                                          tuple(shift), num_heads, score_kind, mask_kind, float(scale), dropout, path)
 

@@ -146,11 +146,11 @@ class MultiheadAttention(nn.Module):
             kind, diag = _lib.MASK_TENSOR, 0
             mask = attn_mask.to(device=q.device, dtype=torch.float32).contiguous()
 
-        p, seed, off = ops.next_dropout_stream(self.attn_dropout, self.training, q.device)
+        p, seed, off, rng = ops.next_dropout_stream(self.attn_dropout, self.training, q.device)
         io = q.dtype                                   # float16 under the reference trainer's autocast: kernels run it as bf16
         q, k, v = ops.kernel_io(q), ops.kernel_io(k), ops.kernel_io(v)
         attn, lse = torch.ops.mmn_b200.mha_fwd(q, k, v, mask, self.num_heads_mult, kind, diag, float(self.scaling),
-                                               p, seed, off)
+                                               p, seed, off, rng)
         if pad:
             w_out = F.pad(self.out_proj.weight.view(E, self.num_heads_mult, self.head_dim), (0, pad - self.head_dim))
             attn = F.linear(attn.to(io), w_out.reshape(E, self.num_heads_mult * pad), self.out_proj.bias)
@@ -161,7 +161,7 @@ class MultiheadAttention(nn.Module):
         if need:
             with torch.no_grad():
                 weights = torch.ops.mmn_b200.mha_avg_weights(q.detach(), k.detach(), mask, lse, self.num_heads_mult, kind,
-                                                             diag, float(self.scaling), p, seed, off).to(attn.dtype)
+                                                             diag, float(self.scaling), p, seed, off, rng).to(attn.dtype)
         return attn, weights
 
     def in_proj_qkv(self, query):

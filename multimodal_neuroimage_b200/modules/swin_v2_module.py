@@ -191,10 +191,10 @@ class WindowAttention(nn.Module):
         return F.linear(x, self.qkv.weight, bias)
 
     def _core(self, qkv, grid, window, shift, mask_kind, mask):
-        p, seed, off = ops.next_dropout_stream(self.attn_drop.p, self.training, qkv.device)
+        p, seed, off, rng = ops.next_dropout_stream(self.attn_drop.p, self.training, qkv.device)
         out, _ = torch.ops.mmn_b200.winattn_fwd(ops.kernel_io(qkv), None, self.position_bias(), self.head_scale(), mask,
                                                 list(grid), list(window), list(shift), self.num_heads_swin,
-                                                _lib.SCORE_COSINE, mask_kind, 1.0, p, seed, off, self.kernel_path)
+                                                _lib.SCORE_COSINE, mask_kind, 1.0, p, seed, off, self.kernel_path, rng)
         return out.to(qkv.dtype)
 
     def forward(self, x, mask=None):

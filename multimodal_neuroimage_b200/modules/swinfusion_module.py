@@ -70,10 +70,10 @@ class _TableBiasAttention(nn.Module):
         return b.view(N, N, -1).permute(2, 0, 1).contiguous()
 
     def _core(self, a, b, grid, window, shift, mask_kind, mask):
-        p, seed, off = ops.next_dropout_stream(self.attn_drop.p, self.training, a.device)
+        p, seed, off, rng = ops.next_dropout_stream(self.attn_drop.p, self.training, a.device)
         out, _ = torch.ops.mmn_b200.winattn_fwd(ops.kernel_io(a), ops.kernel_io(b), self.position_bias(), None, mask,
                                                 list(grid), list(window), list(shift), self.num_heads, _lib.SCORE_SCALED,
-                                                mask_kind, float(self.scale), p, seed, off, self.kernel_path)
+                                                mask_kind, float(self.scale), p, seed, off, self.kernel_path, rng)
         return out.to(a.dtype)
 
     @staticmethod

@@ -170,8 +170,17 @@ class _timed:
         return False
 
 
+def _rng_ptr(rng: Optional[Tensor], like: Tensor) -> Optional[int]:
+    """Device address of a dropout stream {seed, offset} (next_dropout_stream), or None."""
+    if rng is None:
+        return None
+    if rng.dtype != torch.int64 or rng.numel() != 2 or not rng.is_contiguous() or rng.device != like.device:
+        raise RuntimeError("rng must be a contiguous (2,) int64 tensor {seed, offset} on the attention's device")
+    return rng.data_ptr()
+
+
 def _win_desc(a: Tensor, b: Optional[Tensor], grid, window, shift, num_heads, score_kind, mask_kind, mask_windows,
-              scale, dropout_p, seed, offset, path) -> Tuple[WinAttnDesc, int]:
+              scale, dropout_p, seed, offset, path, rng=None) -> Tuple[WinAttnDesc, int]:
     n = len(grid)
     if a.dtype not in _DT:
         raise RuntimeError(f"unsupported dtype {a.dtype}: the window-attention kernels take float32 or bfloat16")
@@ -186,6 +195,7 @@ def _win_desc(a: Tensor, b: Optional[Tensor], grid, window, shift, num_heads, sc
     d.score_kind, d.mask_kind, d.mask_windows = score_kind, mask_kind, mask_windows
     d.io_dtype, d.path = _DT[a.dtype], path
     d.scale, d.dropout_p, d.seed, d.offset = scale, dropout_p, seed, offset
+    d.rng = _rng_ptr(rng, a)
     return d, Cc
 
 
@@ -193,11 +203,12 @@ def _win_desc(a: Tensor, b: Optional[Tensor], grid, window, shift, num_heads, sc
 def winattn_fwd(a: Tensor, b: Optional[Tensor], bias: Optional[Tensor], head_scale: Optional[Tensor],
                 mask: Optional[Tensor], grid: List[int], window: List[int], shift: List[int], num_heads: int,
                 score_kind: int, mask_kind: int, scale: float, dropout_p: float, seed: int, offset: int,
-                path: int) -> Tuple[Tensor, Tensor]:
+                path: int, rng: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
+    """rng: None, or a device {seed, offset} (next_dropout_stream) that replaces seed / offset."""
     _require_cuda(a, b, bias, head_scale, mask)
     lib = _lib.load()
     d, Cc = _win_desc(a, b, grid, window, shift, num_heads, score_kind, mask_kind,
-                      mask.shape[0] if mask is not None else 0, scale, dropout_p, seed, offset, path)
+                      mask.shape[0] if mask is not None else 0, scale, dropout_p, seed, offset, path, rng)
     if tuple(a.shape[1:-1]) != tuple(grid):
         raise RuntimeError(f"tensor grid {tuple(a.shape[1:-1])} != geometry {tuple(grid)}")
     out = torch.empty(*a.shape[:-1], Cc, dtype=a.dtype, device=a.device)
@@ -230,7 +241,7 @@ def winattn_fwd(a: Tensor, b: Optional[Tensor], bias: Optional[Tensor], head_sca
 
 @winattn_fwd.register_fake
 def _(a, b, bias, head_scale, mask, grid, window, shift, num_heads, score_kind, mask_kind, scale, dropout_p, seed,
-      offset, path):
+      offset, path, rng=None):
     Cc = a.shape[-1] // 3 if b is None else a.shape[-1]
     N = nW = 1
     for g, w in zip(grid, window):
@@ -243,13 +254,14 @@ def _(a, b, bias, head_scale, mask, grid, window, shift, num_heads, score_kind, 
 def winattn_bwd(dout: Tensor, a: Tensor, b: Optional[Tensor], bias: Optional[Tensor], head_scale: Optional[Tensor],
                 mask: Optional[Tensor], out: Tensor, lse: Tensor, grid: List[int], window: List[int], shift: List[int],
                 num_heads: int, score_kind: int, mask_kind: int, scale: float, dropout_p: float, seed: int,
-                offset: int, path: int, want_colsum: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+                offset: int, path: int, want_colsum: bool = False,
+                rng: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
     """Returns (da, db, dbias, dhead_scale, dcolsum); unused ones are empty tensors.  dcolsum (3, C) fp32 =
-    column sums over all tokens of dq, dk, dv, i.e. the bias gradients of the q/k/v projections."""
+    column sums over all tokens of dq, dk, dv, i.e. the bias gradients of the q/k/v projections.  rng: the forward's."""
     _require_cuda(dout, a, b, bias, head_scale, mask, out, lse)
     lib = _lib.load()
     d, Cc = _win_desc(a, b, grid, window, shift, num_heads, score_kind, mask_kind,
-                      mask.shape[0] if mask is not None else 0, scale, dropout_p, seed, offset, path)
+                      mask.shape[0] if mask is not None else 0, scale, dropout_p, seed, offset, path, rng)
     dout = dout.contiguous()
     da = torch.empty(a.shape, dtype=a.dtype, device=a.device)
     db = torch.empty(b.shape, dtype=b.dtype, device=b.device) if b is not None else a.new_empty(0)
@@ -282,7 +294,7 @@ def winattn_bwd(dout: Tensor, a: Tensor, b: Optional[Tensor], bias: Optional[Ten
 
 @winattn_bwd.register_fake
 def _(dout, a, b, bias, head_scale, mask, out, lse, grid, window, shift, num_heads, score_kind, mask_kind, scale,
-      dropout_p, seed, offset, path, want_colsum=False):
+      dropout_p, seed, offset, path, want_colsum=False, rng=None):
     Cc = a.shape[-1] // 3 if b is None else a.shape[-1]
     return (torch.empty_like(a), torch.empty_like(b) if b is not None else a.new_empty(0),
             torch.empty_like(bias) if bias is not None else a.new_empty(0, dtype=torch.float32),
@@ -292,17 +304,17 @@ def _(dout, a, b, bias, head_scale, mask, out, lse, grid, window, shift, num_hea
 
 def _winattn_setup(ctx, inputs, output):
     (a, b, bias, head_scale, mask, grid, window, shift, num_heads, score_kind, mask_kind, scale, dropout_p, seed,
-     offset, path) = inputs
+     offset, path, rng) = inputs
     out, lse = output
-    ctx.save_for_backward(a, b, bias, head_scale, mask, out, lse)
+    ctx.save_for_backward(a, b, bias, head_scale, mask, out, lse, rng)
     ctx.cfg = (grid, window, shift, num_heads, score_kind, mask_kind, scale, dropout_p, seed, offset, path)
 
 
 def _winattn_backward(ctx, dout, dlse):
-    a, b, bias, head_scale, mask, out, lse = ctx.saved_tensors
-    da, db, dbias, dhs, _ = torch.ops.mmn_b200.winattn_bwd(dout, a, b, bias, head_scale, mask, out, lse, *ctx.cfg)
+    a, b, bias, head_scale, mask, out, lse, rng = ctx.saved_tensors
+    da, db, dbias, dhs, _ = torch.ops.mmn_b200.winattn_bwd(dout, a, b, bias, head_scale, mask, out, lse, *ctx.cfg, False, rng)
     return (da, db if b is not None else None, dbias if bias is not None else None,
-            dhs if head_scale is not None else None, None) + (None,) * 11
+            dhs if head_scale is not None else None, None) + (None,) * 12
 
 
 torch.library.register_autograd("mmn_b200::winattn_fwd", _winattn_backward, setup_context=_winattn_setup)
@@ -317,7 +329,7 @@ def _tb_strides(t: Tensor) -> Tuple[int, int]:
     return t.stride(0), t.stride(1)
 
 
-def _mha_desc(q, k, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset) -> MhaDesc:
+def _mha_desc(q, k, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset, rng=None) -> MhaDesc:
     if q.dtype not in _DT:
         raise RuntimeError(f"unsupported dtype {q.dtype}: the attention kernels take float32 or bfloat16")
     d = MhaDesc()
@@ -329,15 +341,17 @@ def _mha_desc(q, k, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, off
     d.mask_kind, d.mask_diagonal = mask_kind, mask_diag
     d.io_dtype, d.path = _DT[q.dtype], _lib.PATH_AUTO
     d.scale, d.dropout_p, d.seed, d.offset = scale, dropout_p, seed, offset
+    d.rng = _rng_ptr(rng, q)
     return d
 
 
 @torch.library.custom_op("mmn_b200::mha_fwd", mutates_args=())
 def mha_fwd(q: Tensor, k: Tensor, v: Tensor, mask: Optional[Tensor], num_heads: int, mask_kind: int, mask_diag: int,
-            scale: float, dropout_p: float, seed: int, offset: int) -> Tuple[Tensor, Tensor]:
+            scale: float, dropout_p: float, seed: int, offset: int, rng: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
+    """rng: None, or a device {seed, offset} (next_dropout_stream) that replaces seed / offset."""
     _require_cuda(q, k, v, mask)
     lib = _lib.load()
-    d = _mha_desc(q, k, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset)
+    d = _mha_desc(q, k, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset, rng)
     out = torch.empty(q.shape, dtype=q.dtype, device=q.device)
     lse = torch.empty(q.shape[1] * num_heads, q.shape[0], dtype=torch.float32, device=q.device)
     d.q_stride_t, d.q_stride_b = _tb_strides(q)
@@ -353,7 +367,7 @@ def mha_fwd(q: Tensor, k: Tensor, v: Tensor, mask: Optional[Tensor], num_heads: 
 
 
 @mha_fwd.register_fake
-def _(q, k, v, mask, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset):
+def _(q, k, v, mask, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset, rng=None):
     return torch.empty_like(q, memory_format=torch.contiguous_format), q.new_empty(q.shape[1] * num_heads, q.shape[0],
                                                                                     dtype=torch.float32)
 
@@ -361,10 +375,10 @@ def _(q, k, v, mask, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, of
 @torch.library.custom_op("mmn_b200::mha_bwd", mutates_args=())
 def mha_bwd(dout: Tensor, q: Tensor, k: Tensor, v: Tensor, mask: Optional[Tensor], out: Tensor, lse: Tensor,
             num_heads: int, mask_kind: int, mask_diag: int, scale: float, dropout_p: float, seed: int,
-            offset: int) -> Tuple[Tensor, Tensor, Tensor]:
+            offset: int, rng: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
     _require_cuda(dout, q, k, v, mask, out, lse)
     lib = _lib.load()
-    d = _mha_desc(q, k, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset)
+    d = _mha_desc(q, k, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset, rng)
     dout = dout.contiguous()
     dq = torch.empty(q.shape, dtype=q.dtype, device=q.device)
     dk = torch.empty(k.shape, dtype=k.dtype, device=k.device)
@@ -385,22 +399,22 @@ def mha_bwd(dout: Tensor, q: Tensor, k: Tensor, v: Tensor, mask: Optional[Tensor
 
 
 @mha_bwd.register_fake
-def _(dout, q, k, v, mask, out, lse, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset):
+def _(dout, q, k, v, mask, out, lse, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset, rng=None):
     c = torch.contiguous_format
     return torch.empty_like(q, memory_format=c), torch.empty_like(k, memory_format=c), torch.empty_like(v, memory_format=c)
 
 
 def _mha_setup(ctx, inputs, output):
-    q, k, v, mask, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset = inputs
+    q, k, v, mask, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset, rng = inputs
     out, lse = output
-    ctx.save_for_backward(q, k, v, mask, out, lse)
+    ctx.save_for_backward(q, k, v, mask, out, lse, rng)
     ctx.cfg = (num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset)
 
 
 def _mha_backward(ctx, dout, dlse):
-    q, k, v, mask, out, lse = ctx.saved_tensors
-    dq, dk, dv = torch.ops.mmn_b200.mha_bwd(dout, q, k, v, mask, out, lse, *ctx.cfg)
-    return (dq, dk, dv, None) + (None,) * 7
+    q, k, v, mask, out, lse, rng = ctx.saved_tensors
+    dq, dk, dv = torch.ops.mmn_b200.mha_bwd(dout, q, k, v, mask, out, lse, *ctx.cfg, rng)
+    return (dq, dk, dv, None) + (None,) * 8
 
 
 torch.library.register_autograd("mmn_b200::mha_fwd", _mha_backward, setup_context=_mha_setup)
@@ -408,10 +422,11 @@ torch.library.register_autograd("mmn_b200::mha_fwd", _mha_backward, setup_contex
 
 @torch.library.custom_op("mmn_b200::mha_avg_weights", mutates_args=())
 def mha_avg_weights(q: Tensor, k: Tensor, mask: Optional[Tensor], lse: Tensor, num_heads: int, mask_kind: int,
-                    mask_diag: int, scale: float, dropout_p: float, seed: int, offset: int) -> Tensor:
+                    mask_diag: int, scale: float, dropout_p: float, seed: int, offset: int,
+                    rng: Optional[Tensor] = None) -> Tensor:
     _require_cuda(q, k, mask, lse)
     lib = _lib.load()
-    d = _mha_desc(q, k, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset)
+    d = _mha_desc(q, k, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset, rng)
     d.q_stride_t, d.q_stride_b = _tb_strides(q)
     d.k_stride_t, d.k_stride_b = _tb_strides(k)
     avg = torch.empty(q.shape[1], q.shape[0], k.shape[0], dtype=torch.float32, device=q.device)
@@ -421,7 +436,7 @@ def mha_avg_weights(q: Tensor, k: Tensor, mask: Optional[Tensor], lse: Tensor, n
 
 
 @mha_avg_weights.register_fake
-def _(q, k, mask, lse, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset):
+def _(q, k, mask, lse, num_heads, mask_kind, mask_diag, scale, dropout_p, seed, offset, rng=None):
     return q.new_empty(q.shape[1], q.shape[0], k.shape[0], dtype=torch.float32)
 
 
@@ -792,15 +807,17 @@ class AddLayerNormFn(torch.autograd.Function):
                 None, None, None)
 
 
-def next_dropout_stream(p: float, training: bool, device) -> Tuple[float, int, int]:
-    """(p, seed, offset) for one attention call: a fresh Philox offset drawn from torch's
-    generator so `torch.manual_seed` controls it; p = 0 outside training."""
+def next_dropout_stream(p: float, training: bool, device) -> Tuple[float, int, int, Optional[Tensor]]:
+    """(p, seed, offset, rng) for one attention call, the last four arguments of the attention ops.  rng is a (2,) int64
+    {seed, offset} drawn on `device` from its CUDA generator, so `torch.manual_seed` controls it and a CUDA graph that
+    captured this call draws a fresh one on every replay; the kernels read it when they run (seed and offset are then 0).
+    Outside training, or with p = 0: (0.0, 0, 0, None)."""
     if not training or p <= 0.0:
-        return 0.0, 0, 0
-    s = torch.randint(0, 2 ** 62, (2,), dtype=torch.int64)
-    return float(p), int(s[0]), int(s[1])
+        return 0.0, 0, 0, None
+    return float(p), 0, 0, torch.randint(0, 2 ** 62, (2,), dtype=torch.int64, device=device)
 
 
-def winattn_path_name(a: Tensor, b: Optional[Tensor], grid, window, shift, num_heads, score_kind, mask_kind) -> str:
-    d, _ = _win_desc(a, b, grid, window, shift, num_heads, score_kind, mask_kind, 1, 1.0, 0.0, 0, 0, _lib.PATH_AUTO)
+def winattn_path_name(a: Tensor, b: Optional[Tensor], grid, window, shift, num_heads, score_kind, mask_kind,
+                      dropout_p: float = 0.0) -> str:
+    d, _ = _win_desc(a, b, grid, window, shift, num_heads, score_kind, mask_kind, 1, 1.0, dropout_p, 0, 0, _lib.PATH_AUTO)
     return _lib.load().mmn_winattn_path(C.byref(d)).decode()

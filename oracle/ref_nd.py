@@ -323,8 +323,9 @@ def cross_block(x: Tensor, y: Tensor, p: Dict[str, Tensor], x_size: Sequence[int
 # a12: fairseq-style multi-head attention        modules/multihead_attention.py:51-134
 # ----------------------------------------------------------------------------------------
 def multihead_attention(query: Tensor, key: Tensor, value: Tensor, p: Dict[str, Tensor], num_heads: int,
-                        attn_mask: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
-    """(T,B,E),(S,B,E),(S,B,E) -> ((T,B,E), head-averaged weights (B,T,S)); eval mode.
+                        attn_mask: Optional[Tensor] = None, keep: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
+    """(T,B,E),(S,B,E),(S,B,E) -> ((T,B,E), head-averaged weights (B,T,S)); eval mode, or with `keep` (B*nH, T, S)
+    (oracle/philox.py: 0 or 1/(1-p)) the training-mode attention dropout (:123), which both outputs see.
     The three projection branches of the reference (:69-84) are numerically the same
     slicing of in_proj_weight, so one code path restates all of them."""
     T, B, E = query.shape
@@ -342,6 +343,8 @@ def multihead_attention(query: Tensor, key: Tensor, value: Tensor, p: Dict[str, 
     if attn_mask is not None:
         w = w + attn_mask.unsqueeze(0)                                                      # :112-118
     w = F.softmax(w.float(), dim=-1).type_as(w)                                             # :120
+    if keep is not None:
+        w = w * keep.to(w.dtype)                                                            # :123
     a = torch.bmm(w, v).transpose(0, 1).contiguous().view(T, B, E)
     a = F.linear(a, p["out_proj.weight"], p.get("out_proj.bias"))
     return a, w.view(B, num_heads, T, S).sum(dim=1) / num_heads
@@ -426,10 +429,11 @@ def transformer_encoder(x_in: Tensor, p: Dict[str, Tensor], num_heads: int, num_
 def window_attention_core(q: Tensor, k: Tensor, v: Tensor, grid: Sequence[int], window: Sequence[int],
                           shift: Sequence[int], num_heads: int, *, cosine: bool, scale: float = 1.0,
                           head_scale: Optional[Tensor] = None, bias: Optional[Tensor] = None,
-                          mask: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
+                          mask: Optional[Tensor] = None, keep: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
     """q,k,v: (B, *grid, C) un-windowed.  Returns (out (B,*grid,C), lse (B*nW, nH, N)).
     Same maths as a6/a8 between `qkv = linear(x)` and `proj`, with the roll/partition/
-    reverse/roll-back of the block around it."""
+    reverse/roll-back of the block around it.  keep: attention dropout, (B*nW*nH, N, N) factors 0 or 1/(1-p)
+    (oracle/philox.py) that multiply the probabilities before `@ v`; lse is unaffected."""
     B, C = q.shape[0], q.shape[-1]
     n = len(grid)
     window, shift = _tup(window, n), _tup(shift, n)
@@ -452,6 +456,9 @@ def window_attention_core(q: Tensor, k: Tensor, v: Tensor, grid: Sequence[int], 
         nW = mask.shape[0]
         attn = (attn.view(-1, nW, num_heads, N, N) + mask.unsqueeze(1).unsqueeze(0)).view(-1, num_heads, N, N)
     lse = torch.logsumexp(attn, dim=-1)
-    out = (attn.softmax(-1) @ vw).transpose(1, 2).reshape(-1, *window, C)
+    probs = attn.softmax(-1)
+    if keep is not None:
+        probs = probs * keep.to(probs.dtype).view(-1, num_heads, N, N)
+    out = (probs @ vw).transpose(1, 2).reshape(-1, *window, C)
     out = cyclic_shift_nd(window_reverse_nd(out, window, grid), shift, inverse=True)
     return out, lse

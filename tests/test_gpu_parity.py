@@ -106,7 +106,7 @@ def _core_inputs(case, dtype, cross, seed=0):
     return a, b, bias, hs, mask, dout
 
 
-def _oracle_core(case, a, b, bias, hs, mask, dout):
+def _oracle_core(case, a, b, bias, hs, mask, dout, keep=None):
     grid, window, shift, nH, d, cosine, mask_mode, B = case
     C = nH * d
     dd = torch.float64
@@ -122,7 +122,7 @@ def _oracle_core(case, a, b, bias, hs, mask, dout):
     if mask_mode == "shift":
         m = R.shift_mask_nd(grid, window, shift, dd)
     out, lse = R.window_attention_core(q, k, v, grid, window, shift, nH, cosine=cosine, scale=d ** -0.5,
-                                       head_scale=hs, bias=bias, mask=m)
+                                       head_scale=hs, bias=bias, mask=m, keep=keep)
     wrt = [t for t in (a, b, bias, hs) if t is not None]
     grads = torch.autograd.grad((out * dout.to(dd)).sum(), wrt)
     it = iter(grads)
