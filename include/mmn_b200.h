@@ -54,7 +54,7 @@
 extern "C" {
 #endif
 
-#define MMN_ABI_VERSION 6
+#define MMN_ABI_VERSION 7
 /* scratch every window-attention launch needs: the tensor-core kernels keep the counters of their run-time work queue
  * there (zeroed by the library on the launch's stream; one buffer per launch, never shared between launches in flight) */
 #define MMN_WINATTN_WORK_BYTES 2048
@@ -123,6 +123,16 @@ uint64_t mmn_launch_count(void);
 int mmn_winattn_fwd(const mmn_winattn_desc* desc, const void* q, const void* k, const void* v,
                     const float* bias, const float* head_scale, const float* mask,
                     void* out, float* lse, void* workspace, int device, void* stream);
+
+/* Self-attention forward with the qkv projection fused in: qkv = x w_qkv^T + b_qkv (fp32 accumulation, fp32 bias, bf16
+ * result, written to qkv_out as (tokens, 3C) rows: the packed layout mmn_winattn_bwd reads as q = base, k = base + C,
+ * v = base + 2C), then out, lse and the records exactly as mmn_winattn_fwd computes them from that qkv.  x: (tokens, C)
+ * bf16 rows in the same token order; w_qkv (3C, C) bf16 row-major; b_qkv (3C) fp32 or NULL; the desc's row strides are
+ * ignored (qkv 3C, out C).  Only shapes mmn_winattn_qkv_path accepts; there is no fallback inside this entry point. */
+const char* mmn_winattn_qkv_path(const mmn_winattn_desc* desc, int in_channels);   /* "tcgen05-fused" or why not */
+int mmn_winattn_qkv_fwd(const mmn_winattn_desc* desc, const void* x, const void* w_qkv, const float* b_qkv,
+                        const float* bias, const float* head_scale, const float* mask,
+                        void* qkv_out, void* out, float* lse, void* workspace, int device, void* stream);
 
 /* dbias (num_heads,N,N) fp32 and dhead_scale (num_heads) fp32 are ACCUMULATED into (the
  * caller zeroes them); either may be NULL to skip.  `out` is the forward output (may be NULL:

@@ -19,7 +19,7 @@ LIB_PATH = os.environ.get("MMN_LIB") or os.path.join(PKG_DIR, "libmmn_b200.so")
 # translation unit -> headers it depends on (besides include/mmn_b200.h)
 SOURCES = {"mmn_abi.cu": ["generic_launch.h", "attn_generic.cuh", "winattn_tc.h", "dropout_rng.cuh", "zero_fill.h"],
            "generic_launch.cu": ["generic_launch.h", "attn_generic.cuh", "dropout_rng.cuh", "zero_fill.h"],
-           "winattn_tc.cu": ["winattn_tc.h", "winattn_tc_fwd.cuh", "winattn_tc_bwd.cuh", "tc_window.cuh", "tc_sched.cuh", "tc_common.cuh",
+           "winattn_tc.cu": ["winattn_tc.h", "winattn_tc_fwd.cuh", "winattn_tc_bwd.cuh", "winattn_tc_qkv_fwd.cuh", "tc_window.cuh", "tc_sched.cuh", "tc_common.cuh",
                              "zero_fill.h"],
            "linbwd_tc.cu": ["winattn_tc.h", "tc_window.cuh", "tc_common.cuh"],
            "gemm_tc.cu": ["winattn_tc.h", "tc_window.cuh", "tc_common.cuh"],
@@ -42,11 +42,11 @@ MASK_NONE, MASK_SHIFT, MASK_TENSOR, MASK_FUTURE = 0, 1, 2, 3
 PATH_AUTO, PATH_GENERIC, PATH_TCGEN05 = 0, 1, 2
 ACT_NONE, ACT_RELU, ACT_GELU = 0, 1, 2
 LN_PRE, LN_POST = 0, 1
-ABI_VERSION = 6
+ABI_VERSION = 7
 WINATTN_WORK_BYTES = 2048
 
 EXPORTS = ["mmn_abi_version", "mmn_last_error", "mmn_winattn_path", "mmn_mha_path", "mmn_launch_count",
-           "mmn_winattn_fwd", "mmn_winattn_bwd", "mmn_winattn_bwd_workspace_bytes", "mmn_mha_fwd", "mmn_mha_bwd", "mmn_mha_avg_weights",
+           "mmn_winattn_fwd", "mmn_winattn_qkv_path", "mmn_winattn_qkv_fwd", "mmn_winattn_bwd", "mmn_winattn_bwd_workspace_bytes", "mmn_mha_fwd", "mmn_mha_bwd", "mmn_mha_avg_weights",
            "mmn_colsum", "mmn_colsum_workspace_bytes", "mmn_layernorm_bwd_workspace_bytes",
            "mmn_linear_supported", "mmn_linear_fwd", "mmn_linear_bwd", "mmn_linear_bwd_supported", "mmn_linear_bwd_workspace_bytes",
            "mmn_cpb_bias_fwd", "mmn_cpb_bias_bwd", "mmn_table_bias_fwd", "mmn_table_bias_bwd", "mmn_layernorm_supported", "mmn_layernorm_fwd", "mmn_layernorm_bwd"]
@@ -140,6 +140,10 @@ def load() -> C.CDLL:
         lib.mmn_mha_path.argtypes = [C.POINTER(MhaDesc)]
         lib.mmn_winattn_fwd.restype = C.c_int
         lib.mmn_winattn_fwd.argtypes = [C.POINTER(WinAttnDesc), vp, vp, vp, fp, fp, fp, vp, fp, vp, C.c_int, vp]
+        lib.mmn_winattn_qkv_path.restype = C.c_char_p
+        lib.mmn_winattn_qkv_path.argtypes = [C.POINTER(WinAttnDesc), C.c_int]
+        lib.mmn_winattn_qkv_fwd.restype = C.c_int
+        lib.mmn_winattn_qkv_fwd.argtypes = [C.POINTER(WinAttnDesc), vp, vp, fp, fp, fp, fp, vp, vp, fp, vp, C.c_int, vp]
         lib.mmn_winattn_bwd_workspace_bytes.restype = C.c_size_t
         lib.mmn_winattn_bwd_workspace_bytes.argtypes = [C.POINTER(WinAttnDesc)]
         lib.mmn_winattn_bwd.restype = C.c_int

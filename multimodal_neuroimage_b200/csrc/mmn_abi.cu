@@ -168,6 +168,33 @@ int mmn_winattn_fwd(const mmn_winattn_desc* d, const void* q, const void* k, con
   return finish(e, n, "attn_fwd_generic");
 }
 
+const char* mmn_winattn_qkv_path(const mmn_winattn_desc* d, int in_channels) {
+  if (validate_win(d) != MMN_OK) return "invalid";
+  if (d->path == MMN_PATH_GENERIC) return "generic path requested";
+  const char* why = mmn::tc::qkv_fwd_why_not(d, in_channels);
+  return why ? why : "tcgen05-fused";
+}
+
+int mmn_winattn_qkv_fwd(const mmn_winattn_desc* d, const void* x, const void* w_qkv, const float* b_qkv, const float* bias,
+                        const float* head_scale, const float* mask, void* qkv_out, void* out, float* lse, void* workspace,
+                        int device, void* stream) {
+  int rc = validate_win(d);
+  if (rc) return rc;
+  if (!x || !w_qkv || !qkv_out || !out || !lse || !workspace) return fail(MMN_ERR_INVALID, "null tensor pointer");
+  if (d->score_kind == MMN_SCORE_COSINE && !head_scale) return fail(MMN_ERR_INVALID, "cosine attention needs head_scale");
+  if (d->mask_kind == MMN_MASK_TENSOR && !mask) return fail(MMN_ERR_INVALID, "MMN_MASK_TENSOR needs a mask");
+  if (!have_device()) return fail(MMN_ERR_CUDA, "no CUDA device: libmmn_b200 has no CPU path");
+  if (d->path == MMN_PATH_GENERIC) return fail(MMN_ERR_UNSUPPORTED, "the fused qkv forward has no generic path");
+  if (const char* why = mmn::tc::qkv_fwd_why_not(d, d->num_heads * d->head_dim))
+    return fail(MMN_ERR_UNSUPPORTED, "shape not supported by the fused qkv forward: %s", why);
+  DeviceGuard g(device);
+  if (!g.ok) return fail(MMN_ERR_CUDA, "cannot select device %d", device);
+  rc = mmn::tc::winattn_qkv_fwd(d, x, w_qkv, b_qkv, bias, head_scale, mask, qkv_out, out, lse, workspace, (cudaStream_t)stream,
+                                g_err, sizeof(g_err));
+  if (rc == MMN_OK) g_launches.fetch_add(1, std::memory_order_relaxed);
+  return rc;
+}
+
 size_t mmn_winattn_bwd_workspace_bytes(const mmn_winattn_desc* d) {
   if (validate_win(d) != MMN_OK) return 0;
   const mmn::GenericProblem P = problem_from(d, nullptr, nullptr, nullptr);

@@ -192,9 +192,10 @@ __device__ __forceinline__ int class_region_id(const WinShape& S, int cls, int p
 // Per-class additive table in the item's tile order, in the log2 domain:
 //   tbl[i][j] = log2(e) * (bias[pos(i)][pos(j)] + (region(pos i) != region(pos j) ? -100 : 0)).
 // `bias` is this head's (64,64) fp32 table or null; `pos` the class's 64-entry tile-row -> window-position LUT;
-// `rid` the class's window-position -> region-id LUT (class_region_id, tabulated once per CTA).
+// `rid` the class's window-position -> region-id LUT (class_region_id, tabulated once per CTA).  swz != 0: row i's float4
+// j4 is stored at j4 ^ (i & swz) (an unpadded ld = 64 table that rows of a warp still read without bank conflicts).
 __device__ __forceinline__ void build_class_table(float* tbl, int ld, const float* bias, const uint8_t* pos, const uint8_t* rid,
-                                                  bool shift_mask, int t, int nthreads) {
+                                                  bool shift_mask, int t, int nthreads, int swz = 0) {
   // eight entries per round so that eight L2 loads are in flight per thread (one at a time, a rebuild took ~10 us)
   for (int e0 = t; e0 < kN * kN; e0 += 8 * nthreads) {
     float v[8];
@@ -209,7 +210,7 @@ __device__ __forceinline__ void build_class_table(float* tbl, int ld, const floa
       if (e < kN * kN) {
         const int i = e >> 6, j = e & 63;
         if (shift_mask && rid[pos[i]] != rid[pos[j]]) v[u] -= 100.f;
-        tbl[i * ld + j] = v[u] * 1.4426950408889634f;
+        tbl[i * ld + ((((j >> 2) ^ (i & swz)) << 2) | (j & 3))] = v[u] * 1.4426950408889634f;
       }
     }
   }

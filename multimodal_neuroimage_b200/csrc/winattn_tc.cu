@@ -2,6 +2,7 @@
 #include "winattn_tc.h"
 
 #include "winattn_tc_bwd.cuh"
+#include "winattn_tc_qkv_fwd.cuh"
 
 namespace mmn { namespace tc {
 
@@ -87,5 +88,12 @@ int winattn_bwd(const mmn_winattn_desc* d, const void* q, const void* k, const v
 }
 
 size_t bwd_det_workspace_bytes(const mmn_winattn_desc* d) { return bwd_det_workspace_bytes_impl(d); }
+
+const char* qkv_fwd_why_not(const mmn_winattn_desc* d, int in_channels) { return qkv_fwd_why_not_impl(d, in_channels); }
+
+int winattn_qkv_fwd(const mmn_winattn_desc* d, const void* x, const void* w, const float* b, const float* bias, const float* head_scale,
+                    const float* mask, void* qkv, void* out, float* lse, void* workspace, cudaStream_t st, char* err, size_t errlen) {
+  return winattn_qkv_fwd_launch(d, x, w, b, bias, head_scale, mask, qkv, out, lse, workspace, st, err, errlen);
+}
 
 }}  // namespace mmn::tc

@@ -16,6 +16,11 @@ int winattn_bwd(const mmn_winattn_desc* d, const void* q, const void* k, const v
                 const float* head_scale, const float* mask, const void* out, const float* lse, const void* dout, void* dq,
                 void* dk, void* dv, float* dbias, float* dhead_scale, float* dcolsum, float* workspace, cudaStream_t st,
                 char* err, size_t errlen, int* launches);
+// self-attention forward with the qkv projection fused in (winattn_tc_qkv_fwd.cuh): qkv = x w^T + b (bf16, written), then
+// what winattn_fwd computes from it.  qkv_fwd_why_not: nullptr when the fused kernel takes the shape, else why not.
+const char* qkv_fwd_why_not(const mmn_winattn_desc* d, int in_channels);
+int winattn_qkv_fwd(const mmn_winattn_desc* d, const void* x, const void* w, const float* b, const float* bias, const float* head_scale,
+                    const float* mask, void* qkv, void* out, float* lse, void* workspace, cudaStream_t st, char* err, size_t errlen);
 // workspace of the deterministic backward (desc->deterministic != 0): one slot of partial sums per CTA
 size_t bwd_det_workspace_bytes(const mmn_winattn_desc* d);
 // fused projection backward (linbwd_tc.cu)

@@ -98,24 +98,104 @@ __device__ __forceinline__ void trace_ev(const TraceCfg& trace, int role, int it
 }
 __device__ __forceinline__ void trace_evf(const TraceCfg& trace, int role, int item, int ev) { trace_ev(trace, role, item, ev); }
 
+// sum of squares of 32 bf16 values packed in pairs (u[j] = elements 2j, 2j + 1), in one fixed order: one chain of
+// (low, high) pairs per 8-element chunk, chunks added pairwise.  The fused qkv kernel computes its norms from registers
+// with it and gets the same bits as row_sumsq over the stored row.
+__device__ __forceinline__ float sumsq_bf16x32(const uint32_t (&u)[16]) {
+  uint64_t ss[4] = {0ull, 0ull, 0ull, 0ull};
+#pragma unroll
+  for (int c = 0; c < 4; ++c)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const uint64_t x = pk2u(u[4 * c + e] << 16, u[4 * c + e] & 0xffff0000u);
+      ss[c] = fma2(x, x, ss[c]);
+    }
+  float lo, hi;
+  upk2(add2(add2(ss[0], ss[1]), add2(ss[2], ss[3])), lo, hi);
+  return lo + hi;
+}
+
 // sum of squares of one 64-byte bf16 row.  `row` = the row's index in its tile: chunk c is read at its
 // swizzled place, which also spreads the lanes of a warp over all banks (plain order is a 4-way conflict).
 __device__ __forceinline__ float row_sumsq(const uint8_t* rowp, int row) {
   const int sw = (row >> 1) & 3;
-  uint64_t ss[4] = {0ull, 0ull, 0ull, 0ull};               // one chain of (low, high) element pairs per 16-byte chunk
+  uint32_t u[16];
 #pragma unroll
   for (int c = 0; c < 4; ++c) {
     const uint4 a = *reinterpret_cast<const uint4*>(rowp + ((c ^ sw) << 4));
-    const uint32_t u[4] = {a.x, a.y, a.z, a.w};
+    u[4 * c] = a.x; u[4 * c + 1] = a.y; u[4 * c + 2] = a.z; u[4 * c + 3] = a.w;
+  }
+  return sumsq_bf16x32(u);
+}
+
+// One query row's softmax over its window's 64 keys, shared by both forward kernels.  s2: the row's logits as fp32
+// pairs (overwritten); trow: its row of the class table (float4 j4 stored at j4 ^ (row & TSWZ)); krow: the 64 keys'
+// 1/||k|| (COS); mrow: its mask row (MMN_MASK_TENSOR).  Out: P = exp2(s - max) as bf16 pairs (zero for an invalid
+// slot), the max and the sum.
+template <bool COS, int MASK, int TSWZ>
+__device__ __forceinline__ void softmax_row(uint64_t (&s2)[32], const float* trow_f, int row, const float* krow_f, const float* mrow,
+                                            float a_i, bool valid, uint32_t (&pp)[32], float& mx, float& l) {
+  {
+    const float4* trow = reinterpret_cast<const float4*>(trow_f);
+    const float4* krow = reinterpret_cast<const float4*>(krow_f);
+    const uint64_t a2 = pk2(a_i, a_i);
 #pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const uint64_t x = pk2u(u[e] << 16, u[e] & 0xffff0000u);
-      ss[c] = fma2(x, x, ss[c]);
+    for (int j4 = 0; j4 < 16; ++j4) {
+      float4 tt = trow[j4 ^ (row & TSWZ)];
+      if (MASK == MMN_MASK_TENSOR) {
+        const float4 mm = __ldg(reinterpret_cast<const float4*>(mrow) + j4);
+        tt.x = fmaf(mm.x, kLog2e, tt.x); tt.y = fmaf(mm.y, kLog2e, tt.y); tt.z = fmaf(mm.z, kLog2e, tt.z); tt.w = fmaf(mm.w, kLog2e, tt.w);
+      }
+      if (COS) {
+        const float4 kv = krow[j4];
+        s2[j4 * 2 + 0] = fma2(s2[j4 * 2 + 0], mul2(pk2(kv.x, kv.y), a2), pk2(tt.x, tt.y));
+        s2[j4 * 2 + 1] = fma2(s2[j4 * 2 + 1], mul2(pk2(kv.z, kv.w), a2), pk2(tt.z, tt.w));
+      } else {
+        s2[j4 * 2 + 0] = fma2(s2[j4 * 2 + 0], a2, pk2(tt.x, tt.y));
+        s2[j4 * 2 + 1] = fma2(s2[j4 * 2 + 1], a2, pk2(tt.z, tt.w));
+      }
     }
   }
-  float lo, hi;
-  upk2(add2(add2(ss[0], ss[1]), add2(ss[2], ss[3])), lo, hi);
-  return lo + hi;
+  {
+    float m8[8];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) upk2(s2[j], m8[2 * j], m8[2 * j + 1]);
+#pragma unroll
+    for (int j = 4; j < 32; j += 2) {                // FMNMX3: two new values per instruction
+      float a, b, c, d;
+      upk2(s2[j], a, b); upk2(s2[j + 1], c, d);
+      const int ch = (j >> 1) & 7;
+      m8[ch] = fmaxf(fmaxf(m8[ch], a), b);
+      m8[(ch + 4) & 7] = fmaxf(fmaxf(m8[(ch + 4) & 7], c), d);
+    }
+    mx = fmaxf(fmaxf(fmaxf(m8[0], m8[1]), fmaxf(m8[2], m8[3])), fmaxf(fmaxf(m8[4], m8[5]), fmaxf(m8[6], m8[7])));
+  }
+  {
+    const uint64_t nmx2 = pk2(-mx, -mx);
+    uint64_t l2[4] = {0ull, 0ull, 0ull, 0ull};
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      float a, b;
+      upk2(add2(s2[j], nmx2), a, b);
+      a = fast_exp2(a); b = fast_exp2(b);
+      l2[j & 3] = add2(l2[j & 3], pk2(a, b));
+      pp[j] = valid ? pack_bf16x2(a, b) : 0u;
+    }
+    float la, lb;
+    upk2(add2(add2(l2[0], l2[1]), add2(l2[2], l2[3])), la, lb);
+    l = la + lb;
+  }
+}
+
+// O / l -> bf16 -> row r of a 64B-swizzled (128 x 32) staging tile
+__device__ __forceinline__ void o_row_to_smem(const uint32_t (&oraw)[32], float inv_l, uint8_t* obuf, int r) {
+  const uint64_t inv2 = pk2(inv_l, inv_l);
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+    uint4 v4 = make_uint4(pack_bf16x2(mul2(pk2u(oraw[c * 8 + 0], oraw[c * 8 + 1]), inv2)), pack_bf16x2(mul2(pk2u(oraw[c * 8 + 2], oraw[c * 8 + 3]), inv2)),
+                          pack_bf16x2(mul2(pk2u(oraw[c * 8 + 4], oraw[c * 8 + 5]), inv2)), pack_bf16x2(mul2(pk2u(oraw[c * 8 + 6], oraw[c * 8 + 7]), inv2)));
+    *reinterpret_cast<uint4*>(obuf + ((c ^ ((r >> 1) & 3)) << 4)) = v4;
+  }
 }
 
 // COS: cosine attention (else scaled dot product); MASK: MMN_MASK_NONE / _SHIFT / _TENSOR.
@@ -432,61 +512,11 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
         for (int j = 0; j < 16; ++j) { s2[j] = pk2u(raw0[2 * j], raw0[2 * j + 1]); s2[16 + j] = pk2u(raw1[2 * j], raw1[2 * j + 1]); }
       }
       TR(n, 4);
-      {
-        const float4* trow = reinterpret_cast<const float4*>(tbl + i * kTblLd);
-        const float4* krow = reinterpret_cast<const float4*>(rkbuf + slot * 64);
-        const float* mrow = (MASK == MMN_MASK_TENSOR) ? P.mask + ((size_t)(gw % P.mask_windows) * kN + ipos) * kN : nullptr;
-        const uint64_t a2 = pk2(a_i, a_i);
-#pragma unroll
-        for (int j4 = 0; j4 < 16; ++j4) {
-          float4 tt = trow[j4];
-          if (MASK == MMN_MASK_TENSOR) {
-            const float4 mm = __ldg(reinterpret_cast<const float4*>(mrow) + j4);
-            tt.x = fmaf(mm.x, kLog2e, tt.x); tt.y = fmaf(mm.y, kLog2e, tt.y); tt.z = fmaf(mm.z, kLog2e, tt.z); tt.w = fmaf(mm.w, kLog2e, tt.w);
-          }
-          if (COS) {
-            const float4 kv = krow[j4];
-            s2[j4 * 2 + 0] = fma2(s2[j4 * 2 + 0], mul2(pk2(kv.x, kv.y), a2), pk2(tt.x, tt.y));
-            s2[j4 * 2 + 1] = fma2(s2[j4 * 2 + 1], mul2(pk2(kv.z, kv.w), a2), pk2(tt.z, tt.w));
-          } else {
-            s2[j4 * 2 + 0] = fma2(s2[j4 * 2 + 0], a2, pk2(tt.x, tt.y));
-            s2[j4 * 2 + 1] = fma2(s2[j4 * 2 + 1], a2, pk2(tt.z, tt.w));
-          }
-        }
-      }
-      float mx;
-      {
-        float m8[8];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) upk2(s2[j], m8[2 * j], m8[2 * j + 1]);
-#pragma unroll
-        for (int j = 4; j < 32; j += 2) {                // FMNMX3: two new values per instruction
-          float a, b, c, d;
-          upk2(s2[j], a, b); upk2(s2[j + 1], c, d);
-          const int ch = (j >> 1) & 7;
-          m8[ch] = fmaxf(fmaxf(m8[ch], a), b);
-          m8[(ch + 4) & 7] = fmaxf(fmaxf(m8[(ch + 4) & 7], c), d);
-        }
-        mx = fmaxf(fmaxf(fmaxf(m8[0], m8[1]), fmaxf(m8[2], m8[3])), fmaxf(fmaxf(m8[4], m8[5]), fmaxf(m8[6], m8[7])));
-      }
-      // ---- P = exp2(s - max) as packed bf16 pairs, straight into this row's half of the TMEM operand
       uint32_t pp[32];
-      float l;
-      {
-        const uint64_t nmx2 = pk2(-mx, -mx);
-        uint64_t l2[4] = {0ull, 0ull, 0ull, 0ull};
-#pragma unroll
-        for (int j = 0; j < 32; ++j) {
-          float a, b;
-          upk2(add2(s2[j], nmx2), a, b);
-          a = fast_exp2(a); b = fast_exp2(b);
-          l2[j & 3] = add2(l2[j & 3], pk2(a, b));
-          pp[j] = valid ? pack_bf16x2(a, b) : 0u;
-        }
-        float la, lb;
-        upk2(add2(add2(l2[0], l2[1]), add2(l2[2], l2[3])), la, lb);
-        l = la + lb;
-      }
+      float mx, l;
+      softmax_row<COS, MASK, 0>(s2, tbl + i * kTblLd, i, rkbuf + slot * 64,
+                                (MASK == MMN_MASK_TENSOR) ? P.mask + ((size_t)(gw % P.mask_windows) * kN + ipos) * kN : nullptr,
+                                a_i, valid, pp, mx, l);
       TR(n, 5);
       tmem_st_32x32b_x32(tP, pp);
       tmem_st_wait();
@@ -510,13 +540,7 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
       tmem_ld_wait();
       tcgen05_fence_before();
       mbar_wait(&so_free[g], (kk & 1) ^ 1);              // the store warp has drained this group's staging tile
-      const uint64_t inv2 = pk2(inv_l, inv_l);
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        uint4 v4 = make_uint4(pack_bf16x2(mul2(pk2u(oraw[c * 8 + 0], oraw[c * 8 + 1]), inv2)), pack_bf16x2(mul2(pk2u(oraw[c * 8 + 2], oraw[c * 8 + 3]), inv2)),
-                              pack_bf16x2(mul2(pk2u(oraw[c * 8 + 4], oraw[c * 8 + 5]), inv2)), pack_bf16x2(mul2(pk2u(oraw[c * 8 + 6], oraw[c * 8 + 7]), inv2)));
-        *reinterpret_cast<uint4*>(obuf + ((c ^ ((r >> 1) & 3)) << 4)) = v4;
-      }
+      o_row_to_smem(oraw, inv_l, obuf, r);
       fence_proxy_async_smem();
       mbar_arrive_warp(&so_ready[g]);
       TR(n, 8);

@@ -53,11 +53,19 @@ class WindowAttentionModuleFn(torch.autograd.Function):
             xc, yc = cast(x).reshape(B * L, C), (cast(y).reshape(B * L, C) if y is not None else None)
             castw = (lambda t: None if t is None else ops.weight_bf16(t)) if cdt == torch.bfloat16 else cast
             wa, wb, wp = castw(w_a), castw(w_b), castw(w_proj)       # biases stay in their own dtype: added in fp32
-            a = _project(xc, wa, b_a).view(B, *grid, -1)
-            b = _project(yc, wb, b_b).view(B, *grid, -1) if y is not None else None
             p, seed, off, rng = dropout
-            out, lse = torch.ops.mmn_b200.winattn_fwd(a, b, bias, head_scale, None, list(grid), list(window), list(shift),
-                                                      num_heads, score_kind, mask_kind, scale, p, seed, off, path, rng)
+            if y is None and cdt == torch.bfloat16 and xc.is_contiguous() and ops.winattn_qkv_path_name(
+                    (B, *grid, C), cdt, grid, window, shift, num_heads, score_kind, mask_kind, p, path) == "tcgen05-fused":
+                # one kernel: x read once, qkv written for the backward, the attention computed from it
+                a, out, lse = torch.ops.mmn_b200.winattn_qkv_fwd(
+                    xc.view(B, *grid, C), wa.contiguous(), None if b_a is None else b_a.float().contiguous(), bias,
+                    head_scale, None, list(grid), list(window), list(shift), num_heads, score_kind, mask_kind, scale, path)
+                b = None
+            else:
+                a = _project(xc, wa, b_a).view(B, *grid, -1)
+                b = _project(yc, wb, b_b).view(B, *grid, -1) if y is not None else None
+                out, lse = torch.ops.mmn_b200.winattn_fwd(a, b, bias, head_scale, None, list(grid), list(window), list(shift),
+                                                          num_heads, score_kind, mask_kind, scale, p, seed, off, path, rng)
             res = _project(out.view(B * L, C), wp, b_proj).view(B, L, C).to(odt)
         ctx.save_for_backward(xc, yc, a, b, out, lse, wa, wb, wp, bias, head_scale, rng)
         ctx.cfg = (list(grid), list(window), list(shift), num_heads, score_kind, mask_kind, scale, p, seed, off, path)

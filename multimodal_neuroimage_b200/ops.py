@@ -250,6 +250,55 @@ def _(a, b, bias, head_scale, mask, grid, window, shift, num_heads, score_kind, 
     return a.new_empty(*a.shape[:-1], Cc), a.new_empty(4, a.shape[0] * nW, num_heads, N, dtype=torch.float32)
 
 
+@torch.library.custom_op("mmn_b200::winattn_qkv_fwd", mutates_args=())
+def winattn_qkv_fwd(x: Tensor, w: Tensor, b: Optional[Tensor], bias: Optional[Tensor], head_scale: Optional[Tensor],
+                    mask: Optional[Tensor], grid: List[int], window: List[int], shift: List[int], num_heads: int,
+                    score_kind: int, mask_kind: int, scale: float, path: int) -> Tuple[Tensor, Tensor, Tensor]:
+    """Self-attention forward with the qkv projection fused in (csrc/winattn_tc_qkv_fwd.cuh).  x (B, *grid, C) bf16,
+    w (3C, C) bf16, b (3C) fp32 or None.  Returns (qkv, out, lse): qkv = x w^T + b in bf16, the packed (B, *grid, 3C)
+    tensor winattn_bwd takes as `a`; out and lse as winattn_fwd computes them from that qkv.  Only shapes for which
+    winattn_qkv_path_name says "tcgen05-fused"."""
+    _require_cuda(x, w, b, bias, head_scale, mask)
+    Cc = x.shape[-1]
+    if x.dtype != torch.bfloat16 or w.dtype != torch.bfloat16 or not x.is_contiguous() or not w.is_contiguous() \
+            or tuple(w.shape) != (3 * Cc, Cc):
+        raise RuntimeError("winattn_qkv_fwd expects contiguous bf16 x (..., C) and w (3C, C)")
+    if b is not None and (b.dtype != torch.float32 or not b.is_contiguous() or b.numel() != 3 * Cc):
+        raise RuntimeError("winattn_qkv_fwd takes its qkv bias as a contiguous float32 (3C) tensor")
+    if tuple(x.shape[1:-1]) != tuple(grid):
+        raise RuntimeError(f"tensor grid {tuple(x.shape[1:-1])} != geometry {tuple(grid)}")
+    for t in (bias, head_scale, mask):
+        if t is not None and (t.dtype != torch.float32 or not t.is_contiguous()):
+            raise RuntimeError("bias / head_scale / mask must be contiguous float32")
+    qkv = torch.empty(*x.shape[:-1], 3 * Cc, dtype=x.dtype, device=x.device)
+    d, _ = _win_desc(qkv, None, grid, window, shift, num_heads, score_kind, mask_kind,
+                     mask.shape[0] if mask is not None else 0, scale, 0.0, 0, 0, path)
+    d.q_row_stride = d.k_row_stride = d.v_row_stride = 3 * Cc
+    d.o_row_stride = Cc
+    out = torch.empty_like(x)
+    N = nW = 1
+    for g, w_ in zip(grid, window):
+        N *= w_
+        nW *= g // w_
+    lse = torch.empty(4, x.shape[0] * nW, num_heads, N, dtype=torch.float32, device=x.device)   # as winattn_fwd
+    work = torch.empty(_lib.WINATTN_WORK_BYTES, dtype=torch.uint8, device=x.device)
+    with _timed("winattn_qkv_fwd", x):
+        _lib.check(_lib.load().mmn_winattn_qkv_fwd(C.byref(d), _ptr(x), _ptr(w), _ptr(b), _ptr(bias), _ptr(head_scale),
+                                                   _ptr(mask), _ptr(qkv), _ptr(out), _ptr(lse), _ptr(work), x.device.index,
+                                                   _stream(x)), "mmn_winattn_qkv_fwd")
+    return qkv, out, lse
+
+
+@winattn_qkv_fwd.register_fake
+def _(x, w, b, bias, head_scale, mask, grid, window, shift, num_heads, score_kind, mask_kind, scale, path):
+    N = nW = 1
+    for g, w_ in zip(grid, window):
+        N *= w_
+        nW *= g // w_
+    return (x.new_empty(*x.shape[:-1], 3 * x.shape[-1]), x.new_empty(x.shape),
+            x.new_empty(4, x.shape[0] * nW, num_heads, N, dtype=torch.float32))
+
+
 @torch.library.custom_op("mmn_b200::winattn_bwd", mutates_args=())
 def winattn_bwd(dout: Tensor, a: Tensor, b: Optional[Tensor], bias: Optional[Tensor], head_scale: Optional[Tensor],
                 mask: Optional[Tensor], out: Tensor, lse: Tensor, grid: List[int], window: List[int], shift: List[int],
@@ -815,6 +864,17 @@ def next_dropout_stream(p: float, training: bool, device) -> Tuple[float, int, i
     if not training or p <= 0.0:
         return 0.0, 0, 0, None
     return float(p), 0, 0, torch.randint(0, 2 ** 62, (2,), dtype=torch.int64, device=device)
+
+
+def winattn_qkv_path_name(x_shape, dtype, grid, window, shift, num_heads, score_kind, mask_kind, dropout_p: float = 0.0,
+                          path: int = _lib.PATH_AUTO) -> str:
+    """"tcgen05-fused" when winattn_qkv_fwd takes a self-attention call on x of this shape and dtype, else the reason it
+    does not (the call then runs the projection and winattn_fwd separately)."""
+    a = torch.empty(*x_shape[:-1], 3 * x_shape[-1], dtype=dtype, device="meta")
+    d, Cc = _win_desc(a, None, grid, window, shift, num_heads, score_kind, mask_kind, 1, 1.0, dropout_p, 0, 0, path)
+    d.q_row_stride = d.k_row_stride = d.v_row_stride = 3 * Cc
+    d.o_row_stride = Cc
+    return _lib.load().mmn_winattn_qkv_path(C.byref(d), int(x_shape[-1])).decode()
 
 
 def winattn_path_name(a: Tensor, b: Optional[Tensor], grid, window, shift, num_heads, score_kind, mask_kind,
