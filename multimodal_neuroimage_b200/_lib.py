@@ -32,7 +32,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 # production builds leave it out (it costs ~8 % of the softmax warps' instructions).
 if os.environ.get("MMN_BUILD_TRACE"):
     NVCC_FLAGS.append("-DMMN_TC_TRACING")
-# MMN_NVCC_DEFINES="-DMMN_BWD_KEYS_PER_THREAD=32 ...": tuning experiments (forces a rebuild)
+# MMN_NVCC_DEFINES="-DMMN_DEBUG_WAIT ...": extra nvcc defines for debugging builds (forces a rebuild)
 NVCC_FLAGS += os.environ.get("MMN_NVCC_DEFINES", "").split()
 
 # enums of include/mmn_b200.h

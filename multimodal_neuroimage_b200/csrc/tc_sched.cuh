@@ -11,9 +11,6 @@
 // bias table in shared memory and accumulate the bias gradient in registers without atomics.
 #pragma once
 
-#include <cstdio>
-#include <cstdlib>
-
 #include "tc_window.cuh"
 
 namespace mmn { namespace tc {
@@ -26,25 +23,11 @@ struct Sched {
   long long total_wt;
 };
 
-// Relative item cost by number of wrapped axes (partitioning only).  Tuned on B200 at BASELINE cfg2 by sweeping
-// MMN_SCHED_WT_FWD / MMN_SCHED_WT_BWD="w0,w1,w2,w3" (read once per process).
-inline const int* sched_weights(bool backward) {
-  static int wt[2][4] = {{16, 18, 20, 22}, {16, 18, 20, 22}};
-  static std::once_flag once;
-  std::call_once(once, [] {
-    const char* names[2] = {"MMN_SCHED_WT_FWD", "MMN_SCHED_WT_BWD"};
-    for (int k = 0; k < 2; ++k)
-      if (const char* e = getenv(names[k])) {
-        int w[4];
-        if (sscanf(e, "%d,%d,%d,%d", &w[0], &w[1], &w[2], &w[3]) == 4 && w[0] > 0 && w[1] > 0 && w[2] > 0 && w[3] > 0)
-          for (int i = 0; i < 4; ++i) wt[k][i] = w[i];
-      }
-  });
-  return wt[backward ? 1 : 0];
-}
+// Relative item cost by number of wrapped axes (partitioning only), tuned on B200 at BASELINE cfg2.  The same weights set the
+// static per-CTA ranges of the deterministic backward, so they are part of what makes its sums reproducible.
+constexpr int kSchedWeights[4] = {16, 18, 20, 22};
 
-inline Sched make_sched(const WinShape& S, int batch, bool backward) {
-  const int* wts = sched_weights(backward);
+inline Sched make_sched(const WinShape& S, int batch) {
   Sched sc;
   sc.n_items = 0;
   sc.total_wt = 0;
@@ -58,7 +41,7 @@ inline Sched make_sched(const WinShape& S, int batch, bool backward) {
       n *= d;
     }
     sc.cnt[c] = (int)n;
-    sc.wt[c] = wts[__builtin_popcount(c)];
+    sc.wt[c] = kSchedWeights[__builtin_popcount(c)];
     sc.n_items += (sc.cnt[c] + 1) / 2;
     sc.total_wt += (long long)((sc.cnt[c] + 1) / 2) * sc.wt[c];
   }
@@ -189,6 +172,15 @@ __device__ __forceinline__ int class_region_id(const WinShape& S, int cls, int p
   return rid;
 }
 
+// The per-CTA class LUTs, filled by threads t, t + nthreads, ...: pos[8][64] tile row -> window position and
+// rid[8][64] window position -> shift-mask region id, per wrap class.
+__device__ __forceinline__ void fill_class_luts(const WinShape& S, uint8_t* pos, uint8_t* rid, int t, int nthreads) {
+  for (int i = t; i < 512; i += nthreads) {
+    pos[i] = (uint8_t)piece_position(S, i >> 6, i & 63);
+    rid[i] = (uint8_t)class_region_id(S, i >> 6, i & 63);
+  }
+}
+
 // Per-class additive table in the item's tile order, in the log2 domain:
 //   tbl[i][j] = log2(e) * (bias[pos(i)][pos(j)] + (region(pos i) != region(pos j) ? -100 : 0)).
 // `bias` is this head's (64,64) fp32 table or null; `pos` the class's 64-entry tile-row -> window-position LUT;
@@ -239,15 +231,21 @@ __device__ __forceinline__ WinStart cursor_start(const WinShape& S, const ItemCu
   r.s0 = i0 * S.win[0] + S.shift[0]; r.s1 = i1 * S.win[1] + S.shift[1]; r.s2 = i2 * S.win[2] + S.shift[2];
   return r;
 }
+// Where a warp's T tensors go: map[t] = tensor t's eight per-class maps; dst_base[t] / slot_stride[t] = byte offset of its
+// tile of slot 0 inside a stage, and the stride to slot 1.
+template <int T>
+struct BoxLayout {
+  const CUtensorMap* map[T];
+  int dst_base[T], slot_stride[T];
+};
+
 template <int T>
 struct BoxPlan {
   int cls = -1, nbox = 0;
   int slot[2], o0[2], o1[2], o2[2], dst[2];
   const CUtensorMap* map[2];
 
-  // dst_base[t] / slot_stride[t]: byte offset of tensor t's tile of slot 0 inside a stage, and the stride to slot 1
-  __device__ __forceinline__ void build(const WinShape& S, int c, int lane, const CUtensorMap* const (&maps)[T], const int (&dst_base)[T],
-                                        const int (&slot_stride)[T]) {
+  __device__ __forceinline__ void build(const WinShape& S, int c, int lane, const BoxLayout<T>& L) {
     cls = c;
     const int lp = __popc(c);
     nbox = (2 * T) << lp;
@@ -266,11 +264,11 @@ struct BoxPlan {
         if (bit) qq >>= 1;
       }
       slot[r] = sl; o0[r] = off[0]; o1[r] = off[1]; o2[r] = off[2];
-      const CUtensorMap* m = maps[0];
-      int d = dst_base[0], ss = slot_stride[0];
+      const CUtensorMap* m = L.map[0];
+      int d = L.dst_base[0], ss = L.slot_stride[0];
 #pragma unroll
       for (int u = 1; u < T; ++u)
-        if (t == u) { m = maps[u]; d = dst_base[u]; ss = slot_stride[u]; }
+        if (t == u) { m = L.map[u]; d = L.dst_base[u]; ss = L.slot_stride[u]; }
       map[r] = m + c;
       dst[r] = d + sl * ss + piece * psize_bytes;
     }
@@ -294,5 +292,74 @@ struct BoxPlan {
     }
   }
 };
+
+// ------------------------------------------------------------------------------------------
+// Item descriptor ring.  Only the TMA producer knows the schedule: it publishes item n in entry n % DEPTH of a ring in
+// shared memory before the barrier arrival that hands over item n's stage, and every other warp reads its items from
+// there and stops at the end marker.  The producer may write entry n + DEPTH only once every reader of entry n is past
+// it; each kernel's pipeline depth guarantees that (see its producer).
+// Layout (kBytes): DEPTH int4 {wrap class, window of slot 0, of slot 1, valid slots}, then DEPTH x 2 int4 {sample, start
+// coordinates} of the item's two windows.
+// ------------------------------------------------------------------------------------------
+struct RingItem {
+  int cls;           // wrap class; -1 = end marker
+  int win[2];        // linear window index of slot 0, slot 1
+  int nvalid;        // valid slots: 1 for the last item of an odd class, else 2
+  WinStart ws[2];
+  __device__ __forceinline__ bool end() const { return cls < 0; }
+};
+
+template <int DEPTH>
+struct ItemRing {
+  static_assert((DEPTH & (DEPTH - 1)) == 0, "ring depth must be a power of two");
+  static constexpr int kBytes = DEPTH * 3 * 16;
+  int4* e;
+
+  __device__ __forceinline__ void publish(int n, const RingItem& it) const {
+    const int k = n & (DEPTH - 1);
+    e[k] = make_int4(it.cls, it.win[0], it.win[1], it.nvalid);
+    e[DEPTH + 2 * k] = make_int4(it.ws[0].b, it.ws[0].s0, it.ws[0].s1, it.ws[0].s2);
+    e[DEPTH + 2 * k + 1] = make_int4(it.ws[1].b, it.ws[1].s0, it.ws[1].s1, it.ws[1].s2);
+  }
+  __device__ __forceinline__ void publish_end(int n) const { e[n & (DEPTH - 1)] = make_int4(-1, 0, 0, 0); }
+  __device__ __forceinline__ RingItem read(int n) const {
+    const int k = n & (DEPTH - 1);
+    const int4 d = e[k], a0 = e[DEPTH + 2 * k], a1 = e[DEPTH + 2 * k + 1];
+    return {d.x, {d.y, d.z}, d.w, {{a0.x, a0.y, a0.z, a0.w}, {a1.x, a1.y, a1.z, a1.w}}};
+  }
+};
+
+// ------------------------------------------------------------------------------------------
+// The producer's schedule walk: body(n, item) for this CTA's items in order, numbered n = n0, n0 + 1, ...  walk_range takes
+// m items of the class-sorted list from item c0 (the deterministic backward's static range); walk_queue takes what the
+// ClassQueue hands out.  Both return the number after the last item.  The bodies (the kernels' producers) compute their
+// stage, rebuild their BoxPlan on a class change and publish the item.  They capture the parameter block, the shape and
+// the plan by reference and everything else, the box layout included, by value: with other capture lists ptxas spilled
+// more in the backward kernel, whose warps run at 56 to 104 registers.
+// ------------------------------------------------------------------------------------------
+template <class Body>
+__device__ __forceinline__ int walk_range(const WinShape& S, const Sched& sc, int c0, int m, int n0, Body&& body) {
+  ItemCursor cur;
+  cur.seek(sc, c0);
+  int n = n0;
+  for (int t = 0; t < m; ++t, ++n, cur.next_item(sc)) {
+    RingItem it;
+    it.cls = cur.cls;
+    it.nvalid = cur.slot_valid(1) ? 2 : 1;
+    it.ws[0] = cursor_start(S, cur, 0, it.win[0]);
+    it.ws[1] = cursor_start(S, cur, 1, it.win[1]);
+    body(n, it);
+  }
+  return n;
+}
+
+template <class Body>
+__device__ __forceinline__ int walk_queue(const WinShape& S, const Sched& sc, int home_item, int* work, int chunk, int lane, Body&& body) {
+  ClassQueue wq;
+  wq.init(sc, home_item, work, chunk, lane);
+  int n = 0;
+  for (int c0, m; wq.next(sc, work, chunk, lane, c0, m);) n = walk_range(S, sc, c0, m, n, body);
+  return n;
+}
 
 }}  // namespace mmn::tc

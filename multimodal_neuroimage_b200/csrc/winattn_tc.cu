@@ -1,4 +1,5 @@
-// winattn_tc.cu -- translation unit of the tcgen05 / TMEM / TMA window-attention kernels.
+// winattn_tc.cu -- translation unit of the tcgen05 / TMEM / TMA window-attention kernels: their host entry points
+// (winattn_tc.h) are defined in winattn_tc_fwd.cuh, winattn_tc_qkv_fwd.cuh and winattn_tc_bwd.cuh.
 #include "winattn_tc.h"
 
 #include "winattn_tc_bwd.cuh"
@@ -68,32 +69,6 @@ bool make_window_maps(CUtensorMap* out, const void* ptr, long long row_stride, i
   for (int c = 0; c < 8; ++c) slot.maps[c] = out[c];
   slot.valid = true;
   return true;
-}
-
-const char* fwd_why_not(const mmn_winattn_desc* d) { return fwd_why_not_impl(d); }
-const char* bwd_why_not(const mmn_winattn_desc* d) { return bwd_why_not_impl(d); }
-
-int winattn_fwd(const mmn_winattn_desc* d, const void* q, const void* k, const void* v, const float* bias,
-                const float* head_scale, const float* mask, void* out, float* lse, void* workspace, cudaStream_t st, char* err,
-                size_t errlen) {
-  return winattn_fwd_launch(d, q, k, v, bias, head_scale, mask, out, lse, workspace, st, err, errlen);
-}
-
-int winattn_bwd(const mmn_winattn_desc* d, const void* q, const void* k, const void* v, const float* bias,
-                const float* head_scale, const float* mask, const void* /*out*/, const float* lse, const void* dout, void* dq,
-                void* dk, void* dv, float* dbias, float* dhead_scale, float* dcolsum, float* workspace, cudaStream_t st,
-                char* err, size_t errlen, int* launches) {
-  return winattn_bwd_launch(d, q, k, v, bias, head_scale, mask, lse, dout, dq, dk, dv, dbias, dhead_scale, dcolsum, workspace, st, err, errlen,
-                            launches);
-}
-
-size_t bwd_det_workspace_bytes(const mmn_winattn_desc* d) { return bwd_det_workspace_bytes_impl(d); }
-
-const char* qkv_fwd_why_not(const mmn_winattn_desc* d, int in_channels) { return qkv_fwd_why_not_impl(d, in_channels); }
-
-int winattn_qkv_fwd(const mmn_winattn_desc* d, const void* x, const void* w, const float* b, const float* bias, const float* head_scale,
-                    const float* mask, void* qkv, void* out, float* lse, void* workspace, cudaStream_t st, char* err, size_t errlen) {
-  return winattn_qkv_fwd_launch(d, x, w, b, bias, head_scale, mask, qkv, out, lse, workspace, st, err, errlen);
 }
 
 }}  // namespace mmn::tc

@@ -1,4 +1,4 @@
-// winattn_tc.h -- host entry points of the tcgen05 window-attention kernels (winattn_tc.cu).
+// winattn_tc.h -- host entry points of the tcgen05 kernels.
 #pragma once
 #include <cuda_runtime.h>
 #include <stddef.h>

@@ -36,24 +36,16 @@ namespace mmn { namespace tc {
 constexpr int kStagesB = 3;
 constexpr int kStageBytesB = 2 * kQRegion + 2 * kTile;   // Q0|Z|Q1, K0 K1, V0 V1, dO0|Z|dO1
 constexpr int kOffK = kQRegion, kOffV = kQRegion + kTile, kOffDO = kQRegion + 2 * kTile;
-#ifndef MMN_BWD_KEYS_PER_THREAD
-#define MMN_BWD_KEYS_PER_THREAD 16
-#endif
-constexpr int kKeysPerThread = MMN_BWD_KEYS_PER_THREAD;     // 16: four threads per query row; 32: two
-constexpr int kRowSplit = kN / kKeysPerThread;
-constexpr int kSoftmaxThreadsB = 128 * kRowSplit, kEpiThreads = 128;
+constexpr int kKeysPerThread = 16;                          // four softmax threads per query row
+constexpr int kSoftmaxThreadsB = 4 * 128, kEpiThreads = 128;
 constexpr int kEpiWarp0 = kSoftmaxThreadsB / 32, kProducerWarpB = kEpiWarp0 + 4, kMmaWarpB = kEpiWarp0 + 5, kStoreWarpB = kEpiWarp0 + 6;
 constexpr int kColsumWarpB = kEpiWarp0 + 7;
 constexpr int kBwdThreads = kSoftmaxThreadsB + 256;
-// register budget by warpgroup (setmaxnreg only moves registers inside the CTA's launch allocation):
-//   4 threads/row: launch 80 -> softmax 80, epilogue 104, the rest 56     (512*80 + 128*104 + 128*56 = 768*80)
-//   2 threads/row: launch 128 -> softmax 168, epilogue 112, the rest 64   (256*168 + 128*112 + 128*64 = 512*128)
-constexpr int kRegLaunch = kRowSplit == 4 ? 80 : 128;
-constexpr int kRegSoftmax = kRowSplit == 4 ? 80 : 168, kRegEpi = kRowSplit == 4 ? 104 : 112, kRegAux = kRowSplit == 4 ? 56 : 64;
-#ifndef MMN_BWD_CHUNK
-#define MMN_BWD_CHUNK 1
-#endif
-constexpr int kChunkB = MMN_BWD_CHUNK;  // items a CTA claims per atomic
+// register budget by warpgroup (setmaxnreg only moves registers inside the CTA's launch allocation of 80):
+//   softmax 80, epilogue 104, the rest 56     (512*80 + 128*104 + 128*56 = 768*80)
+constexpr int kRegEpi = 104, kRegAux = 56;
+constexpr int kChunkB = 1;            // items a CTA claims per atomic
+constexpr int kItemRingB = 8;         // descriptor ring: entry n + 8 is written once the epilogue has handed back item n + 5's stage
 constexpr int kPDBytes = 7 * 8192;    // P0[2] | dS'0 | Z | dS'1 | P1[2]
 constexpr int kBwdTmemCols = 512;     // S[b] at 128 b, dP[b] at 128 b + 64; dV|dQ~|dK~ [b] at 256 + 96 b
 
@@ -106,9 +98,8 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
   float* sRed = sDelta + 512;                             // 16 floats: dhead_scale per softmax warp
   uint8_t* sPos = reinterpret_cast<uint8_t*>(sRed + 16);  // [8][64]
   uint8_t* sRid = sPos + 512;                             // [8][64] window position -> shift-mask region id
-  int4* sItem = reinterpret_cast<int4*>(sRid + 512);      // [8] ring: {wrap class (-1: no more items), window index of slot 0, of slot 1, valid slots} of item n & 7
-  int4* sGeo = sItem + 8;                                 // [8][2] ring: {sample, start coordinates} of the item's two windows (store warp)
-  int* sEnd = reinterpret_cast<int*>(sGeo + 16);          // [0] items of this CTA once the epilogue warps know (else INT_MAX)
+  const ItemRing<kItemRingB> ring{reinterpret_cast<int4*>(sRid + 512)};      // item descriptors (tc_sched.cuh)
+  int* sEnd = reinterpret_cast<int*>(sRid + 512 + ring.kBytes);  // [0] items of this CTA once the epilogue warps know (else INT_MAX)
   uint64_t* bars = reinterpret_cast<uint64_t*>(sEnd + 4);
   uint64_t* full = bars;                                  // [kStagesB]
   uint64_t* empty = bars + kStagesB;                      // [kStagesB] (one arrival per warp: epilogue threads)
@@ -130,10 +121,7 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
   // ---- one-time setup
   for (int i = tid; i < (kStagesB * kStageBytesB + kPDBytes) / 16; i += kBwdThreads)
     reinterpret_cast<uint4*>(smem)[i] = make_uint4(0, 0, 0, 0);
-  for (int i = tid; i < 512; i += kBwdThreads) {
-    sPos[i] = (uint8_t)piece_position(S, i >> 6, i & 63);
-    sRid[i] = (uint8_t)class_region_id(S, i >> 6, i & 63);
-  }
+  fill_class_luts(S, sPos, sRid, tid, kBwdThreads);
   for (int i = tid; i < kStagesB * 2 * 3 * kN; i += kBwdThreads) sRec[i] = 0.f;
   if (tid == 0) {
     sEnd[0] = 0x7fffffff;
@@ -164,61 +152,44 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
       // ============================== TMA producer (schedule, descriptor ring, tiles, records) ==============================
       // every lane runs the loop; lane l issues boxes l, l + 32 of the item (BoxPlan: which map, piece offset and
       // shared-memory offset a lane's boxes have depends only on the wrap class)
-      const CUtensorMap* const maps[4] = {P.q, P.dout, P.k, P.v};
-      const int dst_base[4] = {0, kOffDO, kOffK, kOffV};
-      const int slot_stride[4] = {2 * kWinBytes, 2 * kWinBytes, kWinBytes, kWinBytes};
+      const BoxLayout<4> lay{{P.q, P.dout, P.k, P.v}, {0, kOffDO, kOffK, kOffV}, {2 * kWinBytes, 2 * kWinBytes, kWinBytes, kWinBytes}};
       BoxPlan<4> plan;
       // Dynamic schedule (see the forward kernel's producer): chunks of kChunkB items of this head's class-sorted list
-      // through an atomic counter; every other warp follows the descriptor rings sItem / sGeo.  One end marker.
+      // through an atomic counter; every other warp follows the descriptor ring.  One end marker.
       // (An L2 prefetch of item n + 1's boxes issued right after item n's loads made the kernel 33 % SLOWER, 0.46 -> 0.61 ms:
       // the extra boxes queue in the SM's TMA unit in front of the next loads and the gradient stores.)
-      int n = 0;
-      // one item: descriptor ring (sItem is published by the arrival on full[stage]), tiles, and per slot (lane = slot)
-      // the window's record of norms and lse, already in tile row order.  The same in both schedules.
-#define MMN_BWD_LOAD_ITEM(cur)                                                                                           \
-  do {                                                                                                                 \
-    const int stage = n % kStagesB, phase = (n / kStagesB) & 1;                                                       \
-    if ((cur).cls != plan.cls) plan.build(S, (cur).cls, lane, maps, dst_base, slot_stride);                           \
-    const int nvalid = (cur).slot_valid(1) ? 2 : 1;                                                                   \
-    int w0, w1;                                                                                                       \
-    const WinStart ws0 = cursor_start(S, cur, 0, w0), ws1 = cursor_start(S, cur, 1, w1);                              \
-    trace_ev(P.trace, 2, n, 0);                                                                                       \
-    mbar_wait(&empty[stage], phase ^ 1);                                                                              \
-    trace_ev(P.trace, 2, n, 1);                                                                                       \
-    if (lane == 0) {                                                                                                  \
-      sItem[n & 7] = make_int4((cur).cls, w0, w1, nvalid);                                                          \
-      sGeo[(n & 7) * 2] = make_int4(ws0.b, ws0.s0, ws0.s1, ws0.s2);                                                   \
-      sGeo[(n & 7) * 2 + 1] = make_int4(ws1.b, ws1.s0, ws1.s1, ws1.s2);                                               \
-      mbar_arrive_expect_tx(&full[stage], nvalid * (4 * kWinBytes + 3 * kN * 4));                                     \
-    }                                                                                                                 \
-    __syncwarp();                                                                                                     \
-    plan.issue<true>(S, ws0, ws1, nvalid, h * kD, sStage + stage * kStageBytesB, &full[stage], lane);                 \
-    if (lane < nvalid)                                                                                                \
-      bulk_load_1d(sRec + (stage * 2 + lane) * (3 * kN), P.lse + P.slab + ((long long)(lane ? w1 : w0) * P.nH + h) * (3 * kN),\
-                   3 * kN * 4, &full[stage]);                                                                         \
-    trace_ev(P.trace, 2, n, 2);                                                                                       \
-  } while (0)
-      if (DET) {
-        const int k = blockIdx.x / P.nH, end = sched_range_begin(sc, k + 1, P.per_head);
-        int it = sched_range_begin(sc, k, P.per_head);
-        ItemCursor cur;
-        cur.seek(sc, it);
-        for (; it < end; ++it, ++n, cur.next_item(sc)) MMN_BWD_LOAD_ITEM(cur);
-      } else {
-        ClassQueue wq;
-        wq.init(sc, sched_range_begin(sc, blockIdx.x / P.nH, P.per_head), P.work + h * 8, kChunkB, lane);
-        for (int c0, m; wq.next(sc, P.work + h * 8, kChunkB, lane, c0, m);) {
-          ItemCursor cur;
-          cur.seek(sc, c0);
-          for (int t = 0; t < m; ++t, ++n, cur.next_item(sc)) MMN_BWD_LOAD_ITEM(cur);
+      // One item: descriptor (published by the arrival on full[stage]), tiles, and per slot (lane = slot) the window's
+      // record of norms and lse, already in tile row order.  The same in both schedules.
+      auto load_item = [=, &P, &S, &plan](int n, const RingItem& it) {
+        const int stage = n % kStagesB, phase = (n / kStagesB) & 1;
+        if (it.cls != plan.cls) plan.build(S, it.cls, lane, lay);
+        trace_ev(P.trace, 2, n, 0);
+        mbar_wait(&empty[stage], phase ^ 1);
+        trace_ev(P.trace, 2, n, 1);
+        if (lane == 0) {
+          ring.publish(n, it);
+          mbar_arrive_expect_tx(&full[stage], it.nvalid * (4 * kWinBytes + 3 * kN * 4));
         }
+        __syncwarp();
+        plan.issue<true>(S, it.ws[0], it.ws[1], it.nvalid, h * kD, sStage + stage * kStageBytesB, &full[stage], lane);
+        if (lane < it.nvalid)
+          bulk_load_1d(sRec + (stage * 2 + lane) * (3 * kN), P.lse + P.slab + ((long long)(lane ? it.win[1] : it.win[0]) * P.nH + h) * (3 * kN),
+                       3 * kN * 4, &full[stage]);
+        trace_ev(P.trace, 2, n, 2);
+      };
+      const int k = blockIdx.x / P.nH;
+      int n;
+      if (DET) {
+        const int begin = sched_range_begin(sc, k, P.per_head);
+        n = walk_range(S, sc, begin, sched_range_begin(sc, k + 1, P.per_head) - begin, 0, load_item);
+      } else {
+        n = walk_queue(S, sc, sched_range_begin(sc, k, P.per_head), P.work + h * 8, kChunkB, lane, load_item);
       }
-#undef MMN_BWD_LOAD_ITEM
       {   // end marker
         const int stage = n % kStagesB, phase = (n / kStagesB) & 1;
         mbar_wait(&empty[stage], phase ^ 1);
         if (lane == 0) {
-          sItem[n & 7] = make_int4(-1, 0, 0, 0);
+          ring.publish_end(n);
           mbar_arrive(&full[stage]);
         }
         __syncwarp();
@@ -240,7 +211,7 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
       auto issue_sdp = [&](int n) {
         const int stage = n % kStagesB, phase = (n / kStagesB) & 1, b = n & 1;
         mbar_wait(&full[stage], phase);
-        if (sItem[n & 7].x < 0) { total = n; return; }
+        if (ring.read(n).end()) { total = n; return; }
         mbar_wait(&sdp_empty[b], ((n >> 1) & 1) ^ 1);
         tcgen05_fence_after();
         trace_ev(P.trace, 3, n - 2, 4);
@@ -305,29 +276,23 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
       // The three staging tiles (dq, dk, dv) are handed over one by one, so the epilogue warps fill the next
       // tile while this one drains.  Each lane issues its share of a tile's boxes; a tile is returned to the
       // epilogue once the bulk group two behind has finished reading shared memory.
-      const CUtensorMap* const maps[1] = {P.dq};        // dq[8] | dk[8] | dv[8] are contiguous in BwdParams: tensor t's maps are 8 t further
-      const int dst_base[1] = {0};
-      const int slot_stride[1] = {kWinBytes};
+      const BoxLayout<1> lay{{P.dq}, {0}, {kWinBytes}};   // dq[8] | dk[8] | dv[8] are contiguous in BwdParams: tensor t's maps are 8 t further
       BoxPlan<1> plan;
       int grp = 0;
       bool done = false;
       for (int n = 0; !done; ++n) {
-        WinStart w0, w1;
-        int nvalid = 0;
+        RingItem it;
 #pragma unroll
         for (int t = 0; t < 3; ++t, ++grp) {
           if (t == 0) trace_ev(P.trace, 4, n, 0);
           mbar_wait(&so_ready[t], n & 1);
           if (t == 0) {
             if (n >= *reinterpret_cast<volatile int*>(sEnd)) { done = true; break; }   // that arrival was the epilogue warps' farewell
-            const int4 it = sItem[n & 7], a0 = sGeo[(n & 7) * 2], a1 = sGeo[(n & 7) * 2 + 1];
-            nvalid = it.w;
-            if (it.x != plan.cls) plan.build(S, it.x, lane, maps, dst_base, slot_stride);
-            w0.b = a0.x; w0.s0 = a0.y; w0.s1 = a0.z; w0.s2 = a0.w;
-            w1.b = a1.x; w1.s0 = a1.y; w1.s1 = a1.z; w1.s2 = a1.w;
+            it = ring.read(n);
+            if (it.cls != plan.cls) plan.build(S, it.cls, lane, lay);
             trace_ev(P.trace, 4, n, 1);
           }
-          plan.issue<false>(S, w0, w1, nvalid, h * kD, sOut + t * kTile, nullptr, lane, 8 * t);
+          plan.issue<false>(S, it.ws[0], it.ws[1], it.nvalid, h * kD, sOut + t * kTile, nullptr, lane, 8 * t);
           tma_store_commit();
           tma_store_wait_read<2>();        // per thread: the group two behind (tile (t + 1) % 3) has been read out
           __syncwarp();
@@ -392,7 +357,7 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
     const int slot = r >> 6, i = r & 63;
     const uint32_t lane_base = (uint32_t)((warp & 3) * 32) << 16;
     const int rsw = (r >> 1) & 3;                       // 64B-swizzle phase of this thread's tile row
-    if (kRegEpi > kRegLaunch) setmaxnreg_inc<kRegEpi>(); else if (kRegEpi < kRegLaunch) setmaxnreg_dec<kRegEpi>();
+    setmaxnreg_inc<kRegEpi>();
     float dscale_acc = 0.f;                             // sum over rows of q_i . dQ~_i = sum_ij dS_ij (s_ij - bias_ij)
     const float inv_hscale = COS ? 1.f / __ldg(P.head_scale + h) : 1.f;
     int n = 0;
@@ -404,7 +369,7 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
       mbar_wait(&out_full[b], (n >> 1) & 1);
       if (n >= *reinterpret_cast<volatile int*>(sEnd)) break;      // that arrival was the MMA warp's farewell
       tcgen05_fence_after();
-      const bool valid = slot < sItem[n & 7].w;
+      const bool valid = slot < ring.read(n).nvalid;
       if (warp == kEpiWarp0) trace_ev(P.trace, 1, n, 1);
 
       // Everything this item still needs from its stage -- this thread's q and k rows and their norms (ring slot n % 3,
@@ -491,8 +456,7 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
       }
     }
   } else {
-    // ============================== softmax (512 threads: 4 per row, 16 keys each) ==============================
-    if (kRegSoftmax > kRegLaunch) setmaxnreg_inc<kRegSoftmax>();
+    // ============================== softmax (512 threads: 4 per row, 16 keys each; registers as launched) ==============================
     constexpr int KP = kKeysPerThread;
     const int r = tid & 127, qt = tid >> 7;             // tile row; which quarter of its 64 keys
     const int slot = r >> 6, i = r & 63;
@@ -553,10 +517,10 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
       const int b = n & 1, stage = n % kStagesB;
       TRB(n, 0);
       mbar_wait(&full[stage], (n / kStagesB) & 1);
-      const int4 item = sItem[n & 7];                   // written by the producer before it armed full[stage]
-      if (item.x < 0) break;                            // end marker
-      const int cls = item.x;
-      const bool valid = slot < item.w;
+      const RingItem item = ring.read(n);               // written by the producer before it armed full[stage]
+      if (item.end()) break;
+      const int cls = item.cls;
+      const bool valid = slot < item.nvalid;
       const float* rec = sRec + (stage * 2 + slot) * (3 * kN);
       const float lse2 = valid ? rec[2 * kN + i] : 0.f;
       if (cls != cls_loaded) {                          // rare: at most 8 times per CTA
@@ -580,7 +544,7 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
         const float4* trow = reinterpret_cast<const float4*>(sTbl + i * kTblLd + qt * KP);
         const float* mrow = nullptr;
         if (MASK == MMN_MASK_TENSOR) {
-          const int gw = slot ? item.z : item.y, ipos = sPos[cls * 64 + i];
+          const int gw = slot ? item.win[1] : item.win[0], ipos = sPos[cls * 64 + i];
           mrow = P.mask + ((size_t)(gw % P.mask_windows) * kN + ipos) * kN + qt * KP;
         }
 #pragma unroll
@@ -638,7 +602,7 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
       named_bar_sync(2, kSoftmaxThreadsB);
       TRB(n, 7);
       delta = sDelta[r] + sDelta[128 + r];
-      if (kRowSplit == 4) delta += sDelta[256 + r] + sDelta[384 + r];
+      delta += sDelta[256 + r] + sDelta[384 + r];
 
       // ---- (d) dS = P o (dP - delta): dbias; dS' = dS o c into the MMA tile; d(logit scale)
       {
@@ -693,7 +657,7 @@ winattn_bwd_tc_kernel(const __grid_constant__ BwdParams P) {
 }
 
 constexpr size_t kBwdSmemBytes = 1024 + kStagesB * kStageBytesB + kPDBytes + 3 * kTile + kN * kTblLd * 4 +
-                                 (kStagesB * 2 * 3 * kN + 512 + 16) * 4 + 1024 + 24 * 16 + 16 + 24 * 8;
+                                 (kStagesB * 2 * 3 * kN + 512 + 16) * 4 + 1024 + ItemRing<kItemRingB>::kBytes + 16 + 24 * 8;
 
 // Deterministic mode, second launch: for each head, the per_head slots of its CTAs summed in CTA order and added into dbias,
 // dcolsum and dhead_scale (each may be null).  Block = 128 slot entries (one float4 per lane) x 32 slices of the CTA range,
@@ -748,37 +712,34 @@ winattn_bwd_det_reduce(const float* __restrict__ part, int per_head, int nH, flo
 inline int bwd_ctas_per_head(const WinShape& S, const mmn_winattn_desc* d) {
   int per_head = num_sms_cached() / d->num_heads;
   if (per_head < 1) per_head = 1;
-  const int n_items = make_sched(S, d->batch, true).n_items;
+  const int n_items = make_sched(S, d->batch).n_items;
   return per_head > n_items ? n_items : per_head;
 }
 
-inline size_t bwd_det_workspace_bytes_impl(const mmn_winattn_desc* d) {
+size_t bwd_det_workspace_bytes(const mmn_winattn_desc* d) {
   return (size_t)bwd_ctas_per_head(shape_from(d), d) * d->num_heads * kDetSlotFloats * sizeof(float);
 }
 
-inline const char* bwd_why_not_impl(const mmn_winattn_desc* d) {
-  const char* w = fwd_why_not_impl(d);
+const char* bwd_why_not(const mmn_winattn_desc* d) {
+  const char* w = fwd_why_not(d);
   if (w) return w;
   if (d->do_row_stride % 8 || d->dq_row_stride % 8 || d->dk_row_stride % 8 || d->dv_row_stride % 8) return "gradient row stride not 16-byte aligned";
   return nullptr;
 }
 
-inline int winattn_bwd_launch(const mmn_winattn_desc* d, const void* q, const void* k, const void* v, const float* bias,
-                              const float* head_scale, const float* mask, const float* lse, const void* dout, void* dq, void* dk,
-                              void* dv, float* dbias, float* dhead_scale, float* dcolsum, void* workspace, cudaStream_t st, char* err, size_t errlen,
-                              int* launches) {
+int winattn_bwd(const mmn_winattn_desc* d, const void* q, const void* k, const void* v, const float* bias, const float* head_scale,
+                const float* mask, const void* /*out*/, const float* lse, const void* dout, void* dq, void* dk, void* dv, float* dbias,
+                float* dhead_scale, float* dcolsum, float* workspace, cudaStream_t st, char* err, size_t errlen, int* launches) {
   BwdParams P;
   P.S = shape_from(d);
-  P.sc = make_sched(P.S, d->batch, true);
+  P.sc = make_sched(P.S, d->batch);
   const int C = d->num_heads * d->head_dim;
   const int B = d->batch;
   if (!make_window_maps(P.q, q, d->q_row_stride, B, C, P.S) || !make_window_maps(P.k, k, d->k_row_stride, B, C, P.S) ||
       !make_window_maps(P.v, v, d->v_row_stride, B, C, P.S) || !make_window_maps(P.dout, dout, d->do_row_stride, B, C, P.S) ||
       !make_window_maps(P.dq, dq, d->dq_row_stride, B, C, P.S) || !make_window_maps(P.dk, dk, d->dk_row_stride, B, C, P.S) ||
-      !make_window_maps(P.dv, dv, d->dv_row_stride, B, C, P.S)) {
-    snprintf(err, errlen, "cuTensorMapEncodeTiled failed (pointer alignment or strides)");
-    return MMN_ERR_CUDA;
-  }
+      !make_window_maps(P.dv, dv, d->dv_row_stride, B, C, P.S))
+    return tensor_map_failed(err, errlen);
   P.nH = d->num_heads;
   P.mask_windows = d->mask_windows > 0 ? d->mask_windows : 1;
   P.scale = d->scale;
@@ -792,7 +753,7 @@ inline int winattn_bwd_launch(const mmn_winattn_desc* d, const void* q, const vo
   P.part = nullptr;
   if (det) {                                           // static schedule: no counters; the workspace holds the CTA slots
     if (!workspace || reinterpret_cast<uintptr_t>(workspace) % 16) { snprintf(err, errlen, "workspace missing or misaligned"); return MMN_ERR_CUDA; }
-    P.part = static_cast<float*>(workspace);
+    P.part = workspace;
   } else {
     P.work = arm_work_counters(workspace, st, err, errlen);
     if (!P.work) return MMN_ERR_CUDA;
@@ -800,31 +761,21 @@ inline int winattn_bwd_launch(const mmn_winattn_desc* d, const void* q, const vo
   const char* trace_path = getenv("MMN_TC_TRACE_BWD");
   P.trace = trace_setup(trace_path, st);
 
-  using Kern = void (*)(const BwdParams);
-  static const Kern kernels[2][2][3] = {
-      {{winattn_bwd_tc_kernel<false, MMN_MASK_NONE, false>, winattn_bwd_tc_kernel<false, MMN_MASK_SHIFT, false>, winattn_bwd_tc_kernel<false, MMN_MASK_TENSOR, false>},
-       {winattn_bwd_tc_kernel<true, MMN_MASK_NONE, false>, winattn_bwd_tc_kernel<true, MMN_MASK_SHIFT, false>, winattn_bwd_tc_kernel<true, MMN_MASK_TENSOR, false>}},
-      {{winattn_bwd_tc_kernel<false, MMN_MASK_NONE, true>, winattn_bwd_tc_kernel<false, MMN_MASK_SHIFT, true>, winattn_bwd_tc_kernel<false, MMN_MASK_TENSOR, true>},
-       {winattn_bwd_tc_kernel<true, MMN_MASK_NONE, true>, winattn_bwd_tc_kernel<true, MMN_MASK_SHIFT, true>, winattn_bwd_tc_kernel<true, MMN_MASK_TENSOR, true>}}};
-  static std::once_flag once;
-  std::call_once(once, [] {
-    for (int t = 0; t < 2; ++t)
-      for (int c = 0; c < 2; ++c)
-        for (int m = 0; m < 3; ++m) cudaFuncSetAttribute(kernels[t][c][m], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmemBytes);
-  });
-  const Kern kern = kernels[det ? 1 : 0][d->score_kind == MMN_SCORE_COSINE ? 1 : 0][d->mask_kind];
+  // [deterministic][cosine][mask kind]
+  static void (*const kernels[12])(BwdParams) = {
+      winattn_bwd_tc_kernel<false, MMN_MASK_NONE, false>, winattn_bwd_tc_kernel<false, MMN_MASK_SHIFT, false>, winattn_bwd_tc_kernel<false, MMN_MASK_TENSOR, false>,
+      winattn_bwd_tc_kernel<true, MMN_MASK_NONE, false>, winattn_bwd_tc_kernel<true, MMN_MASK_SHIFT, false>, winattn_bwd_tc_kernel<true, MMN_MASK_TENSOR, false>,
+      winattn_bwd_tc_kernel<false, MMN_MASK_NONE, true>, winattn_bwd_tc_kernel<false, MMN_MASK_SHIFT, true>, winattn_bwd_tc_kernel<false, MMN_MASK_TENSOR, true>,
+      winattn_bwd_tc_kernel<true, MMN_MASK_NONE, true>, winattn_bwd_tc_kernel<true, MMN_MASK_SHIFT, true>, winattn_bwd_tc_kernel<true, MMN_MASK_TENSOR, true>};
   P.per_head = bwd_ctas_per_head(P.S, d);
-  kern<<<P.per_head * P.nH, kBwdThreads, kBwdSmemBytes, st>>>(P);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) {
-    snprintf(err, errlen, "winattn_bwd_tc_kernel: %s", cudaGetErrorString(e));
-    return MMN_ERR_CUDA;
-  }
+  const int rc = launch_variant(kernels, (det ? 6 : 0) + (d->score_kind == MMN_SCORE_COSINE ? 3 : 0) + d->mask_kind, kBwdSmemBytes,
+                                P.per_head * P.nH, kBwdThreads, P, st, "winattn_bwd_tc_kernel", err, errlen);
+  if (rc != MMN_OK) return rc;
   ++*launches;
   if (det && (P.dbias || P.dhead_scale || P.dcolsum)) {
     winattn_bwd_det_reduce<<<dim3((kDetSlotFloats / 4 + 31) / 32, P.nH), kDetRedSlices * 32, 0, st>>>(P.part, P.per_head, P.nH, P.dbias,
                                                                                                     P.dcolsum, P.dhead_scale);
-    e = cudaGetLastError();
+    const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {
       snprintf(err, errlen, "winattn_bwd_det_reduce: %s", cudaGetErrorString(e));
       return MMN_ERR_CUDA;

@@ -33,6 +33,7 @@
 #include <mutex>
 
 #include "tc_sched.cuh"
+#include "winattn_tc.h"
 #include "zero_fill.h"
 
 namespace mmn { namespace tc {
@@ -211,9 +212,8 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
   float* sRk = sTbl + G * kN * kTblLd;                    // [G][2][128] per-key 1/||k|| (double-buffered over the group's items)
   uint8_t* sPos = reinterpret_cast<uint8_t*>(sRk + G * 256);  // [8 wrap classes][64]: tile row -> window position
   uint8_t* sRid = sPos + 512;                             // [8 wrap classes][64]: window position -> shift-mask region id
-  int4* sItem = reinterpret_cast<int4*>(sRid + 512);      // [kItemRing] {wrap class (-1: no more items), window of slot 0, of slot 1, valid slots}
-  int4* sGeo = sItem + kItemRing;                         // [kItemRing][2] {sample, start coordinates} of the item's two windows (store warp)
-  int* sEnd = reinterpret_cast<int*>(sGeo + 2 * kItemRing);  // [G] items group g has produced when it left its loop (else INT_MAX)
+  const ItemRing<kItemRing> ring{reinterpret_cast<int4*>(sRid + 512)};      // item descriptors (tc_sched.cuh)
+  int* sEnd = reinterpret_cast<int*>(sRid + 512 + ring.kBytes);   // [G] items group g has produced when it left its loop (else INT_MAX)
   uint64_t* bars = reinterpret_cast<uint64_t*>(sEnd + 4);
   uint64_t* full = bars;                                  // [kStagesF] TMA -> MMA, softmax
   uint64_t* empty = bars + kStagesF;                      // [kStagesF] MMA -> TMA
@@ -234,10 +234,7 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
   // not hold NaN bit patterns, because cross terms multiply stale tiles by the zero blocks)
   for (int i = tid; i < (kStagesF * kStageBytesF) / 16; i += kFwdThreads)
     reinterpret_cast<uint4*>(smem)[i] = make_uint4(0, 0, 0, 0);
-  for (int i = tid; i < 512; i += kFwdThreads) {
-    sPos[i] = (uint8_t)piece_position(S, i >> 6, i & 63);
-    sRid[i] = (uint8_t)class_region_id(S, i >> 6, i & 63);
-  }
+  fill_class_luts(S, sPos, sRid, tid, kFwdThreads);
   if (tid == 0) {
     for (int g = 0; g < G; ++g) sEnd[g] = 0x7fffffff;
     for (int s = 0; s < kStagesF; ++s) { mbar_init(&full[s], 2); mbar_init(&empty[s], 1); mbar_init(&desc_ready[s], 1); }
@@ -268,50 +265,37 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
       // every lane runs the loop; lane l issues boxes l, l + 32 of the item (BoxPlan).  The K and V tiles of the same items
       // are issued by a second warp that follows the descriptor ring (one warp issuing all six boxes of an item, ~65
       // cycles per box plus the cursor arithmetic, was what bounded the kernel).
-      const CUtensorMap* const maps[1] = {P.q};
-      const int dst_base[1] = {0};
-      const int slot_stride[1] = {2 * kWinBytes};
+      const BoxLayout<1> lay{{P.q}, {0}, {2 * kWinBytes}};
       BoxPlan<1> plan;
       // Dynamic schedule (tc_sched.cuh: ClassQueue): chunks of kChunkF items of this head, home class first.
-      // Every other warp learns its items from the descriptor ring sItem (published by the full[] arrival).  Ring
+      // Every other warp learns its items from the descriptor ring (published by the full[] arrival).  Ring
       // depth: entry n + 16 is written only once stage (n + 16) % kStagesF is free, i.e. after PV(n + 11) has completed,
       // so its group has long finished item n + 8 and with it waited for the store of item n + 5 (so_free): every
       // consumer of entry n, the store warp included, has read it.
-      int n = 0;
-      ClassQueue wq;
+      auto load_item = [=, &P, &S, &plan](int n, const RingItem& it) {
+        const int stage = n % kStagesF, phase = (n / kStagesF) & 1;
+        if (it.cls != plan.cls) plan.build(S, it.cls, lane, lay);
+        trace_evf(P.trace, 2, n, 0);
+        mbar_wait(&empty[stage], phase ^ 1);
+        trace_evf(P.trace, 2, n, 1);
+        if (lane == 0) {
+          ring.publish(n, it);                                          // published by the arrivals below
+          mbar_arrive(&desc_ready[stage]);
+          mbar_arrive_expect_tx(&full[stage], it.nvalid * kWinBytes);
+        }
+        __syncwarp();
+        plan.issue<true>(S, it.ws[0], it.ws[1], it.nvalid, h * kD, sStage + stage * kStageBytesF, &full[stage], lane);
+        trace_evf(P.trace, 2, n, 2);
+      };
       // claims of up to kChunkF items (each costs the producer a seek with integer divisions), an eighth of a CTA's share at most
       const int chunk = max(1, min(kChunkF, sc.n_items / (P.per_head * 8)));
-      wq.init(sc, sched_range_begin(sc, blockIdx.x / P.nH, P.per_head), P.work + h * 8, chunk, lane);
-      for (int c0, m; wq.next(sc, P.work + h * 8, chunk, lane, c0, m);) {
-        ItemCursor cur;
-        cur.seek(sc, c0);
-        for (int t = 0; t < m; ++t, ++n, cur.next_item(sc)) {
-          const int stage = n % kStagesF, phase = (n / kStagesF) & 1;
-          if (cur.cls != plan.cls) plan.build(S, cur.cls, lane, maps, dst_base, slot_stride);
-          const int nvalid = cur.slot_valid(1) ? 2 : 1;
-          int w0, w1;
-          const WinStart ws0 = cursor_start(S, cur, 0, w0), ws1 = cursor_start(S, cur, 1, w1);
-          trace_evf(P.trace, 2, n, 0);
-          mbar_wait(&empty[stage], phase ^ 1);
-          trace_evf(P.trace, 2, n, 1);
-          if (lane == 0) {
-            sItem[n % kItemRing] = make_int4(cur.cls, w0, w1, nvalid);     // published by the arrivals below
-            sGeo[(n % kItemRing) * 2] = make_int4(ws0.b, ws0.s0, ws0.s1, ws0.s2);
-            sGeo[(n % kItemRing) * 2 + 1] = make_int4(ws1.b, ws1.s0, ws1.s1, ws1.s2);
-            mbar_arrive(&desc_ready[stage]);
-            mbar_arrive_expect_tx(&full[stage], nvalid * kWinBytes);
-          }
-          __syncwarp();
-          plan.issue<true>(S, ws0, ws1, nvalid, h * kD, sStage + stage * kStageBytesF, &full[stage], lane);
-          trace_evf(P.trace, 2, n, 2);
-        }
-      }
+      int n = walk_queue(S, sc, sched_range_begin(sc, blockIdx.x / P.nH, P.per_head), P.work + h * 8, chunk, lane, load_item);
       // one end marker per softmax group (the MMA warp stops at the first)
       for (int e = 0; e < G; ++e, ++n) {
         const int stage = n % kStagesF, phase = (n / kStagesF) & 1;
         mbar_wait(&empty[stage], phase ^ 1);
         if (lane == 0) {
-          sItem[n % kItemRing] = make_int4(-1, 0, 0, 0);
+          ring.publish_end(n);
           mbar_arrive(&desc_ready[stage]);
           mbar_arrive(&full[stage]);
         }
@@ -338,7 +322,7 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
           const int stage = ns % kStagesF, phase = (ns / kStagesF) & 1;
           if (mbar_test(&full[stage], phase)) {
             progressed = true;
-            if (sItem[ns % kItemRing].x < 0) {
+            if (ring.read(ns).end()) {
               total = ns;
             } else {
               tcgen05_fence_after();
@@ -380,9 +364,7 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
       }
     } else if (warp == kStoreWarp) {
       // ============================== TMA store ==============================
-      const CUtensorMap* const maps[1] = {P.o};
-      const int dst_base[1] = {0};
-      const int slot_stride[1] = {kWinBytes};
+      const BoxLayout<1> lay{{P.o}, {0}, {kWinBytes}};
       BoxPlan<1> plan;
       // A tile goes back to its group one item late: the stores of item n are issued, then the warp waits only for the
       // bulk group before (item n - 1) to have been read out of shared memory -- the read latency of one item's stores
@@ -394,12 +376,9 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
         mbar_wait(&so_ready[g], kk & 1);
         if (kk >= *reinterpret_cast<volatile int*>(&sEnd[g])) break;   // the group left its loop: that arrival was its farewell
         trace_evf(P.trace, 4, n, 1);
-        const int4 item = sItem[n % kItemRing], a0 = sGeo[(n % kItemRing) * 2], a1 = sGeo[(n % kItemRing) * 2 + 1];
-        if (item.x != plan.cls) plan.build(S, item.x, lane, maps, dst_base, slot_stride);
-        WinStart w0, w1;
-        w0.b = a0.x; w0.s0 = a0.y; w0.s1 = a0.z; w0.s2 = a0.w;
-        w1.b = a1.x; w1.s0 = a1.y; w1.s1 = a1.z; w1.s2 = a1.w;
-        plan.issue<false>(S, w0, w1, item.w, h * kD, sO + g * kTile, nullptr, lane);
+        const RingItem it = ring.read(n);
+        if (it.cls != plan.cls) plan.build(S, it.cls, lane, lay);
+        plan.issue<false>(S, it.ws[0], it.ws[1], it.nvalid, h * kD, sO + g * kTile, nullptr, lane);
         tma_store_commit();
         tma_store_wait_read<1>();          // per thread: its boxes of item n - 1 have been read
         __syncwarp();
@@ -412,28 +391,23 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
       tma_store_wait_all<0>();
     } else {
       // ============================== TMA producer (K and V tiles) ==============================
-      const CUtensorMap* const maps[2] = {P.k, P.v};
-      const int dst_base[2] = {kQRegion, kQRegion + kTile};
-      const int slot_stride[2] = {kWinBytes, kWinBytes};
+      const BoxLayout<2> lay{{P.k, P.v}, {kQRegion, kQRegion + kTile}, {kWinBytes, kWinBytes}};
       BoxPlan<2> plan;
       int ends = 0;
       for (int n = 0; ends < G; ++n) {
         const int stage = n % kStagesF, phase = (n / kStagesF) & 1;
         mbar_wait(&desc_ready[stage], phase);             // the Q producer has waited for the stage and published the item
-        const int4 item = sItem[n % kItemRing], a0 = sGeo[(n % kItemRing) * 2], a1 = sGeo[(n % kItemRing) * 2 + 1];
-        if (item.x < 0) {                                 // end marker: complete the phase for its readers
+        const RingItem it = ring.read(n);
+        if (it.end()) {                                   // end marker: complete the phase for its readers
           if (lane == 0) mbar_arrive(&full[stage]);
           __syncwarp();
           ++ends;
           continue;
         }
-        if (item.x != plan.cls) plan.build(S, item.x, lane, maps, dst_base, slot_stride);
-        WinStart w0, w1;
-        w0.b = a0.x; w0.s0 = a0.y; w0.s1 = a0.z; w0.s2 = a0.w;
-        w1.b = a1.x; w1.s0 = a1.y; w1.s1 = a1.z; w1.s2 = a1.w;
-        if (lane == 0) mbar_arrive_expect_tx(&full[stage], item.w * 2 * kWinBytes);
+        if (it.cls != plan.cls) plan.build(S, it.cls, lane, lay);
+        if (lane == 0) mbar_arrive_expect_tx(&full[stage], it.nvalid * 2 * kWinBytes);
         __syncwarp();
-        plan.issue<true>(S, w0, w1, item.w, h * kD, sStage + stage * kStageBytesF, &full[stage], lane);
+        plan.issue<true>(S, it.ws[0], it.ws[1], it.nvalid, h * kD, sStage + stage * kStageBytesF, &full[stage], lane);
       }
     }
   } else {
@@ -468,10 +442,10 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
       const int stage = n % kStagesF, phase = (n / kStagesF) & 1;
       TR(n, 0);
       mbar_wait(&full[stage], phase);
-      const int4 item = sItem[n % kItemRing];           // written by the producer before it armed full[stage]
-      if (item.x < 0) break;
-      const int cls = item.x, gw = slot ? item.z : item.y;
-      const bool valid = slot < item.w;
+      const RingItem it = ring.read(n);                 // written by the producer before it armed full[stage]
+      if (it.end()) break;
+      const int cls = it.cls, gw = slot ? it.win[1] : it.win[0];
+      const bool valid = slot < it.nvalid;
       if (cls != cls_loaded) {                          // rare: a CTA sees few classes (ClassQueue)
         named_bar_sync(1 + g, kGroupThreads);           // everyone is done reading the old table
         build_class_table(tbl, kTblLd, bias_h, sPos + cls * 64, sRid + cls * 64, MASK == MMN_MASK_SHIFT && cls != 0, r, kGroupThreads);
@@ -560,12 +534,12 @@ winattn_fwd_tc_kernel(const __grid_constant__ FwdParams P) {
 }
 
 constexpr size_t kFwdSmemBytes = 1024 /*align slack*/ + kStagesF * kStageBytesF + kGroupsF * kTile + kGroupsF * kN * kTblLd * 4 +
-                                 kGroupsF * 256 * 4 + 1024 + kItemRing * 48 + 16 + (3 * kStagesF + 5 * kGroupsF + 1) * 8;
+                                 kGroupsF * 256 * 4 + 1024 + ItemRing<kItemRing>::kBytes + 16 + (3 * kStagesF + 5 * kGroupsF + 1) * 8;
 
 // ------------------------------------------------------------------------------------------
 // Host side
 // ------------------------------------------------------------------------------------------
-inline const char* fwd_why_not_impl(const mmn_winattn_desc* d) {
+const char* fwd_why_not(const mmn_winattn_desc* d) {
   if (d->io_dtype != MMN_DT_BF16) return "io dtype is not bf16";
   if (d->head_dim != kD) return "head_dim != 32";
   if (d->num_heads * 8 > kWorkDone) return "more than 63 heads";
@@ -625,18 +599,39 @@ inline int* arm_work_counters(void* workspace, cudaStream_t st, char* err, size_
   return static_cast<int*>(workspace);
 }
 
-inline int winattn_fwd_launch(const mmn_winattn_desc* d, const void* q, const void* k, const void* v, const float* bias,
-                              const float* head_scale, const float* mask, void* out, float* lse, void* workspace, cudaStream_t st,
-                              char* err, size_t errlen) {
-  FwdParams P;
-  P.S = shape_from(d);
-  P.sc = make_sched(P.S, d->batch, false);
-  const int C = d->num_heads * d->head_dim;
-  if (!make_window_maps(P.q, q, d->q_row_stride, d->batch, C, P.S) || !make_window_maps(P.k, k, d->k_row_stride, d->batch, C, P.S) ||
-      !make_window_maps(P.v, v, d->v_row_stride, d->batch, C, P.S) || !make_window_maps(P.o, out, d->o_row_stride, d->batch, C, P.S)) {
-    snprintf(err, errlen, "cuTensorMapEncodeTiled failed (pointer alignment or strides)");
+inline int tensor_map_failed(char* err, size_t errlen) {
+  snprintf(err, errlen, "cuTensorMapEncodeTiled failed (pointer alignment or strides)");
+  return MMN_ERR_CUDA;
+}
+
+// Launches kernels[variant] of a table of one kernel's template instantiations and reports a launch error under `name`.  The
+// first launch through a table raises the dynamic shared-memory limit of all its variants to `smem` (one table per
+// parameter type: the flag is per instantiation of this template).
+template <class Params, int N>
+inline int launch_variant(void (*const (&kernels)[N])(Params), int variant, size_t smem, int grid, int threads, const Params& P,
+                          cudaStream_t st, const char* name, char* err, size_t errlen) {
+  static std::once_flag once;
+  std::call_once(once, [&] {
+    for (auto kern : kernels) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  });
+  kernels[variant]<<<grid, threads, smem, st>>>(P);
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    snprintf(err, errlen, "%s: %s", name, cudaGetErrorString(e));
     return MMN_ERR_CUDA;
   }
+  return MMN_OK;
+}
+
+int winattn_fwd(const mmn_winattn_desc* d, const void* q, const void* k, const void* v, const float* bias, const float* head_scale,
+                const float* mask, void* out, float* lse, void* workspace, cudaStream_t st, char* err, size_t errlen) {
+  FwdParams P;
+  P.S = shape_from(d);
+  P.sc = make_sched(P.S, d->batch);
+  const int C = d->num_heads * d->head_dim;
+  if (!make_window_maps(P.q, q, d->q_row_stride, d->batch, C, P.S) || !make_window_maps(P.k, k, d->k_row_stride, d->batch, C, P.S) ||
+      !make_window_maps(P.v, v, d->v_row_stride, d->batch, C, P.S) || !make_window_maps(P.o, out, d->o_row_stride, d->batch, C, P.S))
+    return tensor_map_failed(err, errlen);
   P.nH = d->num_heads;
   P.mask_windows = d->mask_windows > 0 ? d->mask_windows : 1;
   P.scale = d->scale;
@@ -647,26 +642,17 @@ inline int winattn_fwd_launch(const mmn_winattn_desc* d, const void* q, const vo
   const char* trace_path = getenv("MMN_TC_TRACE");
   P.trace = trace_setup(trace_path, st);
 
-  using Kern = void (*)(const FwdParams);
-  static const Kern kernels[2][3] = {
-      {winattn_fwd_tc_kernel<false, MMN_MASK_NONE>, winattn_fwd_tc_kernel<false, MMN_MASK_SHIFT>, winattn_fwd_tc_kernel<false, MMN_MASK_TENSOR>},
-      {winattn_fwd_tc_kernel<true, MMN_MASK_NONE>, winattn_fwd_tc_kernel<true, MMN_MASK_SHIFT>, winattn_fwd_tc_kernel<true, MMN_MASK_TENSOR>}};
-  static std::once_flag once;
-  std::call_once(once, [] {
-    for (int c = 0; c < 2; ++c)
-      for (int m = 0; m < 3; ++m) cudaFuncSetAttribute(kernels[c][m], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmemBytes);
-  });
-  const Kern kern = kernels[d->score_kind == MMN_SCORE_COSINE ? 1 : 0][d->mask_kind];
+  // [cosine][mask kind]
+  static void (*const kernels[6])(FwdParams) = {winattn_fwd_tc_kernel<false, MMN_MASK_NONE>, winattn_fwd_tc_kernel<false, MMN_MASK_SHIFT>,
+                                                winattn_fwd_tc_kernel<false, MMN_MASK_TENSOR>, winattn_fwd_tc_kernel<true, MMN_MASK_NONE>,
+                                                winattn_fwd_tc_kernel<true, MMN_MASK_SHIFT>, winattn_fwd_tc_kernel<true, MMN_MASK_TENSOR>};
   int per_head = num_sms_cached() / P.nH;        // CTAs per head (each CTA keeps one head's table resident)
   if (per_head < 1) per_head = 1;
   if (per_head > P.sc.n_items) per_head = P.sc.n_items;
   P.per_head = per_head;
-  kern<<<per_head * P.nH, kFwdThreads, kFwdSmemBytes, st>>>(P);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) {
-    snprintf(err, errlen, "winattn_fwd_tc_kernel: %s", cudaGetErrorString(e));
-    return MMN_ERR_CUDA;
-  }
+  const int rc = launch_variant(kernels, (d->score_kind == MMN_SCORE_COSINE ? 3 : 0) + d->mask_kind, kFwdSmemBytes, per_head * P.nH,
+                                kFwdThreads, P, st, "winattn_fwd_tc_kernel", err, errlen);
+  if (rc != MMN_OK) return rc;
   if (P.trace.buf) dump_trace(P.trace.buf, trace_path, st);      // debug only: synchronous dump of CTA 0's timeline
   return MMN_OK;
 }

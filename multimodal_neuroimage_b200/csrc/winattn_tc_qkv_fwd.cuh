@@ -3,7 +3,7 @@
 //   qkv = x W_qkv^T + b_qkv        fp32 accumulate, fp32 bias, rounded to bf16 and written to global (the backward reads it)
 //   out, lse, records              exactly what winattn_fwd_tc_kernel computes from that bf16 qkv
 //
-// Shape: C = 96 = 3 heads x 32, 64-token windows (fwd_why_not_impl's shapes), y = None.  The separate projection wrote
+// Shape: C = 96 = 3 heads x 32, 64-token windows (fwd_why_not's shapes), y = None.  The separate projection wrote
 // qkv (3C per token) and the attention read it straight back; here x (C per token) is read once and qkv only written.
 //
 // A work item is a PAIR of windows of one wrap class (tc_sched.cuh, ClassQueue, one queue for all heads), now across all
@@ -46,7 +46,7 @@ constexpr int kOpTile = 128 * 64;                   // the pair's Q, K or V tile
 constexpr int kOpSet = 3 * kOpTile;
 constexpr int kQkvBars = 2 * kXStages + 8 * kGroupsF;
 constexpr size_t kQkvSmemBytes = 1024 /*align slack*/ + kWBytes + kXStages * kXStage + kGroupsF * kOpSet + kGroupsF * kN * kN * 4 +
-                                 kGroupsF * 128 * 4 + 1024 + kItemRing * 48 + 16 + kQkvBars * 8 + 8;
+                                 kGroupsF * 128 * 4 + 1024 + ItemRing<kItemRing>::kBytes + 16 + kQkvBars * 8 + 8;
 static_assert(kQkvSmemBytes <= 227 * 1024, "fused qkv forward: shared memory over the 227 KB a block may use");
 static_assert(kGroupsF * kTmemGroup <= kTmemColsF && 96 <= 128, "fused qkv forward: TMEM columns");
 
@@ -89,9 +89,8 @@ winattn_qkv_fwd_tc_kernel(const __grid_constant__ QkvFwdParams P) {
   float* sRk = sTbl + G * kN * kN;                        // [G][128] per-key 1/||k||
   uint8_t* sPos = reinterpret_cast<uint8_t*>(sRk + G * 128);
   uint8_t* sRid = sPos + 512;
-  int4* sItem = reinterpret_cast<int4*>(sRid + 512);      // [kItemRing] per pair {class (-1: end), window 0, window 1, valid slots}
-  int4* sGeo = sItem + kItemRing;                         // [kItemRing][2]
-  int* sEnd = reinterpret_cast<int*>(sGeo + 2 * kItemRing);
+  const ItemRing<kItemRing> ring{reinterpret_cast<int4*>(sRid + 512)};      // pair descriptors (tc_sched.cuh)
+  int* sEnd = reinterpret_cast<int*>(sRid + 512 + ring.kBytes);
   uint64_t* bars = reinterpret_cast<uint64_t*>(sEnd + 4);
   uint64_t* x_full = bars;                                // [kXStages] TMA -> MMA
   uint64_t* x_empty = x_full + kXStages;                  // [kXStages] the pair's last projection -> TMA
@@ -119,10 +118,7 @@ winattn_qkv_fwd_tc_kernel(const __grid_constant__ QkvFwdParams P) {
     *reinterpret_cast<uint4*>(sW + hp * kWPanel + j * 64 + ((c ^ ((j >> 1) & 3)) << 4)) = v;
   }
   for (int i = tid; i < (kXStages * kXStage) / 16; i += kFwdThreads) reinterpret_cast<uint4*>(sX)[i] = make_uint4(0, 0, 0, 0);
-  for (int i = tid; i < 512; i += kFwdThreads) {
-    sPos[i] = (uint8_t)piece_position(S, i >> 6, i & 63);
-    sRid[i] = (uint8_t)class_region_id(S, i >> 6, i & 63);
-  }
+  fill_class_luts(S, sPos, sRid, tid, kFwdThreads);
   if (tid == 0) {
     for (int g = 0; g < G; ++g) sEnd[g] = 0x7fffffff;
     for (int s = 0; s < kXStages; ++s) { mbar_init(&x_full[s], 1); mbar_init(&x_empty[s], 1); }
@@ -150,41 +146,28 @@ winattn_qkv_fwd_tc_kernel(const __grid_constant__ QkvFwdParams P) {
     setmaxnreg_dec<kRegAuxF>();
     if (warp == kProducerWarp) {
       // ============================== TMA producer: schedule, pair descriptors, x tiles ==============================
-      const CUtensorMap* const maps[3] = {P.x[0], P.x[1], P.x[2]};
-      const int dst_base[3] = {0, kXPanel, 2 * kXPanel};
-      const int slot_stride[3] = {kWinBytes, kWinBytes, kWinBytes};
+      const BoxLayout<3> lay{{P.x[0], P.x[1], P.x[2]}, {0, kXPanel, 2 * kXPanel}, {kWinBytes, kWinBytes, kWinBytes}};
       BoxPlan<3> plan;
       // ring depth (kItemRing): entry n + 16 is written once x stage (n + 16) % 2 is free, i.e. after the projections of
       // pair n + 14, which waited for PV of every sub-item of pair n + 13: every group, and both store warps (one item
       // behind their groups), are past pair n.
-      int n = 0;
-      ClassQueue wq;
-      const int chunk = max(1, min(kChunkF, sc.n_items / ((int)gridDim.x * 8)));
-      wq.init(sc, sched_range_begin(sc, blockIdx.x, gridDim.x), P.work, chunk, lane);
-      for (int c0, m; wq.next(sc, P.work, chunk, lane, c0, m);) {
-        ItemCursor cur;
-        cur.seek(sc, c0);
-        for (int t = 0; t < m; ++t, ++n, cur.next_item(sc)) {
-          const int stage = n % kXStages, phase = (n / kXStages) & 1;
-          if (cur.cls != plan.cls) plan.build(S, cur.cls, lane, maps, dst_base, slot_stride);
-          const int nvalid = cur.slot_valid(1) ? 2 : 1;
-          int w0, w1;
-          const WinStart ws0 = cursor_start(S, cur, 0, w0), ws1 = cursor_start(S, cur, 1, w1);
-          mbar_wait(&x_empty[stage], phase ^ 1);
-          if (lane == 0) {
-            sItem[n % kItemRing] = make_int4(cur.cls, w0, w1, nvalid);     // published by the arrival below
-            sGeo[(n % kItemRing) * 2] = make_int4(ws0.b, ws0.s0, ws0.s1, ws0.s2);
-            sGeo[(n % kItemRing) * 2 + 1] = make_int4(ws1.b, ws1.s0, ws1.s1, ws1.s2);
-            mbar_arrive_expect_tx(&x_full[stage], nvalid * 3 * kWinBytes);
-          }
-          __syncwarp();
-          plan.issue<true>(S, ws0, ws1, nvalid, 0, sX + stage * kXStage, &x_full[stage], lane);
+      auto load_pair = [=, &P, &S, &plan](int n, const RingItem& it) {
+        const int stage = n % kXStages, phase = (n / kXStages) & 1;
+        if (it.cls != plan.cls) plan.build(S, it.cls, lane, lay);
+        mbar_wait(&x_empty[stage], phase ^ 1);
+        if (lane == 0) {
+          ring.publish(n, it);                                          // published by the arrival below
+          mbar_arrive_expect_tx(&x_full[stage], it.nvalid * 3 * kWinBytes);
         }
-      }
+        __syncwarp();
+        plan.issue<true>(S, it.ws[0], it.ws[1], it.nvalid, 0, sX + stage * kXStage, &x_full[stage], lane);
+      };
+      const int chunk = max(1, min(kChunkF, sc.n_items / ((int)gridDim.x * 8)));
+      const int n = walk_queue(S, sc, sched_range_begin(sc, blockIdx.x, gridDim.x), P.work, chunk, lane, load_pair);
       const int stage = n % kXStages, phase = (n / kXStages) & 1;      // end marker
       mbar_wait(&x_empty[stage], phase ^ 1);
       if (lane == 0) {
-        sItem[n % kItemRing] = make_int4(-1, 0, 0, 0);
+        ring.publish_end(n);
         mbar_arrive(&x_full[stage]);
       }
       __syncwarp();
@@ -207,7 +190,7 @@ winattn_qkv_fwd_tc_kernel(const __grid_constant__ QkvFwdParams P) {
           const int pr = nj / G, h = nj - pr * G, xs = pr % kXStages;
           if ((h != 0 || mbar_test(&x_full[xs], (pr / kXStages) & 1)) && (nj < G || mbar_test(&o_full[h], (pr - 1) & 1))) {
             progressed = true;
-            if (h == 0 && sItem[pr % kItemRing].x < 0) {
+            if (h == 0 && ring.read(pr).end()) {
               total = nj;
             } else {
               tcgen05_fence_after();
@@ -269,21 +252,16 @@ winattn_qkv_fwd_tc_kernel(const __grid_constant__ QkvFwdParams P) {
       // Unlike the unfused kernel's store warp, a tile goes back to its group as soon as its stores have read it: the
       // group waits for it before draining its next projection (the tile is its Q tile), at the head of its chain, and
       // handing it back one item late made every group wait for the next group's epilogue.
-      const CUtensorMap* const maps[1] = {P.o};
-      const int dst_base[1] = {0};
-      const int slot_stride[1] = {kWinBytes};
+      const BoxLayout<1> lay{{P.o}, {0}, {kWinBytes}};
       BoxPlan<1> plan;
       int n = 0;
       for (;; ++n) {
         const int g = n % G, kk = n / G;
         mbar_wait(&so_ready[g], kk & 1);
         if (kk >= *reinterpret_cast<volatile int*>(&sEnd[g])) break;
-        const int4 item = sItem[kk % kItemRing], a0 = sGeo[(kk % kItemRing) * 2], a1 = sGeo[(kk % kItemRing) * 2 + 1];
-        if (item.x != plan.cls) plan.build(S, item.x, lane, maps, dst_base, slot_stride);
-        WinStart ws0, ws1;
-        ws0.b = a0.x; ws0.s0 = a0.y; ws0.s1 = a0.z; ws0.s2 = a0.w;
-        ws1.b = a1.x; ws1.s0 = a1.y; ws1.s1 = a1.z; ws1.s2 = a1.w;
-        plan.issue<false>(S, ws0, ws1, item.w, g * kD, sOp + g * kOpSet, nullptr, lane);
+        const RingItem it = ring.read(kk);
+        if (it.cls != plan.cls) plan.build(S, it.cls, lane, lay);
+        plan.issue<false>(S, it.ws[0], it.ws[1], it.nvalid, g * kD, sOp + g * kOpSet, nullptr, lane);
         tma_store_commit();
         tma_store_wait_read<0>();
         __syncwarp();
@@ -292,20 +270,15 @@ winattn_qkv_fwd_tc_kernel(const __grid_constant__ QkvFwdParams P) {
       tma_store_wait_all<0>();
     } else {
       // ============================== TMA store of the Q, K, V tiles to qkv ==============================
-      const CUtensorMap* const maps[3] = {P.q, P.k, P.v};
-      const int dst_base[3] = {0, kOpTile, 2 * kOpTile};
-      const int slot_stride[3] = {kWinBytes, kWinBytes, kWinBytes};
+      const BoxLayout<3> lay{{P.q, P.k, P.v}, {0, kOpTile, 2 * kOpTile}, {kWinBytes, kWinBytes, kWinBytes}};
       BoxPlan<3> plan;
       for (int n = 0;; ++n) {
         const int g = n % G, kk = n / G;
         mbar_wait(&tiles_full[g], kk & 1);
-        const int4 item = sItem[kk % kItemRing], a0 = sGeo[(kk % kItemRing) * 2], a1 = sGeo[(kk % kItemRing) * 2 + 1];
-        if (item.x < 0) break;                       // group 0's farewell: every earlier sub-item is stored
-        if (item.x != plan.cls) plan.build(S, item.x, lane, maps, dst_base, slot_stride);
-        WinStart ws0, ws1;
-        ws0.b = a0.x; ws0.s0 = a0.y; ws0.s1 = a0.z; ws0.s2 = a0.w;
-        ws1.b = a1.x; ws1.s0 = a1.y; ws1.s1 = a1.z; ws1.s2 = a1.w;
-        plan.issue<false>(S, ws0, ws1, item.w, g * kD, sOp + g * kOpSet, nullptr, lane);
+        const RingItem it = ring.read(kk);
+        if (it.end()) break;                         // group 0's farewell: every earlier sub-item is stored
+        if (it.cls != plan.cls) plan.build(S, it.cls, lane, lay);
+        plan.issue<false>(S, it.ws[0], it.ws[1], it.nvalid, g * kD, sOp + g * kOpSet, nullptr, lane);
         tma_store_commit();
         tma_store_wait_read<0>();
         __syncwarp();
@@ -332,11 +305,11 @@ winattn_qkv_fwd_tc_kernel(const __grid_constant__ QkvFwdParams P) {
     int kk = 0;
     for (;; ++kk) {
       mbar_wait(&proj_full[g], kk & 1);
-      const int4 item = sItem[kk % kItemRing];
-      if (item.x < 0) break;
+      const RingItem it = ring.read(kk);
+      if (it.end()) break;
       tcgen05_fence_after();
-      const int cls = item.x, gw = slot ? item.z : item.y;
-      const bool valid = slot < item.w;
+      const int cls = it.cls, gw = slot ? it.win[1] : it.win[0];
+      const bool valid = slot < it.nvalid;
       if (cls != cls_loaded) {
         named_bar_sync(1 + g, kGroupThreads);
         build_class_table(tbl, kN, bias_h, sPos + cls * 64, sRid + cls * 64, MASK == MMN_MASK_SHIFT && cls != 0, r, kGroupThreads, 7);
@@ -447,18 +420,17 @@ winattn_qkv_fwd_tc_kernel(const __grid_constant__ QkvFwdParams P) {
 // ------------------------------------------------------------------------------------------
 // Host side
 // ------------------------------------------------------------------------------------------
-inline const char* qkv_fwd_why_not_impl(const mmn_winattn_desc* d, int in_channels) {
+const char* qkv_fwd_why_not(const mmn_winattn_desc* d, int in_channels) {
   if (d->num_heads != kQkvHeads || d->head_dim != kD) return "the fused qkv kernel is built for 3 heads of 32 channels (C = 96)";
   if (in_channels != kQkvC) return "input channels differ from the attention width";
-  return fwd_why_not_impl(d);
+  return fwd_why_not(d);
 }
 
-inline int winattn_qkv_fwd_launch(const mmn_winattn_desc* d, const void* x, const void* w, const float* b, const float* bias,
-                                  const float* head_scale, const float* mask, void* qkv, void* out, float* lse, void* workspace,
-                                  cudaStream_t st, char* err, size_t errlen) {
+int winattn_qkv_fwd(const mmn_winattn_desc* d, const void* x, const void* w, const float* b, const float* bias, const float* head_scale,
+                    const float* mask, void* qkv, void* out, float* lse, void* workspace, cudaStream_t st, char* err, size_t errlen) {
   QkvFwdParams P;
   P.S = shape_from(d);
-  P.sc = make_sched(P.S, d->batch, false);
+  P.sc = make_sched(P.S, d->batch);
   const char* xb = static_cast<const char*>(x);
   char* qb = static_cast<char*>(qkv);
   bool ok = reinterpret_cast<uintptr_t>(w) % 16 == 0;
@@ -467,10 +439,7 @@ inline int winattn_qkv_fwd_launch(const mmn_winattn_desc* d, const void* x, cons
        make_window_maps(P.k, qb + kQkvC * 2, 3 * kQkvC, d->batch, kQkvC, P.S) &&
        make_window_maps(P.v, qb + 2 * kQkvC * 2, 3 * kQkvC, d->batch, kQkvC, P.S) &&
        make_window_maps(P.o, out, kQkvC, d->batch, kQkvC, P.S);
-  if (!ok) {
-    snprintf(err, errlen, "cuTensorMapEncodeTiled failed (pointer alignment or strides)");
-    return MMN_ERR_CUDA;
-  }
+  if (!ok) return tensor_map_failed(err, errlen);
   P.mask_windows = d->mask_windows > 0 ? d->mask_windows : 1;
   P.scale = d->scale;
   P.w = static_cast<const __nv_bfloat16*>(w); P.b = b;
@@ -479,25 +448,14 @@ inline int winattn_qkv_fwd_launch(const mmn_winattn_desc* d, const void* x, cons
   P.work = arm_work_counters(workspace, st, err, errlen);
   if (!P.work) return MMN_ERR_CUDA;
 
-  using Kern = void (*)(const QkvFwdParams);
-  static const Kern kernels[2][3] = {
-      {winattn_qkv_fwd_tc_kernel<false, MMN_MASK_NONE>, winattn_qkv_fwd_tc_kernel<false, MMN_MASK_SHIFT>, winattn_qkv_fwd_tc_kernel<false, MMN_MASK_TENSOR>},
-      {winattn_qkv_fwd_tc_kernel<true, MMN_MASK_NONE>, winattn_qkv_fwd_tc_kernel<true, MMN_MASK_SHIFT>, winattn_qkv_fwd_tc_kernel<true, MMN_MASK_TENSOR>}};
-  static std::once_flag once;
-  std::call_once(once, [] {
-    for (int c = 0; c < 2; ++c)
-      for (int m = 0; m < 3; ++m) cudaFuncSetAttribute(kernels[c][m], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kQkvSmemBytes);
-  });
-  const Kern kern = kernels[d->score_kind == MMN_SCORE_COSINE ? 1 : 0][d->mask_kind];
+  // [cosine][mask kind]
+  static void (*const kernels[6])(QkvFwdParams) = {
+      winattn_qkv_fwd_tc_kernel<false, MMN_MASK_NONE>, winattn_qkv_fwd_tc_kernel<false, MMN_MASK_SHIFT>, winattn_qkv_fwd_tc_kernel<false, MMN_MASK_TENSOR>,
+      winattn_qkv_fwd_tc_kernel<true, MMN_MASK_NONE>, winattn_qkv_fwd_tc_kernel<true, MMN_MASK_SHIFT>, winattn_qkv_fwd_tc_kernel<true, MMN_MASK_TENSOR>};
   int grid = num_sms_cached();
   if (grid > P.sc.n_items) grid = P.sc.n_items;
-  kern<<<grid, kFwdThreads, kQkvSmemBytes, st>>>(P);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) {
-    snprintf(err, errlen, "winattn_qkv_fwd_tc_kernel: %s", cudaGetErrorString(e));
-    return MMN_ERR_CUDA;
-  }
-  return MMN_OK;
+  return launch_variant(kernels, (d->score_kind == MMN_SCORE_COSINE ? 3 : 0) + d->mask_kind, kQkvSmemBytes, grid, kFwdThreads, P, st,
+                        "winattn_qkv_fwd_tc_kernel", err, errlen);
 }
 
 }}  // namespace mmn::tc
