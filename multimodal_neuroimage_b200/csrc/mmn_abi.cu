@@ -475,7 +475,7 @@ int mmn_layernorm_fwd(const void* resid, int resid_dtype, const void* delta, int
   int n = 0;
   cudaError_t e = mmn::layernorm_fwd(resid, resid_dtype, delta, delta_dtype, gamma, beta, eps, mode, out_sum, sum_dtype, out_norm, norm_dtype,
                                      mean, rstd, rows, cols, (cudaStream_t)stream, &n);
-  return finish(e, n, "ln_fwd_kernel");
+  return finish(e, n, "layernorm_fwd_kernel");
 }
 
 size_t mmn_layernorm_bwd_workspace_bytes(int64_t rows, int32_t cols) {
@@ -499,7 +499,7 @@ int mmn_layernorm_bwd(const void* g_sum, int gs_dtype, const void* g_norm, int g
   int n = 0;
   cudaError_t e = mmn::layernorm_bwd(g_sum, gs_dtype, g_norm, gn_dtype, x, x_dtype, gamma, mean, rstd, mode, d_resid, dr_dtype, d_delta,
                                      dd_dtype, dgamma, dbeta, deterministic ? workspace : nullptr, rows, cols, (cudaStream_t)stream, &n);
-  return finish(e, n, "ln_bwd_kernel");
+  return finish(e, n, "layernorm_bwd_kernel");
 }
 
 }  // extern "C"

@@ -20,6 +20,7 @@ All tensors are in the un-windowed, un-shifted (B, *grid, channels) order.
 from __future__ import annotations
 
 import ctypes as C
+import functools
 from typing import List, Optional, Tuple
 
 import torch
@@ -744,8 +745,13 @@ _DTC = {torch.float32: _lib.DT_F32, torch.bfloat16: _lib.DT_BF16}
 _DTC_INV = {_lib.DT_F32: torch.float32, _lib.DT_BF16: torch.bfloat16}
 
 
+@functools.lru_cache(maxsize=None)
+def _layernorm_width_supported(cols: int) -> bool:
+    return bool(_lib.load().mmn_layernorm_supported(cols))
+
+
 def layernorm_supported(x: Tensor, cols: int) -> bool:
-    return bool(x.is_cuda and x.dtype in _DTC and cols % 2 == 0 and 2 <= cols <= 1536 and x.numel() > 0)
+    return bool(x.is_cuda and x.dtype in _DTC and x.numel() > 0 and _layernorm_width_supported(cols))
 
 
 @torch.library.custom_op("mmn_b200::layernorm_fwd", mutates_args=())

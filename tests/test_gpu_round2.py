@@ -451,10 +451,12 @@ def test_fused_mlp_matches_pytorch(mm, C, act, rep):
 # ------------------------------------------------------------------------------------------
 # LayerNorm fused with the residual add (csrc/layernorm.cu) against torch.nn.functional.layer_norm in fp64
 # ------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("cols", [12, 84, 96, 168, 192, 384, 768, 1536])
+# 98, 1534 and the inputs at a storage offset of 2 elements (not 16-byte aligned) take the two-column chunks (W = 2)
+@pytest.mark.parametrize("cols,offset", [pytest.param(c, 0, id=str(c)) for c in (12, 84, 96, 168, 192, 384, 768, 1536, 98, 1024, 1534)]
+                         + [pytest.param(c, 2, id=f"{c}-offset2") for c in (96, 1024)])
 @pytest.mark.parametrize("stream_dtype,act_dtype", [(torch.float32, torch.float32), (torch.float32, torch.bfloat16), (torch.bfloat16, torch.bfloat16)],
                          ids=["f32_f32", "f32_bf16", "bf16_bf16"])
-def test_fused_layernorm(mm, cols, stream_dtype, act_dtype):
+def test_fused_layernorm(mm, cols, offset, stream_dtype, act_dtype):
     from multimodal_neuroimage_b200 import fused
     F = torch.nn.functional
     rows = (3, 211)
@@ -485,9 +487,15 @@ def test_fused_layernorm(mm, cols, stream_dtype, act_dtype):
             loss = (s * c1.double()).sum() + (s * c2.double()).sum()
         return outs, torch.autograd.grad(loss, (r, d, w, b), allow_unused=True)
 
+    def on_gpu(t):                  # a contiguous copy of t that starts `offset` elements into its storage
+        buf = torch.empty(t.numel() + offset, dtype=t.dtype, device="cuda")
+        buf[offset:].copy_(t.flatten())
+        return buf[offset:].view(t.shape).detach().requires_grad_(True)
+
     lnc = ln.cuda()
     for mode in ("ln", "pre", "post"):
-        rc, dc = resid.cuda().requires_grad_(True), delta.cuda().requires_grad_(True)
+        rc, dc = on_gpu(resid), on_gpu(delta)
+        assert rc.is_contiguous() and (rc.data_ptr() % 16 != 0) == (offset != 0)
         lnc.zero_grad()
         if mode == "ln":
             outs = (fused.layer_norm(rc, lnc, act_dtype),)
